@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the SMPL hot path: SMPL meshes/sec, forward+backward (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--mode fp32|bf16]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--mode fp32|bf16] [--dump-outputs DIR]
 
 One "step" = one forward+backward pass of the batched SMPL layer over one batch of synthetic
 (betas, pose, trans) with upstream gradients (dV, dJ): BASELINE.json configs[1] (B = 4096 bodies on
@@ -11,7 +11,8 @@ Prints ONE JSON line (rank 0).  `value` = bodies processed by all ranks / max-ov
 time with inputs resident in HBM; `e2e` = the same metric through the public module API with the
 step's inputs copied from pinned host memory and the gradients copied back inside the timed region.
 `--impl reference` times the reference's CPU path (the PyTorch-eager oracle port, all host threads)
-on a bounded sample of the same workload.
+on a bounded sample of the same workload.  `--dump-outputs DIR` writes what the last timed step returned
+(rank 0) as DIR/<name>.npy, so that two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -25,6 +26,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -95,6 +97,26 @@ def make_inputs(B, seed, device):
     x = make_smpl_inputs(B, seed)
     dV, dJ = make_upstream_grads(B, seed)
     return [t.to(device) for t in (x["betas"], x["rotmats"], x["trans"], dV, dJ)]
+
+
+DUMP_BODIES = 512              # 512 bodies' vertices are 42 MB: a dump stays under 64 MB at any batch
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, outputs, B):
+    """Write the per-body outputs of one step as float32 DIR/<name>.npy, all of them for the same bodies: every body
+    when B <= DUMP_BODIES, else a fixed sample of DUMP_BODIES bodies drawn with seed 0 (in ascending order)."""
+    if B <= DUMP_BODIES:
+        idx = torch.arange(B)
+    else:
+        idx = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:DUMP_BODIES].sort().values
+    arrays = {name: t.detach()[idx.to(t.device)].float().cpu().numpy() for name, t in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -269,7 +291,15 @@ def main():
     ap.add_argument("--sustain-seconds", type=float, default=2.0,
                     help="extra leg: the same step repeated for this long with NVML clocks (0 = skip)")
     ap.add_argument("--no-extras", action="store_true", help="skip the sustained / small-batch / forward-only legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned on rank 0 (vertices, joints and the "
+                         "gradients of betas, rotation matrices and translation; float32, at most %d bodies) as "
+                         "DIR/<name>.npy" % DUMP_BODIES)
     args = ap.parse_args()
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        raise SystemExit("--dump-outputs writes the outputs of the timed device path (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -326,8 +356,12 @@ def main():
     betas, rot, trans, dV, dJ = make_inputs(B, seed=rank, device=dev)
 
     def step():
-        saved = eng.forward(betas, rot, trans, None, mode=mode, slab=args.slab, save=True)[3]
-        return eng.backward(betas, rot, trans, None, None, dV, dJ, None, mode=mode, slab=args.slab, saved=saved)
+        """One forward + backward; returns what a caller of this path receives."""
+        v, j, _, saved = eng.forward(betas, rot, trans, None, mode=mode, slab=args.slab, save=True)
+        g_betas, g_rot, g_trans, _ = eng.backward(betas, rot, trans, None, None, dV, dJ, None, mode=mode,
+                                                  slab=args.slab, saved=saved)
+        return {"vertices": v, "joints": j, "grad_betas": g_betas, "grad_rotmats": g_rot.view(B, 24, 3, 3),
+                "grad_trans": g_trans}
 
     def sync_all():
         torch.cuda.synchronize(dev)
@@ -335,8 +369,9 @@ def main():
             dist.barrier()
             torch.cuda.synchronize(dev)
 
+    # warm-up and timed steps alike hold one step's outputs while the next runs: the same allocations in both
     for _ in range(warmup):
-        step()
+        last = step()
     sync_all()
     sampler = ClockSampler(local_rank)
     if rank == 0:
@@ -345,12 +380,15 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step()
+        last = step()
     e1.record()
     sync_all()
     launches = lib.b200smpl_launch_count() - launches0
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, B)
+    del last
     from soccerplayershapepose_b200 import sharding
     ms_total = sharding.max_over_ranks(ms_total, dev)           # the slowest rank decides
     value = sharding.aggregate_throughput(B, world, args.steps, ms_total)
