@@ -105,7 +105,9 @@ B200SMPL_API int b200smpl_model_get_info(const b200smpl_model* m, b200smpl_model
 B200SMPL_API int b200smpl_model_debug_array(const b200smpl_model* m, const char* name, const void** data, size_t* bytes);
 
 /* Bytes of caller-provided scratch needed by forward / backward for `batch` bodies.
- * slab_bodies = 0 lets the library pick the slab (bodies processed per L2-resident pass). */
+ * slab_bodies = 0 lets the library pick the slab (bodies processed per L2-resident pass); a
+ * request is rounded up to a multiple of 128 and capped at 40960 bodies (the widest slab the
+ * forward GEMMs' work lists hold).  Results do not depend on the slab. */
 /* Bytes of the optional "saved for backward" buffer (blend output + skinning transforms of the
  * whole batch, ~93 KB per body).  When forward writes it and backward receives it, the backward
  * skips the recomputation of the pose stage and of the blend GEMM. */

@@ -17,7 +17,7 @@ CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(HERE, "csrc", "build")
 LIB = os.path.join(HERE, "libb200smpl.so")
 
-SOURCES = ["api.cu", "pack.cu", "pose.cu", "blend_simt.cu", "blend_umma.cu", "fused_fwd.cu", "fused_bwd.cu", "lbs.cu", "joints.cu", "aux_ops.cu", "fit.cu", "loss.cu"]
+SOURCES = ["api.cu", "pack.cu", "pose.cu", "blend_simt.cu", "blend_umma.cu", "fused_fwd.cu", "lbs.cu", "joints.cu", "aux_ops.cu", "fit.cu", "loss.cu"]
 HEADERS = [os.path.join(CSRC, h) for h in sorted(os.listdir(CSRC)) if h.endswith(".cuh")] + [
     os.path.join(HERE, "..", "include", "b200smpl.h")]
 

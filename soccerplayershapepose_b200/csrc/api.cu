@@ -8,6 +8,7 @@
 #include <nvtx3/nvToolsExt.h>
 
 #include "common.cuh"
+#include "umma_common.cuh"
 
 namespace b200smpl {
 
@@ -60,6 +61,13 @@ static int bwd_gemm_mode(int mode) {
 }
 
 constexpr int DEFAULT_SLAB = 4096;   // bodies per pass (vpT slab = n_pad * S * 4 B)
+// widest slab: the forward GEMMs' work lists hold BS_MAX_WORK pairs of 128-body tiles.  Wider requests are cut to it;
+// results do not depend on the slab width.
+constexpr int MAX_SLAB = 40960;
+static_assert(MAX_SLAB == 2 * BM * BS_MAX_WORK, "slab cap = the forward GEMMs' work-list capacity");
+// fewest 64-row K slabs one split of a row-range gradient GEMM (joints only / vertices only) may get.  Fitting
+// iteration at 1024 players: 74.3 us with 8, 71.3 with 4, 73.6 with 2
+constexpr int MIN_SLABS_PER_SPLIT = 4;
 
 struct Plan {
   int S;                 // slab pitch (multiple of 128)
@@ -71,20 +79,12 @@ struct Plan {
 };
 
 static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
-// fewest 64-row K slabs one split of a row-range gradient GEMM (joints only / vertices only) may get
-static int min_slabs_per_split() {
-  static const int v = [] {
-    const char* e = getenv("B200_BWD_SPLIT_SLABS");
-    return e && atoi(e) > 0 ? atoi(e) : 4;   // fitting iteration at 1024 players: 74.3 us with 8, 71.3 with 4, 73.6 with 2
-  }();
-  return v;
-}
 
 static Plan make_plan(const b200smpl_model* m, int batch, int mode, int slab_bodies, bool backward) {
   const DevModel& d = m->dm;
   Plan p{};
   const int Bp = round_up(std::max(batch, 1), 128);
-  int S = slab_bodies > 0 ? round_up(slab_bodies, 128) : DEFAULT_SLAB;
+  const int S = slab_bodies > 0 ? round_up(std::min(slab_bodies, MAX_SLAB), 128) : DEFAULT_SLAB;
   p.S = std::min(S, Bp);
   size_t off = 0;
   auto take = [&](size_t bytes) {
@@ -108,12 +108,7 @@ static Plan make_plan(const b200smpl_model* m, int batch, int mode, int slab_bod
     p.off_dA = take((size_t)(NJ * AELEMS + 3) * S_ * 4);
     p.off_dtr = p.off_dA + (size_t)NJ * AELEMS * S_ * 4;
     p.off_dJtot = take((size_t)std::max(batch, 1) * d.njout * 3 * 4);
-    // split-K partials of the gradient GEMM; the fused backward (fused_bwd.cu) writes one partial per piece of a body
-    // pair's item range and the virtual (joint) rows keep their own GEMM behind it
-    int parts = p.k_splits;
-    if (bmode != B200SMPL_MODE_FP32_SIMT && d.fl.nf_pad == 224)
-      parts = std::max(parts, std::max(0, fused_bwd_parts(d, p.S, m->num_sms)) + p.k_splits);
-    p.off_dfeat = take((size_t)parts * S_ * d.fl.nf_pad * 4);
+    p.off_dfeat = take((size_t)p.k_splits * S_ * d.fl.nf_pad * 4);   // split-K partials of the gradient GEMM
   }
   p.total = off + 1024;   // slack for aligning the caller's base pointer
   return p;
@@ -223,8 +218,6 @@ int b200smpl_model_create(const b200smpl_model_desc* desc, int device, b200smpl_
   UP(Wf, h.Wf);
   UP(Wb_hi, h.Wb_hi);
   UP(Wb_lo, h.Wb_lo);
-  UP(Wbi_hi, h.Wbi_hi);
-  UP(Wbi_lo, h.Wbi_lo);
   UP(W32, h.W32);
   UP(vmeta, h.vmeta);
   UP(vwts, h.vwts);
@@ -340,19 +333,18 @@ int b200smpl_forward(const b200smpl_model* m, const b200smpl_forward_args* a, vo
       return rc;
     // forward-only calls that want vertices (no products kept for a backward): the blend GEMM skins in its epilogue
     // and v_posed never touches HBM (188 us against 108 + 136 us at B = 4096).  When the products are kept the
-    // fused kernel would write v_posed AND the vertices (658 MB of pure writes, 242 us): no faster than the two
-    // kernels, so that case stays on them (B200_FUSED_FWD=2 forces the fused kernel, 0 disables it).
-    // Below ~512 bodies a call is launch-latency bound and the two kernels (PDL-chained) are as fast or faster
-    // (scripts/fwd_only_sweep.py: 53 vs 47 us at B = 64, 57 vs 65 us at B = 512, 0.211 vs 0.263 ms at B = 4096).
-    const bool fused = a->vertices != nullptr && a->mode != B200SMPL_MODE_FP32_SIMT && d.n_virt0 == d.ntiles * 96 &&
-                       (saved == nullptr ? (fused_fwd_mode() >= 2 || (fused_fwd_mode() == 1 && nb >= 512)) : fused_fwd_mode() >= 2);
+    // fused kernel would have to write v_posed AND the vertices (658 MB of pure writes, 242 us): no faster than the
+    // two kernels, so that case stays on them.  Below ~512 bodies a call is launch-latency bound and the two kernels
+    // (PDL-chained) are as fast or faster (53 vs 47 us at B = 64, 57 vs 65 us at B = 512, 0.211 vs 0.263 ms at
+    // B = 4096).
+    const bool fused = a->vertices != nullptr && a->mode != B200SMPL_MODE_FP32_SIMT && saved == nullptr && nb >= 512;
     if (fused) {
-      rc = launch_blend_lbs_fwd(d, fwd_gemm_mode(a->mode), feat, S, Sw, vpT, A_T, b0, nb, a->transl,
-                                a->vertices, saved != nullptr, m->num_sms, st);
+      rc = launch_blend_lbs_fwd(d, fwd_gemm_mode(a->mode), feat, S, Sw, vpT, A_T, b0, nb, a->transl, a->vertices,
+                                m->num_sms, st);
     } else if (a->mode == B200SMPL_MODE_FP32_SIMT) {
       rc = launch_blend_fwd_simt(d, featf, S, Sw, vpT, row_begin, d.n_pad, st);
     } else {
-      rc = launch_blend_fwd_umma(d, fwd_gemm_mode(a->mode), feat, S, Sw, vpT, row_begin, d.n_pad, st);
+      rc = launch_blend_fwd_umma(d, fwd_gemm_mode(a->mode), feat, S, Sw, vpT, row_begin, d.n_pad, m->num_sms, st);
     }
     if (rc) return rc;
     if (a->vertices && !fused)
@@ -414,7 +406,7 @@ int b200smpl_backward(const b200smpl_model* m, const b200smpl_backward_args* a, 
   int k_splits = 1;
   if (a->mode != B200SMPL_MODE_FP32_SIMT) {
     const int slabs = (row_end + 63) / 64 - row_begin / 64;
-    k_splits = std::max(1, std::min(p.k_splits, slabs / min_slabs_per_split()));
+    k_splits = std::max(1, std::min(p.k_splits, slabs / MIN_SLABS_PER_SPLIT));
   }
   const char* saved = nullptr;
   if (a->saved) {
@@ -435,7 +427,7 @@ int b200smpl_backward(const b200smpl_model* m, const b200smpl_backward_args* a, 
       if (a->mode == B200SMPL_MODE_FP32_SIMT)
         rc = launch_blend_fwd_simt(d, featf, S, Sw, vpT, row_begin, d.n_pad, st);
       else
-        rc = launch_blend_fwd_umma(d, fwd_gemm_mode(a->mode), feat, S, Sw, vpT, row_begin, d.n_pad, st);
+        rc = launch_blend_fwd_umma(d, fwd_gemm_mode(a->mode), feat, S, Sw, vpT, row_begin, d.n_pad, m->num_sms, st);
       if (rc) return rc;
     }
     {  // the gradient GEMM reads whole 64-row K slabs: rows between row_end and the slab boundary must be finite
@@ -446,40 +438,18 @@ int b200smpl_backward(const b200smpl_model* m, const b200smpl_backward_args* a, 
         if (dvp_lo) B200_CUDA_TRY(cudaMemset2DAsync(dvp_lo + c0 * 1024, pitch, 0, width, (size_t)Sw / 128, st));
       }
     }
-    int n_parts = k_splits;
-    if (have_v && fused_bwd_usable(d, a->mode, a->grad_vertices)) {
-      // vertex rows: skinning backward + gradient GEMM in one kernel (dv_posed stays in tensor memory); the virtual
-      // (joint) rows go through joints_bwd and their own small GEMM into the partials behind
-      const int nfp = fused_bwd_parts(d, Sw, m->num_sms);
-      if (nfp < 0) return fail(B200SMPL_ERR_INVALID, "slab too wide for the fused backward work list");
-      B200_CUDA_TRY(cudaMemsetAsync(dfeat_part, 0, (size_t)nfp * S * d.fl.nf_pad * 4, st));
-      if ((rc = launch_lbs_bwd_gemm(d, bmode, vpT, S, Sw, A_T, b0, nb, a->grad_vertices, dA_part, dtr_part, dfeat_part,
-                                    m->num_sms, st)))
+    if (have_v)
+      if ((rc = launch_lbs_bwd(d, vpT, S, Sw, A_T, b0, nb, a->grad_vertices, dvp_hi, dvp_lo, dA_part, dtr_part,
+                               m->num_sms, st)))
         return rc;
-      n_parts = nfp;
-      if (have_j) {
-        if ((rc = launch_joints_bwd(d, vpT, S, Sw, A_T, b0, nb, dJ, dvp_hi, dvp_lo, dA_part, dtr_part, false, st))) return rc;
-        const int vslabs = (row_end + 63) / 64 - d.n_virt0 / 64;
-        const int ksv = std::max(1, std::min(p.k_splits, vslabs / min_slabs_per_split()));
-        if ((rc = launch_blend_bwd_umma(d, bmode, dvp_hi, dvp_lo, S, Sw, dfeat_part + (size_t)nfp * S * d.fl.nf_pad, ksv,
-                                        d.n_virt0, row_end, st)))
-          return rc;
-        n_parts += ksv;
-      }
-    } else {
-      if (have_v)
-        if ((rc = launch_lbs_bwd(d, vpT, S, Sw, A_T, b0, nb, a->grad_vertices, dvp_hi, dvp_lo, dA_part, dtr_part,
-                                 m->num_sms, st)))
-          return rc;
-      if (have_j)
-        if ((rc = launch_joints_bwd(d, vpT, S, Sw, A_T, b0, nb, dJ, dvp_hi, dvp_lo, dA_part, dtr_part, have_v, st))) return rc;
-      if (a->mode == B200SMPL_MODE_FP32_SIMT)
-        rc = launch_blend_bwd_simt(d, dvp_hi, dvp_lo, S, Sw, dfeat_part, row_begin, row_end, st);
-      else
-        rc = launch_blend_bwd_umma(d, bmode, dvp_hi, dvp_lo, S, Sw, dfeat_part, k_splits, row_begin, row_end, st);
-      if (rc) return rc;
-    }
-    if ((rc = launch_pose_bwd(d, a->betas, a->pose, aa, b0, nb, S, A_T, dA_part, 1, dtr_part, dfeat_part, n_parts,
+    if (have_j)
+      if ((rc = launch_joints_bwd(d, vpT, S, Sw, A_T, b0, nb, dJ, dvp_hi, dvp_lo, dA_part, dtr_part, have_v, st))) return rc;
+    if (a->mode == B200SMPL_MODE_FP32_SIMT)
+      rc = launch_blend_bwd_simt(d, dvp_hi, dvp_lo, S, Sw, dfeat_part, row_begin, row_end, st);
+    else
+      rc = launch_blend_bwd_umma(d, bmode, dvp_hi, dvp_lo, S, Sw, dfeat_part, k_splits, row_begin, row_end, st);
+    if (rc) return rc;
+    if ((rc = launch_pose_bwd(d, a->betas, a->pose, aa, b0, nb, S, A_T, dA_part, 1, dtr_part, dfeat_part, k_splits,
                               have_j ? dJ : nullptr, a->grad_betas, a->grad_pose, a->grad_transl, st)))
       return rc;
   }

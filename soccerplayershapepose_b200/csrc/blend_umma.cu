@@ -327,207 +327,17 @@ constexpr int WS_MAX_SLABS = 9;        // resident slabs: constants+shape, 4 x h
 constexpr int WS_BN = 128;
 
 // ---------------------------------------------------------------------------------------------
-// Forward blend GEMM on a CTA PAIR (cta_group::2): the pair owns 256 consecutive model rows -- each CTA keeps
-// ITS 128 rows (all 9 K slabs) resident, the pair's tensor cores read both halves (N = 256) -- and walks pairs
-// of body tiles: each CTA streams the feature tiles of ITS 128 bodies and accumulates 128 bodies x 256 rows in
-// its own TMEM (2 x 256 columns).  Per SM and K step that is 8 KB of operand reads for 128 x 256 x 16 MACs
-// instead of 8 KB for 128 x 128 x 16: the shared-memory operand bandwidth that bounds the single-CTA kernel is
-// halved.  Only the leader issues MMAs; the peer relays its "stage landed" / "model slice landed" /
-// "accumulator drained" events to the leader's barriers with remote arrives.
-// ---------------------------------------------------------------------------------------------
-template <int DUMMY>
-__global__ void __launch_bounds__(GEMM_THREADS, 1)
-blend_fwd_ws2_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUtensorMap map_f, int pslabs,
-                     int ksteps_cs, int ksteps_p, int use_lo, int row0, int mtiles, int ntiles_n, int pairs_per_chunk,
-                     float4* __restrict__ vpB, int nc4) {
-  constexpr int SLAB = BM * BK * 2;
-  constexpr int KS = BK / UMMA_K;
-  constexpr uint32_t TMEM_COLS = 512;
-  const int nslab_f = 1 + 2 * pslabs;
-  const int nslab_w = 1 + (use_lo ? 2 : 1) * pslabs;
-  extern __shared__ unsigned char smem_dyn[];
-  unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~(uintptr_t)1023);
-  unsigned char* w_s = smem;                                          // [nslab_w][16 KB] this CTA's 128 model rows
-  unsigned char* f_s = smem + WS_MAX_SLABS * SLAB;                    // [WS_STAGES][16 KB] this CTA's body tile
-  uint64_t* bars = reinterpret_cast<uint64_t*>(f_s + WS_STAGES * SLAB);
-  uint64_t* w_full = bars;
-  uint64_t* peer_w_full = bars + 1;
-  uint64_t* full_bar = bars + 2;
-  uint64_t* peer_full_bar = full_bar + WS_STAGES;
-  uint64_t* empty_bar = peer_full_bar + WS_STAGES;
-  uint64_t* tfull_bar = empty_bar + WS_STAGES;      // [2]
-  uint64_t* tempty_bar = tfull_bar + 2;             // [2] (leader's are the ones waited on: 8 arrivals)
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty_bar + 2);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const int tile0 = (int)(blockIdx.x & ~1u);                          // first model-row tile of the pair
-  const int m0 = row0 + min((int)blockIdx.x, mtiles - 1) * BM;        // this CTA's rows (clamped for the relay-only CTA)
-  const int m0pair = row0 + tile0 * BM;
-  const bool live_lo = tile0 < mtiles, live_hi = tile0 + 1 < mtiles;
-  const int ntp_total = (ntiles_n + 1) / 2;
-  const int ntp_begin = blockIdx.y * pairs_per_chunk;
-  const int ntp_end = min(ntp_total, ntp_begin + pairs_per_chunk);
-
-  if (warp == 0 && lane == 0) {
-    prefetch_tmap(&map_w);
-    prefetch_tmap(&map_f);
-  }
-  if (warp == 1 && lane == 0) {
-    mbar_init(w_full, 1);
-    mbar_init(peer_w_full, 1);
-    for (int i = 0; i < WS_STAGES; ++i) {
-      mbar_init(&full_bar[i], 1);
-      mbar_init(&peer_full_bar[i], 1);
-      mbar_init(&empty_bar[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&tfull_bar[i], 1);
-      mbar_init(&tempty_bar[i], 8);                 // four epilogue warps of each CTA of the pair
-    }
-    fence_barrier_init();
-  }
-  if (warp == 1) {
-    __syncwarp();
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    // ===== TMA producer (both CTAs): own model rows once, then own body tile of every tile pair =====
-    if (elect_one()) {
-      mbar_arrive_expect_tx(w_full, (uint32_t)nslab_w * SLAB);
-      for (int s = 0; s < nslab_w; ++s) tma_load_2d(w_s + s * SLAB, &map_w, w_full, s * BK, m0);
-    }
-    __syncwarp();
-    int stage = 0;
-    uint32_t phase = 0;
-    for (int ntp = ntp_begin; ntp < ntp_end; ++ntp)
-      for (int s = 0; s < nslab_f; ++s) {
-        mbar_wait(&empty_bar[stage], phase ^ 1);
-        if (elect_one()) {
-          mbar_arrive_expect_tx(&full_bar[stage], SLAB);
-          // rows beyond the slab (odd number of body tiles) are zero-filled by the TMA unit
-          tma_load_2d(f_s + stage * SLAB, &map_f, &full_bar[stage], s * BK, (ntp * 2 + (int)rank) * WS_BN);
-        }
-        __syncwarp();
-        if (++stage == WS_STAGES) { stage = 0; phase ^= 1; }
-      }
-  } else if (warp == 1) {
-    int stage = 0;
-    uint32_t phase = 0;
-    if (rank == 0) {
-      // ===== leader: MMA issuer of the pair =====
-      constexpr uint32_t idesc = make_idesc(2 * BM, 2 * WS_BN);
-      mbar_wait(w_full, 0);
-      mbar_wait(peer_w_full, 0);
-      uint32_t tph0 = 0, tph1 = 0;
-      int acc = 0;
-      for (int ntp = ntp_begin; ntp < ntp_end; ++ntp, acc ^= 1) {
-        const uint32_t tph = acc ? tph1 : tph0;
-        mbar_wait(&tempty_bar[acc], tph ^ 1);           // both CTAs' epilogues have drained this accumulator
-        if (acc) tph1 ^= 1; else tph0 ^= 1;
-        tc_fence_after();
-        const uint32_t d_tmem = tmem_base + (uint32_t)(acc * 2 * WS_BN);
-        int j = 0;
-        for (int s = 0; s < nslab_f; ++s) {
-          mbar_wait(&full_bar[stage], phase);
-          mbar_wait(&peer_full_bar[stage], phase);
-          tc_fence_after();
-          const uint64_t da = make_sw128_desc(smem_u32(f_s + stage * SLAB));
-          int ks = ksteps_cs, w0 = 0, w1 = -1;
-          if (s > 0) {
-            ks = min(KS, ksteps_p - j * KS);
-            w0 = 1 + j;
-            if (s <= pslabs && use_lo) w1 = 1 + pslabs + j;
-            if (++j == pslabs) j = 0;
-          }
-          const uint64_t db0 = make_sw128_desc(smem_u32(w_s + w0 * SLAB));
-          const uint64_t db1 = make_sw128_desc(smem_u32(w_s + max(w1, 0) * SLAB));
-          if (elect_one()) {
-#pragma unroll
-            for (int k = 0; k < KS; ++k)
-              if (k < ks) umma_bf16_2cta(d_tmem, da + 2 * k, db0 + 2 * k, idesc, (s | k) != 0);
-            if (w1 >= 0) {
-#pragma unroll
-              for (int k = 0; k < KS; ++k)
-                if (k < ks) umma_bf16_2cta(d_tmem, da + 2 * k, db1 + 2 * k, idesc, 1u);
-            }
-            umma_commit_2cta(&empty_bar[stage]);
-            if (s == nslab_f - 1) umma_commit_2cta(&tfull_bar[acc]);
-          }
-          __syncwarp();
-          if (++stage == WS_STAGES) { stage = 0; phase ^= 1; }
-        }
-      }
-    } else {
-      // ===== peer: relay "model slice landed" and every "stage landed" to the leader =====
-      mbar_wait(w_full, 0);
-      if (elect_one()) remote_arrive(peer_w_full, 0);
-      __syncwarp();
-      for (int ntp = ntp_begin; ntp < ntp_end; ++ntp)
-        for (int s = 0; s < nslab_f; ++s) {
-          mbar_wait(&full_bar[stage], phase);
-          if (elect_one()) remote_arrive(&peer_full_bar[stage], 0);
-          __syncwarp();
-          if (++stage == WS_STAGES) { stage = 0; phase ^= 1; }
-        }
-    }
-  } else {
-    // ===== epilogue (both CTAs): 128 bodies x 256 model rows of the pair per accumulator =====
-    const int q = warp & 3;
-    uint32_t tph0 = 0, tph1 = 0;
-    int acc = 0;
-    for (int ntp = ntp_begin; ntp < ntp_end; ++ntp, acc ^= 1) {
-      const uint32_t tph = acc ? tph1 : tph0;
-      mbar_wait(&tfull_bar[acc], tph);
-      if (acc) tph1 ^= 1; else tph0 ^= 1;
-      tc_fence_after();
-      const int btile = ntp * 2 + (int)rank;                         // this CTA's body tile
-      if (btile < ntiles_n) {
-        float4* colbase = vpB + ((size_t)(btile * 4 + q) * nc4 + (m0pair >> 2)) * 32 + lane;
-#pragma unroll 1
-        for (int c0 = 0; c0 < 2 * WS_BN; c0 += 32) {
-          if (c0 < WS_BN ? !live_lo : !live_hi) continue;
-          uint32_t v[32];
-          tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * 2 * WS_BN + c0), v);
-          float4* o = colbase + (size_t)(c0 >> 2) * 32;
-#pragma unroll
-          for (int i = 0; i < 8; ++i)
-            o[i * 32] = make_float4(__uint_as_float(v[4 * i]), __uint_as_float(v[4 * i + 1]),
-                                    __uint_as_float(v[4 * i + 2]), __uint_as_float(v[4 * i + 3]));
-        }
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) {
-        if (rank == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&tempty_bar[acc])) : "memory");
-        else remote_arrive(&tempty_bar[acc], 0);
-      }
-    }
-  }
-  tc_fence_before();
-  cluster_sync_all();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
-// Forward blend GEMM on a CTA pair, BODY-stationary: the pair owns one pair of body tiles (each CTA keeps the
-// feature slabs of ITS 128 bodies resident: 9 x 16 KB, loaded once) and walks a contiguous range of model-row
-// tile pairs, streaming ITS 128 rows of each model slab through the stage ring.  Same MMAs, same accumulator
-// layout and epilogue as blend_fwd_ws2_kernel; what changes is what is kept and what is streamed: with
-// 16 body-tile pairs x 4 row chunks the whole GEMM is ONE wave of 64 clusters with ~22 tiles each, so the
-// prologue (resident load, pipeline fill) and the drain (last tile's MMAs + epilogue) are paid once per cluster
-// instead of once per 4 tiles (measured with clock64 counters in the MMA warp: 8-9 k of 35 k cycles waiting for
-// the resident slice, another 12 k refilling the ring, ~10 k draining).
+// Forward blend GEMM on a CTA PAIR (cta_group::2), BODY-stationary: the pair owns one pair of body tiles (each CTA
+// keeps the feature slabs of ITS 128 bodies resident: 9 x 16 KB, loaded once) and walks a contiguous range of
+// model-row tile pairs, streaming ITS 128 rows of each model slab through the stage ring.  The pair's tensor cores
+// read both CTAs' rows (N = 256) and each CTA accumulates 128 bodies x 256 rows in its own TMEM (2 x 256 columns):
+// per SM and K step that is 8 KB of operand reads for 128 x 256 x 16 MACs instead of 8 KB for 128 x 128 x 16, half
+// the shared-memory operand bandwidth that bounds a single-CTA kernel.  Only the leader issues MMAs; the peer relays
+// its "stage landed" / "accumulator drained" events to the leader's barriers with remote arrives.  With 16 body-tile
+// pairs x 4 row chunks the whole GEMM is ONE wave of 64 clusters with ~22 tiles each, so the prologue (resident
+// load, pipeline fill) and the drain (last tile's MMAs + epilogue) are paid once per cluster instead of once per
+// 4 tiles (measured with clock64 counters in the MMA warp: 8-9 k of 35 k cycles waiting for the resident slice,
+// another 12 k refilling the ring, ~10 k draining).
 // ---------------------------------------------------------------------------------------------
 // work list of the body-stationary kernel: cluster c = body-tile pair bp[c], model-row tile pairs [w0[c], w1[c])
 
@@ -751,58 +561,6 @@ int make_map(CUtensorMap* map, const void* base, int k_extent, int rows, int pit
 
 constexpr int BWD_STAGES = 4;
 
-static int launch_blend_fwd_umma_2cta(const DevModel& m, int mode, const __nv_bfloat16* feat, int S, int Sw, float* vpT,
-                                      int row_begin, int row_end, cudaStream_t st) {
-  const int pslabs = m.fl.pseg / BK;
-  const int use_lo = (mode == B200SMPL_MODE_BF16) ? 0 : 1;
-  if (1 + 2 * pslabs > WS_MAX_SLABS) return fail(B200SMPL_ERR_INVALID, "feature pitch too large for the resident operand");
-  CUtensorMap map_w, map_f;
-  int rc;
-  if ((rc = make_map(&map_w, m.Wf, m.fl.pitch, m.n_pad, m.fl.pitch, BM))) return rc;
-  if ((rc = make_map(&map_f, feat, m.fl.pitch, Sw, m.fl.pitch, WS_BN))) return rc;   // rows >= Sw read as zero
-  constexpr int smem = (WS_MAX_SLABS + WS_STAGES) * BM * BK * 2 + 1024 + 256;
-  auto kern = blend_fwd_ws2_kernel<0>;
-  B200_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  const int mtiles = (row_end - row_begin) / BM;
-  const int gx = round_up(mtiles, 2);
-  const int ntiles_n = Sw / WS_BN;
-  const int ntp_total = (ntiles_n + 1) / 2;
-  // chunks of body-tile pairs: CTA pairs are scheduled per TPC (74 per wave); at least 2 pairs per cluster to
-  // amortise the resident-slice load
-  int chunks = 1;
-  {
-    double best = -1.0;
-    for (int c = 1; c <= ntp_total; ++c) {
-      const int ppc = (ntp_total + c - 1) / c;
-      if (ppc < 2 && c > 1) break;
-      const long long clusters = (long long)(gx / 2) * ((ntp_total + ppc - 1) / ppc);
-      const long long waves = (clusters + 73) / 74;
-      const double eff = (double)clusters / (double)(waves * 74);
-      if (eff > best + 1e-9) { best = eff; chunks = (ntp_total + ppc - 1) / ppc; }
-    }
-  }
-  const int ppc = (ntp_total + chunks - 1) / chunks;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(gx, (ntp_total + ppc - 1) / ppc, 1);
-  cfg.blockDim = dim3(GEMM_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  LaunchTimer _timer("blend_fwd_umma", st);
-  B200_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, map_w, map_f, pslabs, (m.fl.k_cs + UMMA_K - 1) / UMMA_K,
-                                   (NPOSE + UMMA_K - 1) / UMMA_K, use_lo, row_begin, mtiles, ntiles_n, ppc,
-                                   reinterpret_cast<float4*>(vpT), m.n_pad / 4));
-  B200_LAUNCH_CHECK("blend_fwd_umma");
-  return 0;
-}
-
 // Work list of the body-stationary forward GEMM (host side; pure arithmetic, also exposed to the CPU tests through
 // b200smpl_debug_fwd_gemm_worklist).  CTA pairs are scheduled per TPC (2 SMs).  The (body pair, row-tile pair) list,
 // body pair major, is cut into one equal range per TPC; a range that crosses into the next body pair becomes two
@@ -846,9 +604,10 @@ int build_bs_work(int bp_total, int wtp_total, int tpcs, BsWork& work) {
   return npieces;
 }
 
-// body-stationary CTA-pair launch: one wave of (body-tile pair) x (row chunk) clusters
-static int launch_blend_fwd_umma_bs2(const DevModel& m, int mode, const __nv_bfloat16* feat, int S, int Sw, float* vpT,
-                                     int row_begin, int row_end, int num_sms, cudaStream_t st) {
+// body-stationary CTA-pair launch: one wave of (body-tile pair) x (row chunk) clusters.  Slabs are at most MAX_SLAB
+// bodies wide (make_plan), which the work list always fits.
+int launch_blend_fwd_umma(const DevModel& m, int mode, const __nv_bfloat16* feat, int S, int Sw, float* vpT,
+                          int row_begin, int row_end, int num_sms, cudaStream_t st) {
   const int pslabs = m.fl.pseg / BK;
   const int use_lo = (mode == B200SMPL_MODE_BF16) ? 0 : 1;
   if (1 + 2 * pslabs > WS_MAX_SLABS) return fail(B200SMPL_ERR_INVALID, "feature pitch too large for the resident operand");
@@ -889,21 +648,6 @@ static int launch_blend_fwd_umma_bs2(const DevModel& m, int mode, const __nv_bfl
   return 0;
 }
 
-int launch_blend_fwd_umma(const DevModel& m, int mode, const __nv_bfloat16* feat, int S, int Sw, float* vpT,
-                          int row_begin, int row_end, cudaStream_t st) {
-  // B200_FWD_2CTA: 2 (default) body-stationary CTA pairs; 1 model-row-stationary CTA pairs (also the fall-back for
-  // slabs wider than the body-stationary work list)
-  static const int sel = getenv("B200_FWD_2CTA") == nullptr ? 2 : atoi(getenv("B200_FWD_2CTA"));
-  if (sel >= 2 && (Sw / WS_BN + 1) / 2 <= BS_MAX_WORK) {     // wider slabs than 160 body-tile pairs: row-stationary kernel
-    int dev = 0, sms = 148;
-    B200_CUDA_TRY(cudaGetDevice(&dev));
-    B200_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    return launch_blend_fwd_umma_bs2(m, mode, feat, S, Sw, vpT, row_begin, row_end, sms, st);
-  }
-  (void)sel;
-  return launch_blend_fwd_umma_2cta(m, mode, feat, S, Sw, vpT, row_begin, row_end, st);   // model-row-stationary pairs
-}
-
 }  // namespace b200smpl
 extern "C" int b200smpl_debug_fwd_gemm_worklist(int body_tiles, int row_tiles, int num_sms, uint16_t* out, int capacity) {
   using namespace b200smpl;
@@ -916,18 +660,12 @@ extern "C" int b200smpl_debug_fwd_gemm_worklist(int body_tiles, int row_tiles, i
 namespace b200smpl {
 
 // number of split-K partials the backward GEMM writes for slab width S
-// CTA-pair kernels are the default; B200_BWD_2CTA=0 selects the single-CTA kernel (kept for comparison)
-static bool bwd_use_2cta() {
-  static const bool v = getenv("B200_BWD_2CTA") == nullptr || atoi(getenv("B200_BWD_2CTA")) != 0;
-  return v;
-}
-
 int blend_bwd_umma_splits(const DevModel& m, int mode, int S, int num_sms) {
   (void)mode;
   const int mtiles = (S + BM - 1) / BM;
   const int slabs = (m.n_rows + BK - 1) / BK;
   // CTA pairs are scheduled per TPC (2 SMs): never more pairs than TPCs, or a second, nearly empty wave runs
-  int want = bwd_use_2cta() ? std::max(1, num_sms / mtiles) : (num_sms + mtiles - 1) / mtiles;
+  int want = std::max(1, num_sms / mtiles);
   want = std::max(1, std::min(want, slabs / 8));
   return want;
 }
@@ -1004,12 +742,13 @@ int launch_blend_bwd_umma(const DevModel& m, int mode, const __nv_bfloat16* dvp_
   }
   const int slab_begin = row_begin / BK, slab_end = (row_end + BK - 1) / BK;
   const long long split_stride = (long long)S * nf_pad;
-  if (bwd_use_2cta() && nf_pad == 224 && (Sw / BM) % 2 == 0)
+  // CTA pairs where the body tiles pair up; the single-CTA kernel takes an odd number of tiles and nf_pad = 208
+  // (1 beta).  nf_pad <= round_up(MAX_BETAS + NPOSE, 16) = 224.
+  if (nf_pad == 224 && (Sw / BM) % 2 == 0)
     return launch_bwd_bn_2cta<224>(ops, m, nseg, row_end, slab_begin, slab_end, nsplit, Sw, dfeat_part, nf_pad, split_stride, st);
   switch (nf_pad) {
     case 224: return launch_bwd_bn<224>(ops, nseg, m.n_pad / 8, slab_begin, slab_end, nsplit, Sw, dfeat_part, nf_pad, split_stride, st);
     case 208: return launch_bwd_bn<208>(ops, nseg, m.n_pad / 8, slab_begin, slab_end, nsplit, Sw, dfeat_part, nf_pad, split_stride, st);
-    case 240: return launch_bwd_bn<240>(ops, nseg, m.n_pad / 8, slab_begin, slab_end, nsplit, Sw, dfeat_part, nf_pad, split_stride, st);
     default: return fail(B200SMPL_ERR_INVALID, "unsupported num_betas for the tensor-core backward (nf_pad=" + std::to_string(nf_pad) + ")");
   }
 }

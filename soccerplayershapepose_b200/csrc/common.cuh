@@ -94,11 +94,6 @@ struct DevModel {
   const __nv_bfloat16* Wf;     // [n_pad][fl.pitch]         forward operand, K-major
   const __nv_bfloat16* Wb_hi;  // [fl.nf_pad][n_pad]        backward operand (K = n), hi part
   const __nv_bfloat16* Wb_lo;  // [fl.nf_pad][n_pad]        lo part
-  // the same rows for the fused skinning-backward + gradient GEMM (fused_bwd.cu): per CTA half (nf_pad / 2 features)
-  // and 16-vertex item (48 rows) one contiguous block [6 chunks of 8 rows][nf_pad / 2][8] = the no-swizzle K-major
-  // core-matrix layout of the MMA's B operand, so a stage is one plain bulk copy
-  const __nv_bfloat16* Wbi_hi; // [2][ntiles * 2][6][nf_pad / 2][8]
-  const __nv_bfloat16* Wbi_lo;
   const float* W32;            // [1 + nf][n_pad]           fp32 rows: template, shapedirs, posedirs
   const uint32_t* vmeta;       // [ntiles*32]
   const float4* vwts;          // [ntiles*32]
@@ -116,7 +111,7 @@ struct DevModel {
 };
 
 struct HostArrays {
-  std::vector<__nv_bfloat16> Wf, Wb_hi, Wb_lo, Wbi_hi, Wbi_lo;
+  std::vector<__nv_bfloat16> Wf, Wb_hi, Wb_lo;
   std::vector<float> W32, Jt, Jsd, term_c;
   std::vector<uint32_t> vmeta;
   std::vector<float> vwts;     // 4 per vertex
@@ -242,24 +237,15 @@ int launch_blend_fwd_simt(const DevModel& m, const float* featf, int S, int Sw, 
 int launch_blend_bwd_simt(const DevModel& m, const __nv_bfloat16* dvp_hi, const __nv_bfloat16* dvp_lo, int S, int Sw,
                           float* dfeat, int row_begin, int row_end, cudaStream_t st);
 int launch_blend_fwd_umma(const DevModel& m, int mode, const __nv_bfloat16* feat, int S, int Sw, float* vpT,
-                          int row_begin, int row_end, cudaStream_t st);
+                          int row_begin, int row_end, int num_sms, cudaStream_t st);
 int launch_blend_bwd_umma(const DevModel& m, int mode, const __nv_bfloat16* dvp_hi, const __nv_bfloat16* dvp_lo,
                           int S, int Sw, float* dfeat_part, int nsplit, int row_begin, int row_end,
                           cudaStream_t st);
 int blend_bwd_umma_splits(const DevModel& m, int mode, int S, int num_sms);
-// skinning backward producing the gradient GEMM's operand in tensor memory (fused_bwd.cu); opt-in with
-// B200_FUSED_BWD=1 (default: lbs_bwd + gradient GEMM, which is faster today).  dfeat_part receives fused_bwd_parts() partials [part][S][nf_pad] (unused ones zero).
-bool fused_bwd_usable(const DevModel& m, int mode, const float* grad_verts);
-int fused_bwd_parts(const DevModel& m, int Sw, int num_sms);
-int launch_lbs_bwd_gemm(const DevModel& m, int mode, const float* vpB, int S, int Sw, const float* A_blk, int b0, int nb,
-                        const float* grad_verts, float* dA_acc, float* dtr_acc, float* dfeat_part, int num_sms,
-                        cudaStream_t st);
-// blend GEMM with the skinning in its epilogue (fused_fwd.cu).  B200_FUSED_FWD: 0 never, 1 (default) forward-only
-// calls, 2 also when the forward products are kept
-int fused_fwd_mode();
+// blend GEMM with the skinning in its epilogue (fused_fwd.cu); forward-only calls
 int launch_blend_lbs_fwd(const DevModel& m, int mode, const __nv_bfloat16* feat, int S, int Sw, float* vpT,
-                         const float* A_blk, int b0, int nb, const float* transl, float* verts, int write_vp,
-                         int num_sms, cudaStream_t st);
+                         const float* A_blk, int b0, int nb, const float* transl, float* verts, int num_sms,
+                         cudaStream_t st);
 
 int launch_lbs_fwd(const DevModel& m, const float* vpT, int S, const float* A_T, int b0, int nb,
                    const float* transl, float* verts, int num_sms, cudaStream_t st);

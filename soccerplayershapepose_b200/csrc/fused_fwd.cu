@@ -1,8 +1,9 @@
 // Fused forward: blend GEMM (SURVEY.md section 8 rows a4 + a7) with the linear blend skinning (row a9) in its
 // epilogue, so that v_posed never makes the HBM round trip between the two.  Used for forward-only calls (no
-// products kept for a backward): 188 us against 108 + 136 us of blend GEMM + skinning kernel at B = 4096; when
-// v_posed must also be written for the backward the kernel stores 658 MB without reading anything and runs at the
-// speed of the two kernels (242 us), so those calls keep the two kernels (see DESIGN.md, "fused forward").
+// products kept for a backward): 188 us against 108 + 136 us of blend GEMM + skinning kernel at B = 4096.  A call
+// that keeps the products needs v_posed in HBM; writing it from this kernel as well stored 658 MB without reading
+// anything and ran at the speed of the two kernels (242 us), so those calls run the two kernels (see DESIGN.md,
+// "fused forward").
 //
 // The GEMM is the body-stationary CTA-pair kernel of blend_umma.cu (tcgen05 cta_group::2, features resident in
 // shared memory, model slabs streamed by TMA) with two changes:
@@ -14,14 +15,13 @@
 //     accumulators leave.  A slot reload is three warp-uniform tcgen05.ld of 4 columns.
 // Epilogue warps (two per TMEM lane quadrant; each takes one half -- 16 vertices, 48 columns -- of every tile, so the
 // epilogue of tile t overlaps the MMAs of tile t + 1): thread = body reads its accumulator columns 24 at a time,
-// stores them to the group-blocked vpB when asked to, skins the 8 vertices with the packed-pair slot arithmetic of
-// lbs.cu and flushes them through a per-warp transposing tile as 96-byte row segments of the (B, V, 3) output.
-// Virtual (joint) row tiles are only stored.
+// skins the 8 vertices with the packed-pair slot arithmetic of lbs.cu and flushes them through a per-warp
+// transposing tile as 96-byte row segments of the (B, V, 3) output.
+// Virtual (joint) row tiles are only stored, to the group-blocked vpB.
 //
 // The variants that lost (three epilogue warps per quadrant on setmaxnreg registers, the half tile staged in 48
 // registers with the accumulator released at once, 192-byte row segments) are in the history (commit cf06df6) and in
-// profiles/r02_experiments.md section 8; what remains of the experiments are the B200_FF_DBG bits that leave parts of
-// the kernel out for timing.
+// profiles/r02_experiments.md section 8.
 #include <algorithm>
 
 #include "lbs_tiles.cuh"
@@ -32,10 +32,7 @@ namespace b200smpl {
 constexpr int FF_BN = 96;                           // model rows per tile = 32 vertices
 constexpr int FF_BNH = FF_BN / 2;                   // rows of a slab each CTA of the pair stages
 constexpr int FF_NW = 2;                            // epilogue warps per TMEM lane quadrant
-#ifndef B200_FF_STAGES
-#define B200_FF_STAGES 7
-#endif
-constexpr int FF_STAGES = B200_FF_STAGES;
+constexpr int FF_STAGES = 7;
 constexpr int FF_STAGE_BYTES = FF_BNH * BK * 2;     // 6 KB
 constexpr int FF_PS = (NPOSE + BK - 1) / BK;        // 64-wide K slabs of one pose segment (4)
 constexpr int FF_KSP = (NPOSE + UMMA_K - 1) / UMMA_K;   // K steps of one pose segment (13)
@@ -49,7 +46,7 @@ constexpr int FF_TR_COL = 2 * FF_BN;                // first TMEM column of the 
 constexpr int FF_WV = TILE_V / 2;                   // vertices of a half tile (one epilogue warp's unit of work)
 constexpr int FF_PLAN_WORDS = (FF_WV / 8) * 40;     // plan records of a half tile
 constexpr int FF_TILE_WORDS = ItemShape<FF_HV>::TILE_WORDS;
-constexpr int FF_NBARS = 2 + 3 * FF_STAGES + 4 + 2 * FF_EPI_WARPS;
+constexpr int FF_NBARS = 1 + 2 * FF_STAGES + 4 + 2 * FF_EPI_WARPS;
 constexpr size_t FF_SMEM = (size_t)FF_MAX_SLABS * FF_SLAB + (size_t)FF_STAGES * FF_STAGE_BYTES +
                            (size_t)FF_EPI_WARPS * (FF_TILE_WORDS + 2 * FF_PLAN_WORDS) * 4 + FF_NBARS * 8 + 16 +
                            1024 /*alignment slack*/;
@@ -57,12 +54,6 @@ static_assert(FF_SMEM <= 232448, "fused forward: shared memory budget");
 static_assert(FF_TR_COL + NJ * AELEMS <= 512, "fused forward: tensor memory budget");
 static_assert(NJ % FF_NW == 0, "joints split evenly over the warps of a quadrant");
 
-// timing experiments (kernel argument dbg): what is left out
-constexpr int FF_DBG_NO_MMA = 1, FF_DBG_NO_FLUSH = 2, FF_DBG_NO_SKIN = 4, FF_DBG_NO_RELOAD = 8, FF_DBG_NO_VP = 16;
-
-#ifndef B200_FF_TMA2SM
-#define B200_FF_TMA2SM 1
-#endif
 // TMA load of a CTA pair: the bytes land in THIS CTA's shared memory, the transaction count on the LEADER's
 // mbarrier (same offset, CTA rank bit of the shared::cluster address cleared), so the MMA issuer waits on one
 // barrier per stage and no warp has to relay the peer's "stage landed"
@@ -129,8 +120,7 @@ __device__ __forceinline__ void skin_fwd4_tm(Slots& s, uint32_t tr_base, const u
                                              uint32_t force, float tx, float ty, float tz, const float (&P)[12],
                                              float* row_out) {
   const uint4 m4 = *reinterpret_cast<const uint4*>(meta_s);
-  uint32_t mts[4] = {m4.x | force, m4.y, m4.z, m4.w};
-  if (force >> 31) { mts[0] &= ~(0xFu << 20); mts[1] &= ~(0xFu << 20); mts[2] &= ~(0xFu << 20); mts[3] &= ~(0xFu << 20); }   // timing experiment
+  const uint32_t mts[4] = {m4.x | force, m4.y, m4.z, m4.w};
   float4 ws[4];
 #pragma unroll
   for (int i = 0; i < 4; ++i) ws[i] = wts_s[i];
@@ -164,7 +154,7 @@ __device__ __forceinline__ void skin_fwd4_tm(Slots& s, uint32_t tr_base, const u
 }
 
 // grid: 2 x (clusters of the work list), cluster = CTA pair.  Row tiles are counted from model row 0.
-//   vpB     group-blocked blend output (skin_common.cuh); written for vertex tiles only when write_vp
+//   vpB     group-blocked blend output (skin_common.cuh); written for the virtual (joint) row tiles only
 //   n_vtiles  vertex tiles (m.ntiles): row tiles below it are skinned into verts, the others only stored
 template <bool USE_LO>
 __global__ void __launch_bounds__(FF_THREADS, 1)
@@ -172,8 +162,7 @@ blend_lbs_fwd_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_con
                      int ksteps_cs, int n_pad, int ntiles_n,
                      const __grid_constant__ BsWork work, float4* __restrict__ vpB, int nc4,
                      const float4* __restrict__ A_blk, int b0, int nb, const float* __restrict__ transl,
-                     float* __restrict__ verts, int V, int n_vtiles, int vec_ok, const uint32_t* __restrict__ vplan,
-                     int write_vp, int dbg) {
+                     float* __restrict__ verts, int V, int n_vtiles, int vec_ok, const uint32_t* __restrict__ vplan) {
   constexpr int KS = BK / UMMA_K;
   constexpr uint32_t TMEM_COLS = 512;
   using SH = ItemShape<FF_HV>;
@@ -190,10 +179,8 @@ blend_lbs_fwd_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_con
   uint32_t* stashes = reinterpret_cast<uint32_t*>(tiles + FF_EPI_WARPS * FF_TILE_WORDS);   // [8][2][160] plan records
   uint64_t* bars = reinterpret_cast<uint64_t*>(stashes + FF_EPI_WARPS * 2 * FF_PLAN_WORDS);
   uint64_t* f_full = bars;
-  uint64_t* peer_f_full = bars + 1;
-  uint64_t* full_bar = bars + 2;
-  uint64_t* peer_full_bar = full_bar + FF_STAGES;
-  uint64_t* empty_bar = peer_full_bar + FF_STAGES;
+  uint64_t* full_bar = bars + 1;
+  uint64_t* empty_bar = full_bar + FF_STAGES;
   uint64_t* tfull_bar = empty_bar + FF_STAGES;      // [2]
   uint64_t* tempty_bar = tfull_bar + 2;             // [2] (the leader's are waited on: 8 arrivals)
   uint64_t* wbars = tempty_bar + 2;                 // [8][2] plan records landed
@@ -211,10 +198,8 @@ blend_lbs_fwd_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_con
   }
   if (warp == 1 && lane == 0) {
     mbar_init(f_full, 1);
-    mbar_init(peer_f_full, 1);
     for (int i = 0; i < FF_STAGES; ++i) {
       mbar_init(&full_bar[i], 1);
-      mbar_init(&peer_full_bar[i], 1);
       mbar_init(&empty_bar[i], 1);
     }
     for (int i = 0; i < 2; ++i) {
@@ -243,14 +228,8 @@ blend_lbs_fwd_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_con
     // ===== TMA producer (both CTAs): own body tile once, then own half of every model slab of every row tile =====
     const uint64_t pol_keep = l2_policy_evict_last();       // the model slabs are re-read by every body pair
     if (elect_one()) {
-#if B200_FF_TMA2SM
       if (rank == 0) mbar_arrive_expect_tx(f_full, 2u * (uint32_t)nslab_f * FF_SLAB);   // both CTAs' bytes count here
       for (int s = 0; s < nslab_f; ++s) tma_load_2d_pair(f_s + s * FF_SLAB, &map_f, f_full, s * BK, btile * BM, l2_policy_evict_first());
-#else
-      mbar_arrive_expect_tx(f_full, (uint32_t)nslab_f * FF_SLAB);
-      // rows beyond the slab (odd number of body tiles) are zero-filled by the TMA unit
-      for (int s = 0; s < nslab_f; ++s) tma_load_2d(f_s + s * FF_SLAB, &map_f, f_full, s * BK, btile * BM);
-#endif
     }
     __syncwarp();
     int stage = 0;
@@ -259,15 +238,8 @@ blend_lbs_fwd_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_con
       for (int s = 0; s < nslab_w; ++s) {
         mbar_wait(&empty_bar[stage], phase ^ 1);
         if (elect_one()) {
-#if B200_FF_TMA2SM
           if (rank == 0) mbar_arrive_expect_tx(&full_bar[stage], 2 * FF_STAGE_BYTES);
           tma_load_2d_pair(w_s + stage * FF_STAGE_BYTES, &map_w, &full_bar[stage], s * BK, wt * FF_BN + (int)rank * FF_BNH, pol_keep);
-#else
-          mbar_arrive_expect_tx(&full_bar[stage], FF_STAGE_BYTES);
-          // rows beyond the model are zero-filled by the TMA unit
-          tma_load_2d_hint(w_s + stage * FF_STAGE_BYTES, &map_w, &full_bar[stage], s * BK, wt * FF_BN + (int)rank * FF_BNH,
-                           pol_keep);
-#endif
         }
         __syncwarp();
         if (++stage == FF_STAGES) { stage = 0; phase ^= 1; }
@@ -281,7 +253,6 @@ blend_lbs_fwd_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_con
       // division / descriptor rebuild; it was ~1000 cycles per slab with the schedule computed at run time) =====
       constexpr uint32_t idesc = make_idesc(2 * BM, FF_BN);
       mbar_wait(f_full, 0);
-      if (!B200_FF_TMA2SM) mbar_wait(peer_f_full, 0);
       const uint64_t da_base = make_sw128_desc(smem_u32(f_s));
       const uint64_t db_base = make_sw128_desc(smem_u32(w_s));
       uint32_t tph0 = 0, tph1 = 0;
@@ -289,19 +260,18 @@ blend_lbs_fwd_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_con
       // one model slab against one or two resident feature slabs; `first`: the tile's first MMA overwrites
       auto slab = [&](uint32_t d_tmem, int ks, int f0, int f1, bool first, uint64_t* tfull) {
         mbar_wait(&full_bar[stage], phase);
-        if (!B200_FF_TMA2SM) mbar_wait(&peer_full_bar[stage], phase);
         tc_fence_after();
         const uint64_t db = db_base + (uint64_t)(stage * (FF_STAGE_BYTES >> 4));
         if (elect_one()) {
           const uint64_t da0 = da_base + (uint64_t)(f0 * (FF_SLAB >> 4));
 #pragma unroll
           for (int k = 0; k < KS; ++k)
-            if (k < ks && !(dbg & FF_DBG_NO_MMA)) umma_bf16_2cta(d_tmem, da0 + 2 * k, db + 2 * k, idesc, (first && k == 0) ? 0u : 1u);
+            if (k < ks) umma_bf16_2cta(d_tmem, da0 + 2 * k, db + 2 * k, idesc, (first && k == 0) ? 0u : 1u);
           if (f1 >= 0) {
             const uint64_t da1 = da_base + (uint64_t)(f1 * (FF_SLAB >> 4));
 #pragma unroll
             for (int k = 0; k < KS; ++k)
-              if (k < ks && !(dbg & FF_DBG_NO_MMA)) umma_bf16_2cta(d_tmem, da1 + 2 * k, db + 2 * k, idesc, 1u);
+              if (k < ks) umma_bf16_2cta(d_tmem, da1 + 2 * k, db + 2 * k, idesc, 1u);
           }
           umma_commit_2cta(&empty_bar[stage]);
           if (tfull != nullptr) umma_commit_2cta(tfull);
@@ -328,18 +298,6 @@ blend_lbs_fwd_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_con
             slab(d_tmem, min(KS, FF_KSP - j * KS), 1 + j, -1, false, j == PS - 1 ? &tfull_bar[acc] : nullptr);
         }
       }
-    } else if (!B200_FF_TMA2SM) {
-      // ===== peer: relay "body tile landed" and every "stage landed" to the leader =====
-      mbar_wait(f_full, 0);
-      if (elect_one()) remote_arrive(peer_f_full, 0);
-      __syncwarp();
-      for (int wt = wt_begin; wt < wt_end; ++wt)
-        for (int s = 0; s < nslab_w; ++s) {
-          mbar_wait(&full_bar[stage], phase);
-          if (elect_one()) remote_arrive(&peer_full_bar[stage], 0);
-          __syncwarp();
-          if (++stage == FF_STAGES) { stage = 0; phase ^= 1; }
-        }
     }
   }
   } else {
@@ -411,7 +369,6 @@ blend_lbs_fwd_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_con
       }
       const int row_w = wt * FF_BN + half * (FF_BN / 2);                // first blend row of this half tile
       const uint32_t acc_base = lane_base + (uint32_t)(acc * FF_BN + half * (FF_BN / 2));
-      float4* colbase = vpB + ((size_t)g * nc4 + (row_w >> 2)) * 32 + lane;
       if (skin && wt < n_vtiles) {
         const uint32_t b = n_plan & 1;
         if (is_vhalf(h + FF_NW) && lane == 0) issue_plan(b ^ 1, h + FF_NW);
@@ -422,26 +379,17 @@ blend_lbs_fwd_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_con
           uint32_t v[24];
           tmem_ld_24(acc_base + (uint32_t)(sub * 24), v);
           if (sub == FF_WV / FF_HV - 1) release(acc);                  // the MMAs of the tile after next may start
-          if (write_vp && !(dbg & FF_DBG_NO_VP)) {
 #pragma unroll
-            for (int i = 0; i < 6; ++i)
-              colbase[(size_t)(sub * 6 + i) * 32] = make_float4(__uint_as_float(v[4 * i]), __uint_as_float(v[4 * i + 1]),
-                                                                __uint_as_float(v[4 * i + 2]), __uint_as_float(v[4 * i + 3]));
-          }
-          if (!(dbg & FF_DBG_NO_SKIN)) {
+          for (int u = 0; u < FF_HV / 4; ++u) {
+            float P[12];
 #pragma unroll
-            for (int u = 0; u < FF_HV / 4; ++u) {
-              float P[12];
-#pragma unroll
-              for (int i = 0; i < 12; ++i)
-                P[i] = __uint_as_float(v[u * 12 + i]);
-              skin_fwd4_tm(sl, tr_base, plan_meta(st, sub * (FF_HV / 4) + u), plan_wts(st, sub * (FF_HV / 4) + u),
-                           ((sub == 0 && u == 0) ? (0xFu << 20) : 0u) | ((dbg & FF_DBG_NO_RELOAD) ? (1u << 31) : 0u), tx, ty, tz,
-                           P, my_row + u * 12);
-            }
+            for (int i = 0; i < 12; ++i)
+              P[i] = __uint_as_float(v[u * 12 + i]);
+            skin_fwd4_tm(sl, tr_base, plan_meta(st, sub * (FF_HV / 4) + u), plan_wts(st, sub * (FF_HV / 4) + u),
+                         (sub == 0 && u == 0) ? (0xFu << 20) : 0u, tx, ty, tz, P, my_row + u * 12);
           }
           __syncwarp();
-          if (!(dbg & FF_DBG_NO_FLUSH)) {
+          {
             const int vbase = wt * TILE_V + half * FF_WV + sub * FF_HV;
             const int ncols = max(0, min(FF_HV, V - vbase)) * 3;
             float* dst0 = v_g + (size_t)vbase * 3;
@@ -453,6 +401,7 @@ blend_lbs_fwd_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_con
         ++n_plan;
       } else {
         // virtual (joint) rows, or a call without a vertex output: store the blend rows only
+        float4* colbase = vpB + ((size_t)g * nc4 + (row_w >> 2)) * 32 + lane;
 #pragma unroll 1
         for (int c0 = 0; c0 < FF_BN / 2; c0 += 24) {
           uint32_t v[24];
@@ -477,21 +426,14 @@ blend_lbs_fwd_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_con
 }
 
 // ---- host side ------------------------------------------------------------------------------
-int fused_fwd_mode() {
-  static const int v = getenv("B200_FUSED_FWD") == nullptr ? 1 : atoi(getenv("B200_FUSED_FWD"));
-  return v;
-}
-
 // Sw = active slab width (multiple of 128).  Blends every row tile of the model (vertex rows and virtual joint rows)
-// for the slab; vertex tiles are skinned into verts when it is given.  vpB receives the virtual rows always and the
-// vertex rows when write_vp (the backward's operand).
+// for the slab; vertex tiles are skinned into verts when it is given.  vpB receives the virtual rows.
 int launch_blend_lbs_fwd(const DevModel& m, int mode, const __nv_bfloat16* feat, int S, int Sw, float* vpT,
-                         const float* A_blk, int b0, int nb, const float* transl, float* verts, int write_vp,
-                         int num_sms, cudaStream_t st) {
+                         const float* A_blk, int b0, int nb, const float* transl, float* verts, int num_sms,
+                         cudaStream_t st) {
   (void)S;
   const bool use_lo = mode != B200SMPL_MODE_BF16;
   if (m.fl.pseg != FF_PS * BK) return fail(B200SMPL_ERR_INVALID, "fused forward: unexpected pose segment width");
-  static const int dbg = getenv("B200_FF_DBG") == nullptr ? 0 : atoi(getenv("B200_FF_DBG"));   // timing experiments only
   if (m.n_virt0 != m.ntiles * FF_BN) return fail(B200SMPL_ERR_INVALID, "fused forward: vertex tiles must be 96 rows");
   CUtensorMap map_w, map_f;
   int rc;
@@ -525,7 +467,7 @@ int launch_blend_lbs_fwd(const DevModel& m, int mode, const __nv_bfloat16* feat,
   LaunchTimer _timer("blend_lbs_fwd", st);
   B200_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, map_w, map_f, (m.fl.k_cs + UMMA_K - 1) / UMMA_K, m.n_pad, ntiles_n, work,
                                    reinterpret_cast<float4*>(vpT), m.n_pad / 4, reinterpret_cast<const float4*>(A_blk), b0, nb,
-                                   transl, verts, m.V, m.ntiles, vec_ok, m.vplan, write_vp, dbg));
+                                   transl, verts, m.V, m.ntiles, vec_ok, m.vplan));
   B200_LAUNCH_CHECK("blend_lbs_fwd");
   return 0;
 }

@@ -16,10 +16,7 @@
 
 namespace b200smpl {
 
-#ifndef B200_JW
-#define B200_JW 8
-#endif
-constexpr int JW = B200_JW;                 // warps per CTA
+constexpr int JW = 8;                       // warps per CTA
 constexpr int JQ = 4;                       // warps per virtual tile: each takes 8 of its 32 q-groups (24 rows = 3 dvp chunks)
 constexpr int JTL = JW / JQ;                // virtual tiles per CTA
 constexpr int JT = JW * 32;

@@ -43,58 +43,6 @@ __device__ __forceinline__ void issue_item(float4* vbuf, uint32_t* stash, uint64
   bulk_g2s(vbuf, vp_group + (size_t)t * (SH::NCH4 * 32), SH::VP_WORDS * 4, bar);
   bulk_g2s(stash, vplan + (size_t)t * SH::PLAN_WORDS, SH::PLAN_WORDS * 4, bar);
 }
-// gradient rows: global -> registers (issued one item ahead) -> staging tile
-template <int HV>
-struct RowRegs {
-  float2 v[ItemShape<HV>::PAIRS];
-};
-template <int HV>
-__device__ __forceinline__ void rows_load(RowRegs<HV>& R, const float* __restrict__ src0, size_t row_stride, int nrows,
-                                          int ncols, int lane) {
-  using SH = ItemShape<HV>;
-  constexpr int RPP = 96 / SH::PAIRS, J = 32 / RPP;
-  if (nrows == 32 && ncols == SH::ROWS) {
-    const float* gp[3];
-#pragma unroll
-    for (int kk = 0; kk < 3; ++kk) {
-      const int piece = kk * 32 + lane, rr = piece / SH::PAIRS, c = (piece - rr * SH::PAIRS) * 2;
-      gp[kk] = src0 + (size_t)rr * row_stride + c;
-    }
-    const size_t step = (size_t)RPP * row_stride;
-#pragma unroll
-    for (int j = 0; j < J; ++j)
-#pragma unroll
-      for (int kk = 0; kk < 3; ++kk) {
-        R.v[j * 3 + kk] = ld_stream2(gp[kk]);
-        gp[kk] += step;
-      }
-  } else {
-#pragma unroll
-    for (int k = 0; k < SH::PAIRS; ++k) {        // same piece order: k = j * 3 + kk
-      const int piece = (k % 3) * 32 + lane, rr = piece / SH::PAIRS, c = (piece - rr * SH::PAIRS) * 2;
-      const int r = (k / 3) * RPP + rr;
-      float2 x = make_float2(0.f, 0.f);
-      if (r < nrows) {
-        const float* src = src0 + (size_t)r * row_stride + c;
-        if (c + 1 < ncols) x = ld_stream2(src);
-        else if (c < ncols) x.x = ld_stream(src);
-      }
-      R.v[k] = x;
-    }
-  }
-}
-template <int HV>
-__device__ __forceinline__ void rows_store(float* tile, const RowRegs<HV>& R, int lane) {
-  using SH = ItemShape<HV>;
-  constexpr int RPP = 96 / SH::PAIRS, J = 32 / RPP;
-#pragma unroll
-  for (int kk = 0; kk < 3; ++kk) {
-    const int piece = kk * 32 + lane, rr = piece / SH::PAIRS, c = (piece - rr * SH::PAIRS) * 2;
-    float* sp = tile + rr * SH::HROW + c;
-#pragma unroll
-    for (int j = 0; j < J; ++j) *reinterpret_cast<float2*>(sp + j * RPP * SH::HROW) = R.v[j * 3 + kk];
-  }
-}
 template <int HV>
 __device__ __forceinline__ void global_to_tile_scalar(float* tile, const float* src0, size_t row_stride, int nrows,
                                                       int ncols, int lane) {
@@ -106,18 +54,9 @@ __device__ __forceinline__ void global_to_tile_scalar(float* tile, const float* 
 // ---------------------------------------------------------------------------------------------
 // forward
 // ---------------------------------------------------------------------------------------------
-#ifndef B200_FWD_HV
-#define B200_FWD_HV 16
-#endif
-#ifndef B200_FWD_WARPS
-#define B200_FWD_WARPS 8
-#endif
-#ifndef B200_FWD_RUN
-#define B200_FWD_RUN 1
-#endif
-constexpr int FWD_RUN = B200_FWD_RUN;       // consecutive items per warp and round (slots persist inside a run)
-constexpr int FWD_HV = B200_FWD_HV;
-constexpr int FWD_WARPS = B200_FWD_WARPS;
+constexpr int FWD_RUN = 1;                  // consecutive items per warp and round (slots persist inside a run)
+constexpr int FWD_HV = 16;
+constexpr int FWD_WARPS = 8;
 constexpr int FWD_THREADS = FWD_WARPS * 32;
 // per warp: output tile | 2 x (v_posed block, plan records) | 2 mbarriers
 constexpr int FWD_WARP_WORDS = ItemShape<FWD_HV>::TILE_WORDS + 2 * (ItemShape<FWD_HV>::VP_WORDS + ItemShape<FWD_HV>::PLAN_WORDS) + 4;
@@ -269,22 +208,13 @@ lbs_fwd_kernel(const float4* __restrict__ vpB, int nc4, const float4* __restrict
 //   dv_posed = sum_s w_s R_s^T dV            -> bf16 hi (+lo) chunks of dvp (GEMM operand)
 //   dA_j    += w_s [dV (x) p | dV]           -> per-slot register accumulators -> fp32 RED into dA_acc
 //   dtransl += dV                            -> fp32 RED into dtr_acc
-// The gradient rows are 8-byte aligned only (no TMA): they are loaded into registers one item ahead and
-// dropped into the staging tile when the previous item has been packed.
+// The gradient rows are 8-byte aligned only (no TMA): they are copied by cp.async one item ahead into the other
+// tile of a double-buffered staging tile.
 // ---------------------------------------------------------------------------------------------
-#ifndef B200_BWD_HV
-#define B200_BWD_HV 8
-#endif
-#ifndef B200_BWD_WARPS
-#define B200_BWD_WARPS 8
-#endif
-constexpr int BWD_HV = B200_BWD_HV;
-constexpr int BWD_WARPS = B200_BWD_WARPS;
+constexpr int BWD_HV = 8;
+constexpr int BWD_WARPS = 8;
 constexpr int BWD_THREADS = BWD_WARPS * 32;
-#ifndef B200_BWD_ASYNC_ROWS
-#define B200_BWD_ASYNC_ROWS 1          // 1: dV rows via cp.async into a double-buffered tile; 0: via registers
-#endif
-constexpr int BWD_NTILE = B200_BWD_ASYNC_ROWS ? 2 : 1;
+constexpr int BWD_NTILE = 2;                // dV rows arrive by cp.async in a double-buffered tile
 constexpr int BWD_WARP_WORDS = BWD_NTILE * ItemShape<BWD_HV>::TILE_WORDS + 2 * (ItemShape<BWD_HV>::VP_WORDS + ItemShape<BWD_HV>::PLAN_WORDS) + 4;
 constexpr size_t BWD_SMEM = (size_t)(AG_WORDS + BWD_WARPS * BWD_WARP_WORDS) * 4 + 16;
 
@@ -406,18 +336,9 @@ lbs_bwd_kernel(const float4* __restrict__ vpB, int nc4, const float4* __restrict
         issue_item<HV>(vbufs + b * (SH::NCH4 * 32), stash + b * SH::PLAN_WORDS, &wbar[b], vp_g, vplan, it0);
       }
       // first item's gradient rows
-#if B200_BWD_ASYNC_ROWS
       int tb = 0;
       if (vec_ok) issue_rows<HV>(tiles, dv_g + (size_t)it0 * HV * 3, row_stride, nrows, max(0, min(HV, V - it0 * HV)) * 3, lane);
       cp_async_commit();
-#else
-      constexpr int tb = 0;
-      RowRegs<HV> R;
-      if (vec_ok) {
-        rows_load<HV>(R, dv_g + (size_t)it0 * HV * 3, row_stride, nrows, max(0, min(HV, V - it0 * HV)) * 3, lane);
-        rows_store<HV>(tiles, R, lane);
-      }
-#endif
       if (!vec_ok)
         global_to_tile_scalar<HV>(tiles, dv_g + (size_t)it0 * HV * 3, row_stride, nrows, max(0, min(HV, V - it0 * HV)) * 3, lane);
       BwdState st;
@@ -437,20 +358,13 @@ lbs_bwd_kernel(const float4* __restrict__ vpB, int nc4, const float4* __restrict
         if (more) {                                               // next item: TMA for v_posed + plan, dV rows
           if (lane == 0)
             issue_item<HV>(vbufs + (b ^ 1) * (SH::NCH4 * 32), stash + (b ^ 1) * SH::PLAN_WORDS, &wbar[b ^ 1], vp_g, vplan, t + 1);
-#if B200_BWD_ASYNC_ROWS
           if (vec_ok)
             issue_rows<HV>(tiles + (tb ^ 1) * SH::TILE_WORDS, dv_g + (size_t)(t + 1) * HV * 3, row_stride, nrows,
                            max(0, min(HV, V - (t + 1) * HV)) * 3, lane);
-#else
-          if (vec_ok)
-            rows_load<HV>(R, dv_g + (size_t)(t + 1) * HV * 3, row_stride, nrows, max(0, min(HV, V - (t + 1) * HV)) * 3, lane);
-#endif
         }
-#if B200_BWD_ASYNC_ROWS
         cp_async_commit();
         cp_async_wait<1>();
         __syncwarp();                                              // this item's dV rows were copied by other lanes
-#endif
         mbar_wait(&wbar[b], (n_used >> 1) & 1);
         const float4* vp_s = vbufs + b * (SH::NCH4 * 32) + lane;
         const uint32_t* ps = stash + b * SH::PLAN_WORDS;
@@ -472,18 +386,10 @@ lbs_bwd_kernel(const float4* __restrict__ vpB, int nc4, const float4* __restrict
           }
         }
         __syncwarp();                                              // every lane is done with its row of the tile
-#if B200_BWD_ASYNC_ROWS
         if (more && !vec_ok)
           global_to_tile_scalar<HV>(tiles + (tb ^ 1) * SH::TILE_WORDS, dv_g + (size_t)(t + 1) * HV * 3, row_stride, nrows,
                                     max(0, min(HV, V - (t + 1) * HV)) * 3, lane);
         tb ^= 1;
-#else
-        if (more) {
-          if (vec_ok) rows_store<HV>(tile, R, lane);
-          else global_to_tile_scalar<HV>(tile, dv_g + (size_t)(t + 1) * HV * 3, row_stride, nrows,
-                                         max(0, min(HV, V - (t + 1) * HV)) * 3, lane);
-        }
-#endif
         __syncwarp();                                              // the next item's rows were written by other lanes
         ++n_used;
       }

@@ -238,23 +238,6 @@ int pack_model(const b200smpl_model_desc* d, HostArrays& h, DevModel& dm, std::s
     }
   }
 
-  // ---- the backward operand again, blocked per (CTA half, 16-vertex item) for the fused backward ----
-  {
-    const int nh = fl.nf_pad / 2, nitems = ntiles * 2;                 // nf_pad is a multiple of 16: nh of 8
-    h.Wbi_hi.assign((size_t)2 * nitems * 6 * nh * 8, h_bf16(0.f));
-    h.Wbi_lo.assign((size_t)2 * nitems * 6 * nh * 8, h_bf16(0.f));
-    for (int half = 0; half < 2; ++half)
-      for (int it = 0; it < nitems; ++it)
-        for (int c = 0; c < 6; ++c)
-          for (int f = 0; f < nh; ++f)
-            for (int r = 0; r < 8; ++r) {
-              const size_t src = (size_t)(half * nh + f) * n_pad + (size_t)it * 48 + c * 8 + r;
-              const size_t dst = ((((size_t)half * nitems + it) * 6 + c) * nh + f) * 8 + r;
-              h.Wbi_hi[dst] = h.Wb_hi[src];
-              h.Wbi_lo[dst] = h.Wb_lo[src];
-            }
-  }
-
   // ---- rest joints as an affine function of betas (fp64 fold of J_regressor) ----
   h.Jt.assign(NJ * 3, 0.f);
   h.Jsd.assign((size_t)NJ * 3 * nb, 0.f);

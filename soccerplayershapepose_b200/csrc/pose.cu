@@ -1,23 +1,19 @@
 // Pose stage (SURVEY.md section 8 rows a6, a7 (feature), a8): Rodrigues, rest joints, pose
 // feature, the 24-joint kinematic chain and the skinning transforms A = [G_R | G_t - G_R J].
 //
-// One warp per body, lane j owns joint j.  The chain G_j = G_parent(j) . L_j is a level-synchronous
-// shuffle scan over the tree depth (8 rounds for SMPL) instead of the reference's 23-iteration
-// Python loop of batched matmuls (smplx.lbs.batch_rigid_transform).  Rest joints use the
-// pack-time folds J_template = J_regressor.v_template, J_shapedirs = J_regressor.shapedirs.
-// Outputs are written body-fastest (A_T[j*12+e][b]) through a shared-memory transpose because
-// the skinning kernels run with lane = body.
+// Lane = body: one CTA (16 warps) per 32-body group, each lane holds one body.  The chain G_j = G_parent(j) . L_j
+// is walked one tree level at a time (9 levels on the SMPL tree), one warp per joint of the level, instead of the
+// reference's 23-iteration Python loop of batched matmuls (smplx.lbs.batch_rigid_transform).  There is no shuffle,
+// no divergence and no idle lane.  Per-joint state that is indexed dynamically (local rotations, global transforms,
+// rest joints, gradient accumulators) lives in shared memory as [row][lane] (conflict-free); the group-blocked
+// operands of the skinning kernels (A_blk, dA) are read / written straight from registers, coalesced; row-major
+// per-body tensors (pose, grad_pose) go through a transposing stage.  Rest joints use the pack-time folds
+// J_template = J_regressor.v_template, J_shapedirs = J_regressor.shapedirs.
 #include "common.cuh"
 #include "rodrigues.cuh"
 #include "skin_common.cuh"
 
 namespace b200smpl {
-
-constexpr int POSE_WARPS = 16;
-constexpr int POSE_THREADS = POSE_WARPS * 32;
-constexpr int BODIES_PER_WARP = 2;          // 32 bodies per CTA
-constexpr int OUT_ROWS = NJ * AELEMS + NJ * 3;  // 288 A rows + 72 posed-joint rows
-constexpr int OUT_PITCH = 33;
 
 // G <- P . G   for 3x4 affine matrices [R|t] (implicit last row 0 0 0 1)
 __device__ __forceinline__ void compose(const float P[12], float G[12]) {
@@ -32,336 +28,11 @@ __device__ __forceinline__ void compose(const float P[12], float G[12]) {
   for (int i = 0; i < 12; ++i) G[i] = o[i];
 }
 
-struct LaneChain {
-  float R[9];     // local rotation
-  float Jr[3];    // rest joint
-  float rel[3];   // Jr - Jr[parent]   (root: Jr)
-  float G[12];    // global transform
-  float PR[9];    // parent's global rotation (identity for the root)
-};
-
-template <bool AA>
-__device__ __forceinline__ void chain_forward(const DevModel& m, const float* __restrict__ betas,
-                                              const float* __restrict__ pose, int b, int lane, bool live,
-                                              LaneChain& L, float raa[3]) {
-  const int j = lane < NJ ? lane : 0;
-  const int nb = m.fl.nb;
-#pragma unroll
-  for (int e = 0; e < 9; ++e) L.R[e] = (e == 0 || e == 4 || e == 8) ? 1.f : 0.f;
-  raa[0] = raa[1] = raa[2] = 0.f;
-  if (live && lane < NJ) {
-    if (AA) {
-      raa[0] = pose[(size_t)b * (NJ * 3) + j * 3 + 0];
-      raa[1] = pose[(size_t)b * (NJ * 3) + j * 3 + 1];
-      raa[2] = pose[(size_t)b * (NJ * 3) + j * 3 + 2];
-      rodrigues_fwd(raa, L.R);
-    } else {
-#pragma unroll
-      for (int e = 0; e < 9; ++e) L.R[e] = pose[(size_t)b * (NJ * 9) + j * 9 + e];
-    }
-  }
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
-    float acc = m.Jt[j * 3 + k];
-    if (live)
-      for (int l = 0; l < nb; ++l) acc = fmaf(m.Jsd[(j * 3 + k) * nb + l], betas[(size_t)b * nb + l], acc);
-    L.Jr[k] = acc;
-  }
-  const int parent = m.chain.parent[j];
-  const int psrc = parent < 0 ? 0 : parent;
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
-    const float pj = __shfl_sync(0xffffffffu, L.Jr[k], psrc);
-    L.rel[k] = parent < 0 ? L.Jr[k] : L.Jr[k] - pj;
-  }
-#pragma unroll
-  for (int r = 0; r < 3; ++r) {
-#pragma unroll
-    for (int c = 0; c < 3; ++c) L.G[r * 4 + c] = L.R[r * 3 + c];
-    L.G[r * 4 + 3] = L.rel[r];
-  }
-#pragma unroll
-  for (int e = 0; e < 9; ++e) L.PR[e] = (e == 0 || e == 4 || e == 8) ? 1.f : 0.f;
-  const int depth = lane < NJ ? m.chain.depth[j] : -1;
-  for (int d = 1; d <= m.chain.maxdepth; ++d) {
-    float P[12];
-#pragma unroll
-    for (int e = 0; e < 12; ++e) P[e] = __shfl_sync(0xffffffffu, L.G[e], psrc);
-    if (depth == d) {
-#pragma unroll
-      for (int r = 0; r < 3; ++r)
-#pragma unroll
-        for (int c = 0; c < 3; ++c) L.PR[r * 3 + c] = P[r * 4 + c];
-      compose(P, L.G);
-    }
-  }
-}
-
 __device__ __forceinline__ __nv_bfloat16 bf_hi(float x) { return __float2bfloat16_rn(x); }
 __device__ __forceinline__ __nv_bfloat16 bf_lo(float x, __nv_bfloat16 hi) {
   return __float2bfloat16_rn(x - __bfloat162float(hi));
 }
 
-template <bool AA>
-__global__ void __launch_bounds__(POSE_THREADS)
-pose_fwd_kernel(DevModel m, const float* __restrict__ betas, const float* __restrict__ pose, int b0, int nb, int S,
-                __nv_bfloat16* __restrict__ feat, float* __restrict__ featf, float* __restrict__ A_T,
-                const float* __restrict__ transl, float* __restrict__ joints) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  float* sOut = reinterpret_cast<float*>(smem_raw);                        // [OUT_ROWS][OUT_PITCH]
-  __nv_bfloat16* sF_all = reinterpret_cast<__nv_bfloat16*>(sOut + OUT_ROWS * OUT_PITCH);  // [warps][pitch]
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const FeatLayout fl = m.fl;
-  __nv_bfloat16* sF = sF_all + warp * fl.pitch;
-
-  for (int i = 0; i < BODIES_PER_WARP; ++i) {
-    const int bl = warp * BODIES_PER_WARP + i;
-    const int sc = blockIdx.x * 32 + bl;                // slab column
-    const int b = b0 + sc;                              // global body
-    const bool live = sc < nb;
-    LaneChain L;
-    float raa[3];
-    chain_forward<AA>(m, betas, pose, b, lane, live, L, raa);
-    if (lane < NJ) {
-      // A = [G_R | G_t - G_R Jr] ; posed joint = G_t
-      float* o = sOut + (lane * AELEMS) * OUT_PITCH + bl;
-#pragma unroll
-      for (int r = 0; r < 3; ++r) {
-#pragma unroll
-        for (int c = 0; c < 3; ++c) o[(r * 4 + c) * OUT_PITCH] = live ? L.G[r * 4 + c] : 0.f;
-        const float t = L.G[r * 4 + 3] - (L.G[r * 4] * L.Jr[0] + L.G[r * 4 + 1] * L.Jr[1] + L.G[r * 4 + 2] * L.Jr[2]);
-        o[(r * 4 + 3) * OUT_PITCH] = live ? t : 0.f;
-        sOut[(NJ * AELEMS + lane * 3 + r) * OUT_PITCH + bl] = live ? L.G[r * 4 + 3] : 0.f;
-      }
-    }
-    // feature row (bf16 split), staged per warp then written as 16-byte chunks
-    for (int k = lane; k < fl.pitch; k += 32) sF[k] = __float2bfloat16_rn(0.f);
-    if (featf != nullptr)
-      for (int k = lane; k < fl.nf_pad; k += 32) featf[(size_t)sc * fl.nf_pad + k] = 0.f;
-    __syncwarp();
-    if (live) {
-      if (lane < 3) sF[lane] = __float2bfloat16_rn(1.f);
-      if (lane < fl.nb) {
-        const float be = betas[(size_t)b * fl.nb + lane];
-        const __nv_bfloat16 h = bf_hi(be), l = bf_lo(be, h);
-        sF[fl.off_s0 + lane] = h;
-        sF[fl.off_s1 + lane] = l;
-        sF[fl.off_s2 + lane] = h;
-        if (featf != nullptr) featf[(size_t)sc * fl.nf_pad + lane] = be;
-      }
-      if (lane >= 1 && lane < NJ) {
-#pragma unroll
-        for (int e = 0; e < 9; ++e) {
-          const float pf = L.R[e] - ((e == 0 || e == 4 || e == 8) ? 1.f : 0.f);
-          const int idx = (lane - 1) * 9 + e;
-          const __nv_bfloat16 h = bf_hi(pf), l = bf_lo(pf, h);
-          sF[fl.off_p0 + idx] = h;
-          sF[fl.off_p1 + idx] = l;
-          if (featf != nullptr) featf[(size_t)sc * fl.nf_pad + fl.nb + idx] = pf;
-        }
-      }
-    }
-    __syncwarp();
-    {
-      const uint4* src = reinterpret_cast<const uint4*>(sF);
-      uint4* dst = reinterpret_cast<uint4*>(feat + (size_t)sc * fl.pitch);
-      for (int k = lane; k < fl.pitch / 8; k += 32) dst[k] = src[k];
-    }
-    __syncwarp();
-  }
-  __syncthreads();
-  // group-blocked output A_blk[group][joint][3][lane] float4 (one contiguous 36 KB block per 32 bodies), the
-  // three float4 of a joint holding (r00 r10 r01 r11) (r02 r12 t0 t1) (r20 r21 r22 t2): x/y rows interleaved
-  // as the operand pairs of the packed-fp32 skinning arithmetic (skin_common.cuh)
-  (void)S;
-  for (int idx = threadIdx.x; idx < NJ * AELEMS * 32; idx += POSE_THREADS) {
-    const int c = idx & 3, bl = (idx >> 2) & 31, jf = idx >> 7;          // jf = joint * 3 + float4 index
-    const int joint = jf / 3, f = jf - joint * 3;
-    const int e = f == 2 ? 8 + c : (f * 2 + (c >> 1)) + 4 * (c & 1);      // row-major [R | t] element
-    A_T[(size_t)blockIdx.x * NJ * AELEMS * 32 + idx] = sOut[(joint * AELEMS + e) * OUT_PITCH + bl];
-  }
-  // the 24 posed chain joints (+ transl) go straight into joints[:, 0:24] as 288 B row segments
-  if (joints != nullptr) {
-    const size_t ncol_all = (size_t)m.njout * 3;
-    for (int idx = threadIdx.x; idx < 32 * NJ * 3; idx += POSE_THREADS) {
-      const int body = idx / (NJ * 3), col = idx - body * (NJ * 3);
-      const int sc = blockIdx.x * 32 + body;
-      if (sc < nb) {
-        const float t = transl != nullptr ? transl[(size_t)(b0 + sc) * 3 + col % 3] : 0.f;
-        joints[(size_t)(b0 + sc) * ncol_all + col] = sOut[(NJ * AELEMS + col) * OUT_PITCH + body] + t;
-      }
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
-// backward of the pose stage.  Inputs (all body-fastest, pitch Bp):
-//   dA_part[p][G][288][32] partial sums of dL/dA, dtr_part[p][G][3][32] (group-blocked, slab-local),
-//   dfeat_part[p][S][nf_pad] : dL/d[beta | pose_feature] from the blend-GEMM backward,
-//   dJ (B, NJout, 3) total joint gradient (may be null): its first 24 joints are the chain joints.
-// ---------------------------------------------------------------------------------------------
-constexpr int IN_ROWS = NJ * AELEMS + 3;
-
-template <bool AA>
-__global__ void __launch_bounds__(POSE_THREADS)
-pose_bwd_kernel(DevModel m, const float* __restrict__ betas, const float* __restrict__ pose, int b0, int nb, int S,
-                const float* __restrict__ dA_part, int n_dA_parts, const float* __restrict__ dtr_part,
-                const float* __restrict__ dfeat_part, int n_dfeat_parts, const float* __restrict__ dJ,
-                float* __restrict__ grad_betas, float* __restrict__ grad_pose, float* __restrict__ grad_transl) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  float* sIn = reinterpret_cast<float*>(smem_raw);                         // [IN_ROWS][OUT_PITCH]
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const FeatLayout fl = m.fl;
-  const int G = S / 32, g = blockIdx.x;                  // group-blocked partials [part][group][rows][32]
-  for (int r = warp; r < IN_ROWS; r += POSE_WARPS) {
-    float v = 0.f;
-    if (r < NJ * AELEMS) {
-      for (int p = 0; p < n_dA_parts; ++p) v += dA_part[(((size_t)p * G + g) * NJ * AELEMS + r) * 32 + lane];
-    } else {
-      const int k = r - NJ * AELEMS;
-      for (int p = 0; p < n_dA_parts; ++p) v += dtr_part[(((size_t)p * G + g) * 3 + k) * 32 + lane];
-    }
-    sIn[r * OUT_PITCH + lane] = v;
-  }
-  __syncthreads();
-
-  for (int i = 0; i < BODIES_PER_WARP; ++i) {
-    const int bl = warp * BODIES_PER_WARP + i;
-    const int sc = blockIdx.x * 32 + bl;
-    if (sc >= nb) break;                                // warp-uniform
-    const int b = b0 + sc;
-    LaneChain L;
-    float raa[3];
-    chain_forward<AA>(m, betas, pose, b, lane, true, L, raa);
-    const int j = lane < NJ ? lane : 0;
-    const bool act = lane < NJ;
-    float dGR[9], dGt[3], dJr[3], dJp[3];
-    {
-      float dAr[12];
-#pragma unroll
-      for (int e = 0; e < 12; ++e) dAr[e] = act ? sIn[(j * AELEMS + e) * OUT_PITCH + bl] : 0.f;
-#pragma unroll
-      for (int r = 0; r < 3; ++r) {
-        const float dat = dAr[r * 4 + 3];
-        dJp[r] = (act && dJ != nullptr) ? dJ[((size_t)b * m.njout + j) * 3 + r] : 0.f;
-        dGt[r] = dat + dJp[r];
-#pragma unroll
-        for (int c = 0; c < 3; ++c) dGR[r * 3 + c] = dAr[r * 4 + c] - dat * L.Jr[c];
-      }
-#pragma unroll
-      for (int c = 0; c < 3; ++c)
-        dJr[c] = -(L.G[c] * dAr[3] + L.G[4 + c] * dAr[7] + L.G[8 + c] * dAr[11]);
-    }
-    const int depth = act ? m.chain.depth[j] : -1;
-    const int nchild = act ? m.chain.nchild[j] : 0;
-    float dRl[9], drel[3];
-#pragma unroll
-    for (int e = 0; e < 9; ++e) dRl[e] = 0.f;
-    drel[0] = drel[1] = drel[2] = 0.f;
-    for (int d = m.chain.maxdepth; d >= 1; --d) {
-      // child-side quantities (valid on lanes with depth == d, whose dG is final by now)
-      float cR[9], cdrel[3];
-#pragma unroll
-      for (int r = 0; r < 3; ++r)
-#pragma unroll
-        for (int c = 0; c < 3; ++c)
-          cR[r * 3 + c] = dGR[r * 3] * L.R[c * 3] + dGR[r * 3 + 1] * L.R[c * 3 + 1] + dGR[r * 3 + 2] * L.R[c * 3 + 2] +
-                          dGt[r] * L.rel[c];
-#pragma unroll
-      for (int c = 0; c < 3; ++c) cdrel[c] = L.PR[c] * dGt[0] + L.PR[3 + c] * dGt[1] + L.PR[6 + c] * dGt[2];
-      if (depth == d) {
-#pragma unroll
-        for (int r = 0; r < 3; ++r)
-#pragma unroll
-          for (int c = 0; c < 3; ++c)
-            dRl[r * 3 + c] = L.PR[r] * dGR[c] + L.PR[3 + r] * dGR[3 + c] + L.PR[6 + r] * dGR[6 + c];
-#pragma unroll
-        for (int c = 0; c < 3; ++c) drel[c] = cdrel[c];
-      }
-      // parent-side gather
-      const int kmax = m.chain.maxchild_at[d];          // warp-uniform: most levels of the SMPL tree have 1
-#pragma unroll 1
-      for (int k = 0; k < kmax; ++k) {
-        const int ch = (k < nchild) ? m.chain.child[j][k] : -1;
-        const int src = ch < 0 ? 0 : ch;
-        const int chd = __shfl_sync(0xffffffffu, depth, src);
-        const bool take = ch >= 0 && chd == d;
-#pragma unroll
-        for (int e = 0; e < 9; ++e) {
-          const float v = __shfl_sync(0xffffffffu, cR[e], src);
-          if (take) dGR[e] += v;
-        }
-#pragma unroll
-        for (int e = 0; e < 3; ++e) {
-          const float v = __shfl_sync(0xffffffffu, dGt[e], src);
-          const float w = __shfl_sync(0xffffffffu, cdrel[e], src);
-          if (take) {
-            dGt[e] += v;
-            dJr[e] -= w;
-          }
-        }
-      }
-    }
-    if (lane == 0) {
-#pragma unroll
-      for (int e = 0; e < 9; ++e) dRl[e] = dGR[e];
-#pragma unroll
-      for (int c = 0; c < 3; ++c) dJr[c] += dGt[c];
-    } else {
-#pragma unroll
-      for (int c = 0; c < 3; ++c) dJr[c] += drel[c];
-    }
-    // d beta = sum_j Jsd_j^T dJr_j  + blend part
-    for (int l = 0; l < fl.nb; ++l) {
-      float p = act ? (m.Jsd[(j * 3 + 0) * fl.nb + l] * dJr[0] + m.Jsd[(j * 3 + 1) * fl.nb + l] * dJr[1] +
-                       m.Jsd[(j * 3 + 2) * fl.nb + l] * dJr[2])
-                    : 0.f;
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) p += __shfl_xor_sync(0xffffffffu, p, o);
-      if (lane == l) {
-        for (int q = 0; q < n_dfeat_parts; ++q) p += dfeat_part[((size_t)q * S + sc) * fl.nf_pad + l];
-        grad_betas[(size_t)b * fl.nb + l] = p;
-      }
-    }
-    if (act && lane >= 1) {
-      for (int q = 0; q < n_dfeat_parts; ++q) {
-        const float* df = dfeat_part + ((size_t)q * S + sc) * fl.nf_pad + fl.nb + (lane - 1) * 9;
-#pragma unroll
-        for (int e = 0; e < 9; ++e) dRl[e] += df[e];
-      }
-    }
-    if (act) {
-      if (AA) {
-        float dr[3];
-        rodrigues_bwd(raa, dRl, dr);
-#pragma unroll
-        for (int k = 0; k < 3; ++k) grad_pose[(size_t)b * (NJ * 3) + j * 3 + k] = dr[k];
-      } else {
-#pragma unroll
-        for (int e = 0; e < 9; ++e) grad_pose[(size_t)b * (NJ * 9) + j * 9 + e] = dRl[e];
-      }
-    }
-    if (grad_transl != nullptr) {                     // skinning / joint partials + the chain joints' own gradient
-#pragma unroll
-      for (int r = 0; r < 3; ++r) {
-        float t = dJp[r];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
-        if (lane == r) grad_transl[(size_t)b * 3 + r] = t + sIn[(NJ * AELEMS + r) * OUT_PITCH + bl];
-      }
-    }
-  }
-}
-
-// =============================================================================================
-// lane = body versions (default).  One warp per 32-body group, each lane walks ITS body's 24 joints
-// sequentially (parents precede children in the SMPL tree), so there is no shuffle, no divergence and no idle
-// lane: ~10x fewer warp instructions per body than the lane = joint kernels above (ncu: 3800 warp instructions
-// per body in pose_bwd, issue-bound at 16 warps per SM).  Per-joint state that is indexed dynamically (local
-// rotations, global transforms, rest joints, gradient accumulators) lives in shared memory as [row][lane]
-// (conflict-free); the group-blocked operands of the skinning kernels (A_blk, dA) are read / written straight
-// from registers, coalesced; row-major per-body tensors (pose, grad_pose) go through a transposing stage.
-// =============================================================================================
 constexpr int LB_P = 33;                     // pitch of the transposed staging rows
 constexpr int LB_MAXB = 20;                  // betas that fit slab 0 of the feature layout
 
@@ -386,7 +57,7 @@ struct LbFwdSmem {
 // ---- forward, lane = body.  One CTA (16 warps) per 32-body group:
 //   P1 all threads: pose rows (transposed through registers), betas, translation, model constants;
 //   P2 all threads: rest joints (and Rodrigues for axis-angle input);
-//   P3 warp 0: the walk down the 24 joints, each lane ITS body: G_j = G_parent . [R_j | Jr_j - Jr_parent];
+//   P3 level by level, one warp per joint, each lane ITS body: G_j = G_parent . [R_j | Jr_j - Jr_parent];
 //   P4 all threads: A = [G_R | G_t - G_R Jr] as coalesced float4, posed joints, the bf16 hi / lo feature row.
 template <bool AA>
 __global__ void __launch_bounds__(LBF_THREADS, 1)
@@ -573,12 +244,12 @@ pose_fwd_lb_kernel(DevModel m, const float* __restrict__ betas, const float* __r
   }
 }
 
-// ---- backward, lane = body.  One CTA (4 warps) per 32-body group:
+// ---- backward, lane = body.  One CTA (16 warps) per 32-body group:
 //   P1 all threads: every input of the group staged into shared memory with coalesced, batched loads (pose rows,
 //      betas, the group's A block -> global rotations, dA, the split-K partials of dfeat summed, the chain
 //      joints' dJ), accumulators cleared;
 //   P2 all threads: rest joints (and Rodrigues for axis-angle input), G_t = A_t + G_R Jr;
-//   P3 warp 0: the reverse walk over the 24 joints, each lane ITS body, shared memory only (the critical path:
+//   P3 the reverse walk, deepest level first, one warp per joint, each lane ITS body, shared memory only (the critical path:
 //      ~200 instructions per joint);
 //   P4 all threads: + pose-blend gradient (Rodrigues backward for axis-angle), betas / transl gradients, coalesced
 //      write-out.
@@ -877,39 +548,25 @@ pose_bwd_lb_kernel(DevModel m, const float* __restrict__ betas, const float* __r
 constexpr size_t LB_FWD_SMEM = sizeof(LbFwdSmem);
 constexpr size_t LB_BWD_SMEM = sizeof(LbBwdSmem);
 
-// B200_POSE_LB=0 selects the lane = joint kernels (kept for comparison)
-static int pose_use_lb() {   // bit 0: forward, bit 1: backward
-  static const int v = getenv("B200_POSE_LB") == nullptr ? 3 : atoi(getenv("B200_POSE_LB"));
-  return v;
-}
+// pack_model rejects more than MAX_BETAS betas, so every model fits these kernels: one thread per (body, beta)
+// stages the betas, slab 0 of the feature layout holds them, and dfeat rows (nf_pad) fit sm.DF
+static_assert(MAX_BETAS * 32 <= LBF_THREADS && MAX_BETAS * 32 <= LBB_THREADS, "betas staging: one thread per (body, beta)");
+static_assert(MAX_BETAS <= LB_MAXB, "betas staging arrays");
+static_assert((MAX_BETAS + NPOSE + 15) / 16 * 16 <= 224, "sm.DF holds nf_pad <= 224 rows");
 
 // Sw = active slab width (multiple of 32, >= nb); columns in [nb, Sw) are written as zeros
 int launch_pose_fwd(const DevModel& m, const float* betas, const float* pose, bool axis_angle, int b0, int nb, int S,
                     int Sw, __nv_bfloat16* feat, float* featf, float* A_T, const float* transl, float* joints,
                     cudaStream_t st) {
   const int grid = Sw / 32;
-  if ((pose_use_lb() & 1) && m.fl.nb * 32 <= LBF_THREADS) {
-    if (axis_angle) {
-      B200_SMEM_ATTR_ONCE(pose_fwd_lb_kernel<true>, LB_FWD_SMEM);
-      LaunchTimer _timer("pose_fwd", st);
-      pose_fwd_lb_kernel<true><<<grid, LBF_THREADS, LB_FWD_SMEM, st>>>(m, betas, pose, b0, nb, S, feat, featf, A_T, transl, joints);
-    } else {
-      B200_SMEM_ATTR_ONCE(pose_fwd_lb_kernel<false>, LB_FWD_SMEM);
-      LaunchTimer _timer("pose_fwd", st);
-      pose_fwd_lb_kernel<false><<<grid, LBF_THREADS, LB_FWD_SMEM, st>>>(m, betas, pose, b0, nb, S, feat, featf, A_T, transl, joints);
-    }
-    B200_LAUNCH_CHECK("pose_fwd");
-    return 0;
-  }
-  const size_t smem = (size_t)OUT_ROWS * OUT_PITCH * sizeof(float) + (size_t)POSE_WARPS * m.fl.pitch * 2;
   if (axis_angle) {
-    B200_CUDA_TRY(cudaFuncSetAttribute(pose_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    LaunchTimer _timer_405("pose_fwd", st);
-    pose_fwd_kernel<true><<<grid, POSE_THREADS, smem, st>>>(m, betas, pose, b0, nb, S, feat, featf, A_T, transl, joints);
+    B200_SMEM_ATTR_ONCE(pose_fwd_lb_kernel<true>, LB_FWD_SMEM);
+    LaunchTimer _timer("pose_fwd", st);
+    pose_fwd_lb_kernel<true><<<grid, LBF_THREADS, LB_FWD_SMEM, st>>>(m, betas, pose, b0, nb, S, feat, featf, A_T, transl, joints);
   } else {
-    B200_CUDA_TRY(cudaFuncSetAttribute(pose_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    LaunchTimer _timer_408("pose_fwd", st);
-    pose_fwd_kernel<false><<<grid, POSE_THREADS, smem, st>>>(m, betas, pose, b0, nb, S, feat, featf, A_T, transl, joints);
+    B200_SMEM_ATTR_ONCE(pose_fwd_lb_kernel<false>, LB_FWD_SMEM);
+    LaunchTimer _timer("pose_fwd", st);
+    pose_fwd_lb_kernel<false><<<grid, LBF_THREADS, LB_FWD_SMEM, st>>>(m, betas, pose, b0, nb, S, feat, featf, A_T, transl, joints);
   }
   B200_LAUNCH_CHECK("pose_fwd");
   return 0;
@@ -921,36 +578,18 @@ int launch_pose_bwd(const DevModel& m, const float* betas, const float* pose, bo
                     float* grad_transl, cudaStream_t st) {
   if (nb <= 0) return 0;
   const int grid = (nb + 31) / 32;
-  if ((pose_use_lb() & 2) && A_blk != nullptr && m.fl.nf_pad <= 224 && m.fl.nb * 32 <= LBB_THREADS) {
-    if (axis_angle) {
-      B200_SMEM_ATTR_ONCE(pose_bwd_lb_kernel<true>, LB_BWD_SMEM);
-      LaunchTimer _timer("pose_bwd", st);
-      B200_CUDA_TRY(launch_k(pose_bwd_lb_kernel<true>, dim3(grid), dim3(LBB_THREADS), LB_BWD_SMEM, st, true, m, betas, pose, b0, nb,
-                             S, A_blk, dA_part, n_dA_parts, dtr_part, dfeat_part, n_dfeat_parts, dJ, grad_betas, grad_pose,
-                             grad_transl));
-    } else {
-      B200_SMEM_ATTR_ONCE(pose_bwd_lb_kernel<false>, LB_BWD_SMEM);
-      LaunchTimer _timer("pose_bwd", st);
-      B200_CUDA_TRY(launch_k(pose_bwd_lb_kernel<false>, dim3(grid), dim3(LBB_THREADS), LB_BWD_SMEM, st, true, m, betas, pose, b0, nb,
-                             S, A_blk, dA_part, n_dA_parts, dtr_part, dfeat_part, n_dfeat_parts, dJ, grad_betas, grad_pose,
-                             grad_transl));
-    }
-    B200_LAUNCH_CHECK("pose_bwd");
-    return 0;
-  }
-  const size_t smem = (size_t)IN_ROWS * OUT_PITCH * sizeof(float);
   if (axis_angle) {
-    B200_CUDA_TRY(cudaFuncSetAttribute(pose_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    LaunchTimer _timer_423("pose_bwd", st);
-    pose_bwd_kernel<true><<<grid, POSE_THREADS, smem, st>>>(m, betas, pose, b0, nb, S, dA_part, n_dA_parts, dtr_part,
-                                                            dfeat_part, n_dfeat_parts, dJ, grad_betas,
-                                                            grad_pose, grad_transl);
+    B200_SMEM_ATTR_ONCE(pose_bwd_lb_kernel<true>, LB_BWD_SMEM);
+    LaunchTimer _timer("pose_bwd", st);
+    B200_CUDA_TRY(launch_k(pose_bwd_lb_kernel<true>, dim3(grid), dim3(LBB_THREADS), LB_BWD_SMEM, st, true, m, betas, pose, b0, nb,
+                           S, A_blk, dA_part, n_dA_parts, dtr_part, dfeat_part, n_dfeat_parts, dJ, grad_betas, grad_pose,
+                           grad_transl));
   } else {
-    B200_CUDA_TRY(cudaFuncSetAttribute(pose_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    LaunchTimer _timer_428("pose_bwd", st);
-    pose_bwd_kernel<false><<<grid, POSE_THREADS, smem, st>>>(m, betas, pose, b0, nb, S, dA_part, n_dA_parts, dtr_part,
-                                                             dfeat_part, n_dfeat_parts, dJ, grad_betas,
-                                                             grad_pose, grad_transl);
+    B200_SMEM_ATTR_ONCE(pose_bwd_lb_kernel<false>, LB_BWD_SMEM);
+    LaunchTimer _timer("pose_bwd", st);
+    B200_CUDA_TRY(launch_k(pose_bwd_lb_kernel<false>, dim3(grid), dim3(LBB_THREADS), LB_BWD_SMEM, st, true, m, betas, pose, b0, nb,
+                           S, A_blk, dA_part, n_dA_parts, dtr_part, dfeat_part, n_dfeat_parts, dJ, grad_betas, grad_pose,
+                           grad_transl));
   }
   B200_LAUNCH_CHECK("pose_bwd");
   return 0;

@@ -60,11 +60,6 @@ __device__ __forceinline__ float ld_stream(const float* p) {
   asm volatile("ld.global.nc.L1::no_allocate.f32 %0, [%1];" : "=f"(v) : "l"(p));
   return v;
 }
-__device__ __forceinline__ float2 ld_stream2(const float* p) {
-  float2 v;
-  asm volatile("ld.global.nc.L1::no_allocate.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "l"(p));
-  return v;
-}
 __device__ __forceinline__ float4 ld_stream4(const float4* p) {
   float4 v;
   asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];"
@@ -75,21 +70,8 @@ __device__ __forceinline__ float4 ld_stream4(const float4* p) {
 __device__ __forceinline__ void st_stream(float* p, float v) {
   asm volatile("st.global.L1::no_allocate.f32 [%0], %1;" ::"l"(p), "f"(v) : "memory");
 }
-#ifndef B200_ST_MODE
-#define B200_ST_MODE 0
-#endif
 __device__ __forceinline__ void st_stream2(float* p, float2 v) {
-#if B200_ST_MODE == 0
   asm volatile("st.global.L1::no_allocate.v2.f32 [%0], {%1, %2};" ::"l"(p), "f"(v.x), "f"(v.y) : "memory");
-#elif B200_ST_MODE == 1
-  asm volatile("st.global.v2.f32 [%0], {%1, %2};" ::"l"(p), "f"(v.x), "f"(v.y) : "memory");
-#elif B200_ST_MODE == 2
-  asm volatile("st.global.cs.v2.f32 [%0], {%1, %2};" ::"l"(p), "f"(v.x), "f"(v.y) : "memory");
-#elif B200_ST_MODE == 3
-  asm volatile("st.global.cg.v2.f32 [%0], {%1, %2};" ::"l"(p), "f"(v.x), "f"(v.y) : "memory");
-#elif B200_ST_MODE == 4
-  asm volatile("st.global.L2::evict_first.v2.f32 [%0], {%1, %2};" ::"l"(p), "f"(v.x), "f"(v.y) : "memory");
-#endif
 }
 __device__ __forceinline__ void st_stream_u4(void* p, uint4 v) {
   asm volatile("st.global.L1::no_allocate.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w)

@@ -243,6 +243,15 @@ def test_bf16_split_operand(host_engine):
     assert not Wb_hi[nf:].any() and not Wb_lo[nf:].any()
 
 
+def test_slab_request_is_capped(host_engine):
+    """A slab wider than the forward GEMMs' work lists hold (40960 bodies) plans exactly like the widest slab."""
+    lib, h, B = _lib.load(), host_engine.handle, 65536
+    assert lib.b200smpl_saved_bytes(h, B, 65536) == lib.b200smpl_saved_bytes(h, B, 40960)
+    for mode in _lib.MODES.values():
+        assert lib.b200smpl_forward_workspace_bytes(h, B, mode, 65536) == lib.b200smpl_forward_workspace_bytes(h, B, mode, 40960)
+        assert lib.b200smpl_backward_workspace_bytes(h, B, mode, 65536) == lib.b200smpl_backward_workspace_bytes(h, B, mode, 40960)
+
+
 def test_forward_gemm_worklist_covers_every_tile_once():
     """Host arithmetic of the forward blend GEMM's cluster work list (no device): for every slab width and row
     range, every (body-tile pair, row-tile pair) is covered exactly once, no cluster is empty, the list fits one
@@ -253,7 +262,7 @@ def test_forward_gemm_worklist_covers_every_tile_once():
     buf = (ctypes.c_uint16 * (3 * cap))()
     for num_sms in (148, 132, 2):
         tpcs = max(1, num_sms // 2)
-        for body_tiles in (1, 2, 3, 8, 15, 16, 29, 30, 31, 32, 64):
+        for body_tiles in (1, 2, 3, 8, 15, 16, 29, 30, 31, 32, 64, 319, 320):   # 320 = the widest slab, 40960 bodies
             for row_tiles in (1, 2, 3, 17, 162, 177, 178):
                 n = lib.b200smpl_debug_fwd_gemm_worklist(body_tiles, row_tiles, num_sms, ctypes.cast(buf, ctypes.c_void_p), cap)
                 bp_total, wtp_total = (body_tiles + 1) // 2, (row_tiles + 1) // 2
