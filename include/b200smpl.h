@@ -275,7 +275,7 @@ B200SMPL_API int b200smpl_fit_update(const b200smpl_fit_group* groups, int ngrou
 
 /*
  * Fused multi-task loss of the regressor training step -- replaces HomoscedasticUncertaintyWeightedMultiTaskLoss
- * (losses/multi_task_loss.py:92-130, without its silhouette term) as called at PyTorch3DTest.py:1072-1106:
+ * (losses/multi_task_loss.py:92-130, without its silhouette term; see b200smpl_silhouette_loss) as called at PyTorch3DTest.py:1072-1106:
  *   loss = sum over the present terms of  mean((pred - label)^2) * exp(-log_var_t) + log_var_t
  * terms t = 0 vertices, 1 2D joints (orthographic_project_torch(joints, cam)[:, map2d] -> undo_keypoint_normalisation
  * (proj_wh) -> both sides 2x/norm_wh - 1, optional vis mask over (body, joint) pairs), 2 3D joints (joints[:, map3d]),
@@ -309,6 +309,43 @@ B200SMPL_API int b200smpl_multitask_loss(const b200smpl_multitask_loss_args* arg
 B200SMPL_API int b200smpl_multitask_loss_backward(const b200smpl_multitask_loss_args* args, const float* grad_loss,
                                                   float* grad_verts, float* grad_joints, float* grad_cam,
                                                   float* grad_shape, float* grad_pose, void* stream);
+
+/*
+ * Batched silhouette rasteriser of posed meshes -- replaces the reference's neural-renderer call
+ * nmr(vertices, faces, t) (player_recon.py:1226-1229, 1084-1087) and pytorch3d's SoftSilhouetteShader
+ * (PyTorch3DTest.py:64-238).  Definition (DESIGN.md section 11):
+ *   camera   R = I, t = cam_t[b], K = [[f,0,S/2],[0,f,S/2],[0,0,1]] at S = img_wh:
+ *            u = f (x+tx)/(z+tz) + S/2, v = f (y+ty)/(z+tz) + S/2; alpha[b][i][j] is the pixel centred at
+ *            (u, v) = (j + 0.5, i + 0.5), no vertical flip;
+ *   dropped  faces with a vertex at z+tz <= 1e-3 or |projected signed area| < 1e-8 px^2; winding is ignored;
+ *   hard     sigma == 0: 1 where the pixel centre is inside or on the boundary of a kept face, else 0;
+ *   soft     sigma  > 0 (px^2): D_f = sigmoid(+d^2/sigma) inside, sigmoid(-d^2/sigma) outside, d = distance to the
+ *            face's nearest edge segment; an outside face with d^2 > sigma ln(1/1e-4 - 1) contributes nothing;
+ *            alpha = 1 - prod_f (1 - D_f).
+ * vertices [B][V][3], cam_t [B][3], faces [F][3] device int32 (V <= 65535; the projected vertices, a face list and,
+ * for the backward, a per-vertex gradient accumulator must fit in one CTA's shared memory: SMPL needs 193 KB).
+ * The backward is the exact derivative w.r.t. vertices and cam_t; the hard mode has none (B200SMPL_ERR_INVALID).
+ * grad_vertices [B][V][3] and grad_t [B][3] are written, not accumulated.
+ * silhouette_loss: loss_per_body[b] += weight * mean over the S^2 pixels of (alpha - target)^2 (target [B][S][S]
+ * uint8, non-zero = inside), with the gradient of that term written to grad_vertices / grad_t; it never writes the
+ * image.  The call adds into loss_per_body so that it can follow b200smpl_fit_loss on the same buffer.
+ * No workspace is needed at present (workspace_bytes returns 0; the fields may be NULL / 0).
+ */
+typedef struct b200smpl_silhouette_args {
+  int32_t batch, num_verts, num_faces, img_wh;
+  float focal_length, sigma;
+  const float* vertices;         /* [B][V][3] */
+  const float* cam_t;            /* [B][3] camera translation */
+  const int32_t* faces;          /* [F][3] */
+  void* workspace;
+  size_t workspace_bytes;
+} b200smpl_silhouette_args;
+B200SMPL_API size_t b200smpl_silhouette_workspace_bytes(const b200smpl_silhouette_args* args);
+B200SMPL_API int b200smpl_silhouette_render(const b200smpl_silhouette_args* args, float* alpha, void* stream);
+B200SMPL_API int b200smpl_silhouette_render_backward(const b200smpl_silhouette_args* args, const float* grad_alpha,
+                                                     float* grad_vertices, float* grad_t, void* stream);
+B200SMPL_API int b200smpl_silhouette_loss(const b200smpl_silhouette_args* args, const uint8_t* target, float weight,
+                                          float* loss_per_body, float* grad_vertices, float* grad_t, void* stream);
 
 /* Test hook (host arithmetic only, no device): the cluster work list of the forward blend GEMM for `body_tiles`
  * 128-body tiles x `row_tiles` 128-row tiles on a device with `num_sms` SMs.  Writes (body-tile pair, first row-tile

@@ -80,6 +80,15 @@ class MultiTaskLossArgs(Structure):
     ]
 
 
+class SilhouetteArgs(Structure):
+    _fields_ = [
+        ("batch", c_int32), ("num_verts", c_int32), ("num_faces", c_int32), ("img_wh", c_int32),
+        ("focal_length", c_float), ("sigma", c_float),
+        ("vertices", c_void_p), ("cam_t", c_void_p), ("faces", c_void_p),
+        ("workspace", c_void_p), ("workspace_bytes", c_size_t),
+    ]
+
+
 # every symbol include/b200smpl.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "b200smpl_model_create": (c_int, [POINTER(ModelDesc), c_int, POINTER(c_void_p)]),
@@ -118,7 +127,12 @@ SYMBOLS = {
     "b200smpl_multitask_loss": (c_int, [POINTER(MultiTaskLossArgs), c_void_p, c_void_p]),
     "b200smpl_multitask_loss_backward": (c_int, [POINTER(MultiTaskLossArgs), c_void_p, c_void_p, c_void_p, c_void_p,
                                                  c_void_p, c_void_p, c_void_p]),
-    "b200smpl_debug_fwd_gemm_worklist": (c_int, [c_int, c_int, c_int, c_void_p, c_int]),
+    "b200smpl_silhouette_workspace_bytes": (c_size_t, [POINTER(SilhouetteArgs)]),
+    "b200smpl_silhouette_render": (c_int, [POINTER(SilhouetteArgs), c_void_p, c_void_p]),
+    "b200smpl_silhouette_render_backward": (c_int, [POINTER(SilhouetteArgs), c_void_p, c_void_p, c_void_p, c_void_p]),
+    "b200smpl_silhouette_loss": (c_int, [POINTER(SilhouetteArgs), c_void_p, c_float, c_void_p, c_void_p, c_void_p,
+                                         c_void_p]),
+    "b200smpl_debug_fwd_gemm_worklist":(c_int, [c_int, c_int, c_int, c_void_p, c_int]),
     "b200smpl_last_error": (c_char_p, []),
     "b200smpl_abi_version": (c_int, []),
     "b200smpl_launch_count": (c_int64, []),

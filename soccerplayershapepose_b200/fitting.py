@@ -10,7 +10,9 @@ Restates the optimisation loop of the reference's `single_view_optimization`
     `orthographic_project_torch` and `undo_keypoint_normalisation` (player_recon.py:1217-1221,
     losses/multi_task_loss.py:97-113), optionally plus a shape prior `shape_weight * mean(betas^2)`
     (BASELINE.json asks for one; the reference loop has none -- default 0 reproduces the reference);
-    the silhouette term of the reference needs its neural renderer and is out of scope (SURVEY.md section 8);
+    optionally plus a silhouette term `silhouette_weight * mean over pixels of (alpha - target)^2` on the soft
+    silhouette of the posed mesh (player_recon.py:1226-1229 renders it with the neural renderer; here the
+    rasteriser of csrc/silhouette.cu, DESIGN.md section 11) when `fit(..., silhouettes=...)` is given;
   * optimiser: `torch.optim.Adam(params, lr)` arithmetic (player_recon.py:1199), elementwise, so a batch of
     players with a summed loss is exactly a set of independent per-player optimisations;
   * the best iterate per player is kept (player_recon.py:1254-1266) -- here on the device, by loss value,
@@ -18,9 +20,12 @@ Restates the optimisation loop of the reference's `single_view_optimization`
   * results under the reference's `.npz` keys (player_recon.py:1293-1294): body_pose, global_orient, betas,
     translation (`convert_weak_perspective_to_camera_translation`, cam_utils.py:44-52).
 
-Only the joints are computed (virtual rows of the blend GEMM, no vertex is skinned).  One iteration = 7 kernel
-launches through the C-ABI (the backward reuses the forward's transforms and blend rows); after one eager iteration, twenty consecutive iterations are captured in one CUDA
-graph (kept, with its state buffers, for later calls of the same shape) and replayed.
+Without silhouettes only the joints are computed (virtual rows of the blend GEMM, no vertex is skinned).  One
+iteration = 7 kernel launches through the C-ABI (the backward reuses the forward's transforms and blend rows); after
+one eager iteration, twenty consecutive iterations are captured in one CUDA graph (kept, with its state buffers, for
+later calls of the same shape) and replayed.  With silhouettes an iteration is the full-vertex forward, fit_loss, the
+fused silhouette loss (forward, loss and backward in one kernel), the backward with vertex and joint gradients and
+fit_update, with the camera-translation gradient chained into the camera's Adam step; it is captured the same way.
 CUDA float32 only: there is no CPU path.
 """
 from __future__ import annotations
@@ -41,7 +46,11 @@ class BatchedFitter:
     def __init__(self, smpl: SMPL, lr: float = 1e-3, shape_weight: float = 0.0, joints2d_log_var: float = 0.0,
                  proj_wh: float = 512.0, norm_wh: float = float(config.REGRESSOR_IMG_WH),
                  betas: tuple = (0.9, 0.999), eps: float = 1e-8, use_cuda_graph: bool = True,
-                 frozen_joints=FROZEN_FULL_JOINTS, mode: Optional[str] = None, graph_iterations: int = 20):
+                 frozen_joints=FROZEN_FULL_JOINTS, mode: Optional[str] = None, graph_iterations: int = 20,
+                 silhouette_weight: float = 0.0, silhouette_sigma: float = 1.0, silhouette_wh: int = 256):
+        """silhouette_weight > 0 adds the silhouette term to the loss of every player when `fit` receives target
+        silhouettes (silhouette_wh x silhouette_wh masks); silhouette_sigma (px^2 at that resolution) is the blur of
+        the soft silhouette (SMPL.render_silhouettes frames the image like the `proj_wh` crop)."""
         dev = next(smpl.buffers()).device
         if dev.type != "cuda":
             raise RuntimeError("BatchedFitter needs the SMPL module on a CUDA device (no CPU path)")
@@ -59,6 +68,10 @@ class BatchedFitter:
         for j in frozen_joints:
             frozen[j] = 1
         self.frozen_rot = frozen.reshape(-1).to(dev)
+        self.sil_weight, self.sil_sigma, self.sil_wh = float(silhouette_weight), float(silhouette_sigma), int(silhouette_wh)
+        if self.sil_weight > 0.0 and not self.sil_sigma > 0.0:
+            raise ValueError("the silhouette term needs silhouette_sigma > 0 (the hard silhouette has no gradient)")
+        self.faces = smpl.faces_int32(dev)
         self._cache = {}
         self._state = None
         self._parity = 0
@@ -67,9 +80,10 @@ class BatchedFitter:
     def _iteration(self, st: Dict[str, torch.Tensor]) -> None:
         lib, B = self.lib, st["rot"].shape[0]
         stream = ctypes.c_void_p(torch.cuda.current_stream(self.dev).cuda_stream)
+        sil = "sil" in st
         # the transforms and the virtual rows of the blend output are kept for the backward (no recomputation)
-        _, joints, _, saved = self.eng.forward(st["betas"], st["rot"], None, None, axis_angle=False, mode=self.mode,
-                                               want_vertices=False, save=True, saved_buffer=st.get("saved"))
+        verts, joints, _, saved = self.eng.forward(st["betas"], st["rot"], None, None, axis_angle=False, mode=self.mode,
+                                                   want_vertices=sil, save=True, saved_buffer=st.get("saved"))
         st["saved"] = saved
         vis = st.get("vis")
         _lib.check(lib.b200smpl_fit_loss(
@@ -77,13 +91,15 @@ class BatchedFitter:
             None if vis is None else vis.data_ptr(), st["betas"].data_ptr(), B, joints.shape[1], self.jmap.numel(),
             st["betas"].shape[1], self.proj_wh, self.norm_wh, self.log_var, self.shape_weight, st["loss"].data_ptr(),
             st["gj"].data_ptr(), st["gcam"].data_ptr(), st["gbetas_prior"].data_ptr(), stream), "fit_loss")
-        gb, gp, _, _ = self.eng.backward(st["betas"], st["rot"], None, None, None, None, st["gj"], None,
-                                         axis_angle=False, mode=self.mode, need_transl=False, need_cam=False, saved=saved)
+        cam_extra = self._silhouette_term(st, verts, stream) if sil else None
+        gb, gp, _, _ = self.eng.backward(st["betas"], st["rot"], None, None, None, st["gv"] if sil else None, st["gj"],
+                                         None, axis_angle=False, mode=self.mode, need_transl=False, need_cam=False,
+                                         saved=saved)
         # best-iterate bookkeeping + the Adam step of the three parameter tensors: one launch
         groups = (_lib.FitGroup * 3)()
         for k, (name, grad, extra, frozen) in enumerate((("rot", gp, None, self.frozen_rot),
                                                          ("betas", gb, st["gbetas_prior"], None),
-                                                         ("cam", st["gcam"], None, None))):
+                                                         ("cam", st["gcam"], cam_extra, None))):
             p = st[name]
             groups[k] = _lib.FitGroup(p.data_ptr(), grad.data_ptr(), None if extra is None else extra.data_ptr(),
                                       st["m_" + name].data_ptr(), st["v_" + name].data_ptr(), st["best_" + name].data_ptr(),
@@ -94,15 +110,50 @@ class BatchedFitter:
                    "fit_update")
         self._parity ^= 1
 
+    def _silhouette_term(self, st: Dict[str, torch.Tensor], verts: torch.Tensor, stream) -> torch.Tensor:
+        """Adds the silhouette term to st['loss'], writes d loss / d vertices to st['gv'] and returns d loss / d cam
+        through t = [tx, ty, 2 f / (proj_wh s + 1e-9)] (cam_utils.py:44-52), the cam group's extra gradient."""
+        cam, t, gt, gce = st["cam"], st["t"], st["gt"], st["gcam_sil"]
+        f = config.FOCAL_LENGTH
+        den = self.proj_wh * cam[:, 0] + 1e-9
+        t[:, :2] = cam[:, 1:]
+        t[:, 2] = (2 * f) / den
+        from .ops import silhouette_args
+        args = silhouette_args(verts, self.faces, t, self.sil_wh, f * self.sil_wh / self.proj_wh, self.sil_sigma)
+        _lib.check(self.lib.b200smpl_silhouette_loss(ctypes.byref(args), st["sil"].data_ptr(), self.sil_weight,
+                                                     st["loss"].data_ptr(), st["gv"].data_ptr(), gt.data_ptr(), stream),
+                   "silhouette_loss")
+        gce[:, 0] = -gt[:, 2] * (2 * f * self.proj_wh) / (den * den)
+        gce[:, 1:] = gt[:, :2]
+        return gce
+
+    def silhouette_iou(self, rotmats: torch.Tensor, betas: torch.Tensor, cam: torch.Tensor,
+                       silhouettes: torch.Tensor) -> torch.Tensor:
+        """IoU (B,) of the binary silhouettes of the given parameters against `silhouettes` (ops.silhouette_iou)."""
+        from .ops import silhouette_iou
+        B = rotmats.shape[0]
+        verts, _, _ = self.eng.forward(betas.float().contiguous(), rotmats.float().reshape(B, 216).contiguous(), None,
+                                       None, axis_angle=False, mode=self.mode)
+        alpha = self.smpl.render_silhouettes(verts, cam.float(), img_wh=silhouettes.shape[-1], sigma=0.0,
+                                             proj_wh=self.proj_wh)
+        return silhouette_iou(alpha, silhouettes.to(alpha.device))
+
     def fit(self, rotmats: torch.Tensor, betas: torch.Tensor, cam: torch.Tensor, keypoints2d: torch.Tensor,
-            vis: Optional[torch.Tensor] = None, iterations: int = 200) -> Dict[str, torch.Tensor]:
+            vis: Optional[torch.Tensor] = None, iterations: int = 200,
+            silhouettes: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
         """rotmats (B,24,3,3) initial pose, betas (B,10), cam (B,3) weak-perspective [s,tx,ty], keypoints2d
-        (B,17,2) target COCO keypoints in pixels of the `proj_wh` image, vis (B,17) bool or None."""
+        (B,17,2) target COCO keypoints in pixels of the `proj_wh` image, vis (B,17) bool or None.
+        silhouettes (B, silhouette_wh, silhouette_wh) target masks or None: with silhouette_weight > 0 the loss gains
+        the silhouette term; either way the result then carries `silhouette_iou` of the best iterate."""
         dev = self.dev
         B = rotmats.shape[0]
         f32 = dict(dtype=torch.float32, device=dev)
+        use_sil = silhouettes is not None and self.sil_weight > 0.0
+        if silhouettes is not None and tuple(silhouettes.shape) != (B, self.sil_wh, self.sil_wh):
+            raise ValueError("silhouettes has shape {}, expected {}".format(tuple(silhouettes.shape),
+                                                                           (B, self.sil_wh, self.sil_wh)))
         # the state buffers (and the graph captured over them) are kept per problem shape and reused by later calls
-        key = (B, int(betas.shape[1]), vis is not None)
+        key = (B, int(betas.shape[1]), vis is not None) + (("sil",) if use_sil else ())
         cached = self._cache.get(key)
         if cached is None:
             st = {"rot": torch.empty((B, 216), **f32), "betas": torch.empty((B, betas.shape[1]), **f32),
@@ -122,6 +173,11 @@ class BatchedFitter:
             st["gj"] = torch.empty((B, self.eng.num_joints_out, 3), **f32)
             st["gcam"] = torch.empty((B, 3), **f32)
             st["gbetas_prior"] = torch.empty((B, betas.shape[1]), **f32)
+            if use_sil:
+                st["sil"] = torch.empty((B, self.sil_wh, self.sil_wh), dtype=torch.uint8, device=dev)
+                st["gv"] = torch.empty((B, self.eng.num_verts, 3), **f32)
+                for name in ("t", "gt", "gcam_sil"):
+                    st[name] = torch.empty((B, 3), **f32)
             cached = {"st": st, "graph": None, "per": 0}
             self._cache[key] = cached
         st = cached["st"]
@@ -131,6 +187,8 @@ class BatchedFitter:
         st["label"].copy_(keypoints2d.to(**f32))
         if vis is not None:
             st["vis"].copy_(vis.to(device=dev, dtype=torch.uint8))
+        if use_sil:
+            st["sil"].copy_(silhouettes.to(device=dev) != 0)
         for name in ("rot", "betas", "cam"):
             st["m_" + name].zero_()
             st["v_" + name].zero_()
@@ -179,6 +237,8 @@ class BatchedFitter:
                "best_loss": st["best_loss"].clone(), "best_iter": st["best_iter"].clone(), "initial_loss": first_loss,
                "final_rotmats": st["rot"].reshape(B, 24, 3, 3).clone(), "final_betas": st["betas"].clone(),
                "final_cam": st["cam"].clone(), "last_loss": st["loss"].clone()}
+        if silhouettes is not None:
+            out["silhouette_iou"] = self.silhouette_iou(best_rot, st["best_betas"], st["best_cam"], silhouettes)
         self._state = st
         return out
 
@@ -197,7 +257,7 @@ class MultiViewFitter:
     (the `is_train = False` pass) and the parameters of the epoch are kept when the summed validation loss is the
     best the player has seen in any phase so far (:1823-1838, 1938-1954); each phase ends by restoring its
     parameters to their best epoch (:1846-1847, 1961-1962).  Differences, stated: the loss is the joints2D term only
-    (the silhouette term needs the reference's renderer), model selection uses that loss instead of the
+    (the silhouette term of `BatchedFitter` is not wired into this loop), model selection uses that loss instead of the
     metrics tracker's joints2D / silhouette metrics, and the shuffled view order of an epoch is shared by all
     players of the batch (the reference shuffles per player).
 

@@ -8,7 +8,7 @@ from typing import Optional
 
 import torch
 
-from . import _lib
+from . import _lib, config
 
 
 def _stream(t: torch.Tensor) -> ctypes.c_void_p:
@@ -342,3 +342,129 @@ def multitask_loss(log_var: torch.Tensor, *, verts=None, verts_label=None, joint
     evaluated when its prediction (its joint map for the joint terms) is given.  Returns (loss, parts (5,))."""
     return _MultiTaskLoss.apply(log_var, verts, joints, cam, shape, pose, verts_label, map2d, label2d, vis, map3d,
                                 label3d, shape_label, pose_label, proj_wh, norm_wh)
+
+
+# ---- silhouettes (DESIGN.md section 11) ------------------------------------------------------------------------------
+_FACES_I32 = {}
+
+
+def _faces_int32(faces: torch.Tensor, device: torch.device, V: int) -> torch.Tensor:
+    """(F,3) integer faces as contiguous int32 on `device`, range-checked once per (tensor, version) like the joint
+    maps (the kernels drop a face with an out-of-range index, but a wrong topology should fail loudly)."""
+    if not isinstance(faces, torch.Tensor):
+        faces = torch.as_tensor(faces)
+    if faces.dim() != 2 or faces.shape[1] != 3:
+        raise ValueError("faces has shape {}, expected (F, 3)".format(tuple(faces.shape)))
+    if faces.dtype.is_floating_point or faces.dtype == torch.bool:
+        raise TypeError("faces must be an integer tensor, got {}".format(faces.dtype))
+    key = (faces.data_ptr(), faces.numel(), faces._version, str(faces.dtype), str(faces.device), str(device), V)
+    hit = _FACES_I32.get(key)
+    if hit is not None and hit[0]() is faces:
+        return hit[1]
+    f32 = faces.to(device=device, dtype=torch.int32).contiguous()
+    if torch.cuda.is_current_stream_capturing():
+        return f32
+    if f32.numel() and (int(f32.min()) < 0 or int(f32.max()) >= V):
+        raise IndexError("faces entries must lie in [0, {})".format(V))
+    if len(_FACES_I32) > 64:
+        _FACES_I32.clear()
+    _FACES_I32[key] = (weakref.ref(faces), f32)
+    return f32
+
+
+def silhouette_args(vertices: torch.Tensor, faces32: torch.Tensor, cam_t: torch.Tensor, img_wh: int,
+                    focal_length: float, sigma: float) -> "_lib.SilhouetteArgs":
+    """The C-ABI argument struct over caller-owned device tensors (kept alive by the caller)."""
+    B, V = vertices.shape[0], vertices.shape[1]
+    if vertices.dim() != 3 or vertices.shape[2] != 3:
+        raise ValueError("vertices has shape {}, expected (B, V, 3)".format(tuple(vertices.shape)))
+    if tuple(cam_t.shape) != (B, 3):
+        raise ValueError("cam_t has shape {}, expected {}".format(tuple(cam_t.shape), (B, 3)))
+    if cam_t.device != vertices.device or faces32.device != vertices.device:
+        raise RuntimeError("vertices, faces and cam_t must be on the same device")
+    if int(img_wh) < 1 or not float(sigma) >= 0.0:
+        raise ValueError("need img_wh >= 1 and sigma >= 0")
+    return _lib.SilhouetteArgs(batch=B, num_verts=V, num_faces=faces32.shape[0], img_wh=int(img_wh),
+                               focal_length=float(focal_length), sigma=float(sigma), vertices=vertices.data_ptr(),
+                               cam_t=cam_t.data_ptr(), faces=faces32.data_ptr(), workspace=None, workspace_bytes=0)
+
+
+class _Silhouette(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, vertices, cam_t, faces32, img_wh, focal_length, sigma):
+        vertices, cam_t = _req(vertices, "vertices"), _req(cam_t, "cam_t")
+        args = silhouette_args(vertices, faces32, cam_t, img_wh, focal_length, sigma)
+        B, S = vertices.shape[0], int(img_wh)
+        alpha = torch.empty((B, S, S), dtype=torch.float32, device=vertices.device)
+        with torch.cuda.device(vertices.device):
+            _lib.check(_lib.load().b200smpl_silhouette_render(ctypes.byref(args), alpha.data_ptr(), _stream(vertices)),
+                       "silhouette_render")
+        ctx.save_for_backward(vertices, cam_t, faces32)
+        ctx.img_wh, ctx.focal_length, ctx.sigma = S, float(focal_length), float(sigma)
+        if sigma == 0.0:
+            ctx.mark_non_differentiable(alpha)
+        return alpha
+
+    @staticmethod
+    def backward(ctx, g):
+        vertices, cam_t, faces32 = ctx.saved_tensors
+        args = silhouette_args(vertices, faces32, cam_t, ctx.img_wh, ctx.focal_length, ctx.sigma)
+        g = g.contiguous().float()
+        gv = torch.empty_like(vertices)
+        gt = torch.empty_like(cam_t)
+        with torch.cuda.device(vertices.device):
+            _lib.check(_lib.load().b200smpl_silhouette_render_backward(
+                ctypes.byref(args), g.data_ptr(), gv.data_ptr(), gt.data_ptr(), _stream(vertices)),
+                "silhouette_render_backward")
+        return gv, gt, None, None, None, None
+
+
+def render_silhouettes(vertices: torch.Tensor, faces, cam_t: torch.Tensor, img_wh: int,
+                       focal_length: float = config.FOCAL_LENGTH, sigma: float = 0.0) -> torch.Tensor:
+    """Silhouettes (B, S, S) of the meshes `vertices` (B,V,3) / `faces` (F,3) seen through the camera of the
+    reference's neural-renderer call nmr(vertices, faces, t) (player_recon.py:1226-1229): R = I, translation `cam_t`
+    (B,3), K = [[f,0,S/2],[0,f,S/2],[0,0,1]], S = img_wh.  Element [i, j] is the pixel centred at (j + 0.5, i + 0.5)
+    with u = f (x+tx)/(z+tz) + S/2 and v likewise -- what cam_utils.perspective_project_torch returns -- and no
+    vertical flip (the orientation of the reference's renderer could not be checked; use torch.flip if a caller
+    needs the other one).  sigma == 0: binary coverage, no gradient (a backward raises ValueError).  sigma > 0 (px^2):
+    the SoftRas / SoftSilhouetteShader soft silhouette, differentiable w.r.t. `vertices` and `cam_t`."""
+    vertices = _req(vertices, "vertices")
+    faces32 = _faces_int32(faces, vertices.device, vertices.shape[1])
+    return _Silhouette.apply(vertices, cam_t, faces32, int(img_wh), float(focal_length), float(sigma))
+
+
+def silhouette_loss(vertices: torch.Tensor, faces, cam_t: torch.Tensor, target: torch.Tensor, img_wh: int,
+                    focal_length: float = config.FOCAL_LENGTH, sigma: float = 1.0, weight: float = 1.0,
+                    loss_per_body: Optional[torch.Tensor] = None):
+    """Fused silhouette term of the fitting loop (one kernel; the image is never written):
+    loss_per_body[b] += weight * mean over the S^2 pixels of (alpha_b - target_b)^2, target (B,S,S) mask.  Returns
+    (loss_per_body, grad_vertices, grad_cam_t) -- plain tensors, no autograd.  The form of the reference's silhouette
+    loss term (losses/multi_task_loss.py:132-144) could not be read; this squared error is the stated definition."""
+    vertices, cam_t = _req(vertices, "vertices"), _req(cam_t, "cam_t")
+    B = vertices.shape[0]
+    faces32 = _faces_int32(faces, vertices.device, vertices.shape[1])
+    args = silhouette_args(vertices, faces32, cam_t, img_wh, focal_length, sigma)
+    S = int(img_wh)
+    if tuple(target.shape) != (B, S, S):
+        raise ValueError("target has shape {}, expected {}".format(tuple(target.shape), (B, S, S)))
+    tgt = target.to(device=vertices.device, dtype=torch.uint8).contiguous()
+    if loss_per_body is None:
+        loss_per_body = torch.zeros(B, dtype=torch.float32, device=vertices.device)
+    gv = torch.empty_like(vertices)
+    gt = torch.empty_like(cam_t)
+    with torch.cuda.device(vertices.device):
+        _lib.check(_lib.load().b200smpl_silhouette_loss(ctypes.byref(args), tgt.data_ptr(), float(weight),
+                                                        loss_per_body.data_ptr(), gv.data_ptr(), gt.data_ptr(),
+                                                        _stream(vertices)), "silhouette_loss")
+    return loss_per_body, gv, gt
+
+
+def silhouette_iou(pred: torch.Tensor, target: torch.Tensor) -> torch.Tensor:
+    """IoU per body of compute_silh_error_metrics (metrics/silhouettes_joints_metrics.py:5-37) on masks
+    `alpha >= 0.5`: (B,S,S) x (B,S,S) -> (B,).  A metric, not on the hot path: plain torch ops.  An empty union
+    gives IoU 1."""
+    p = pred >= 0.5 if pred.dtype.is_floating_point else pred.bool()
+    t = target >= 0.5 if target.dtype.is_floating_point else target.bool()
+    inter = (p & t).flatten(1).sum(1).double()
+    union = (p | t).flatten(1).sum(1).double()
+    return torch.where(union > 0, inter / union.clamp(min=1), torch.ones_like(union)).float()

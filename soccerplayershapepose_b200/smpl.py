@@ -195,6 +195,31 @@ class SMPL(nn.Module):
         t = convert_weak_perspective_to_camera_translation_torch(cam_wp, config.FOCAL_LENGTH, proj_wh)
         return {"vertices": vertices.contiguous(), "faces": faces[None].expand(B, -1, -1), "t": t.unsqueeze(1)}
 
+    def faces_int32(self, device: torch.device) -> torch.Tensor:
+        """The model's faces (F,3) as int32 on `device`, uploaded once per device."""
+        device = torch.device(device)
+        cache = self.__dict__.setdefault("_faces_dev", {})
+        f = cache.get(device)
+        if f is None:
+            f = torch.from_numpy(np.ascontiguousarray(self.faces, dtype=np.int32)).to(device)
+            cache[device] = f
+        return f
+
+    def render_silhouettes(self, vertices: torch.Tensor, cam_wp: torch.Tensor, img_wh: int = 256, sigma: float = 0.0,
+                           proj_wh: float = 512.0, focal_length: Optional[float] = None) -> torch.Tensor:
+        """Silhouettes (B, img_wh, img_wh) of posed meshes (ops.render_silhouettes) with the camera translation
+        built as `silhouette_inputs` builds it from the weak-perspective camera [s, tx, ty] of the `proj_wh`-pixel
+        crop: t = [tx, ty, 2 f / (proj_wh s)], f = config.FOCAL_LENGTH.  The render focal length defaults to
+        f * img_wh / proj_wh, so the image frames the same view as that crop at any resolution (img_wh = proj_wh
+        renders at f itself).  sigma == 0: binary; sigma > 0: soft, differentiable into `vertices` (and through
+        SMPLFunction into betas / pose) and `cam_wp`."""
+        from . import config, ops
+        from .cam_utils import convert_weak_perspective_to_camera_translation_torch
+        t = convert_weak_perspective_to_camera_translation_torch(cam_wp, config.FOCAL_LENGTH, proj_wh)
+        f = config.FOCAL_LENGTH * float(img_wh) / float(proj_wh) if focal_length is None else float(focal_length)
+        return ops.render_silhouettes(vertices, self.faces_int32(vertices.device), t.contiguous(), img_wh,
+                                      focal_length=f, sigma=sigma)
+
 
 class SMPLLayer(SMPL):
     """north_star surface: forward(betas, pose, trans) -> (vertices, joints).
