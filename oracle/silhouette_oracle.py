@@ -139,7 +139,7 @@ def edge_distance(vertices, faces, cam_t, img_wh, focal_length, b, rows, cols):
         tri, kept, _ = face_table(vertices[b:b + 1], cam_t[b:b + 1], faces, focal_length, img_wh)
         tri = tri[0][kept[0]]
         p = torch.stack([cols, rows], -1).to(tri.dtype) + 0.5
-        best = torch.full((p.shape[0],), float("inf"), dtype=tri.dtype)
+        best = torch.full((p.shape[0],), float("inf"), dtype=tri.dtype, device=tri.device)
         for s in range(0, tri.shape[0], 4096):
             d2 = _edge_d2(tri[None, s:s + 4096], p[:, None, :])
             best = torch.minimum(best, d2.min(1).values)
