@@ -101,7 +101,7 @@ static Plan make_plan(const b200smpl_model* m, int batch, int mode, int slab_bod
   p.saved_slab_bytes = align_up((size_t)NJ * AELEMS * S_ * 4, 1024) + align_up((size_t)d.n_pad * S_ * 4, 1024);
   if (backward) {
     const int bmode = bwd_gemm_mode(mode);
-    p.k_splits = bmode == B200SMPL_MODE_FP32_SIMT ? 1 : blend_bwd_umma_splits(d, bmode, p.S, m->num_sms);
+    p.k_splits = bmode == B200SMPL_MODE_FP32_SIMT ? 1 : blend_bwd_umma_splits(d, p.S, m->num_sms);
     p.off_dvp_hi = take(S_ * d.n_pad * 2);
     p.off_dvp_lo = take(bmode == B200SMPL_MODE_BF16 ? 0 : S_ * d.n_pad * 2);
     // dA accumulator [S/32][288][32] directly followed by the dtransl accumulator [S/32][3][32]

@@ -10,10 +10,11 @@
 // error-compensated split laid out along K (see FeatLayout in common.cuh), so the tensor pipe only
 // ever sees kind::f16 MMAs with fp32 accumulation in TMEM.
 //
-// CTA = 6 warps: warp 0 TMA producer, warp 1 MMA issuer (+ TMEM alloc), warps 2-5 epilogue
-// (tcgen05.ld -> registers -> 16-byte global stores).  One 128 x BN output tile per CTA; smem ring
-// of STAGES x (128x64 + BNx64) bf16 tiles in the 128-byte swizzle; two CTAs can share an SM in
-// the forward configuration so one CTA's epilogue overlaps the other's main loop.
+// Both GEMMs run on CTA pairs (tcgen05 cta_group::2, cluster of 2): M = 256 bodies, 128 per CTA, and each
+// CTA holds half of the model operand, which halves the per-SM shared-memory operand traffic that bounds a
+// single-CTA tensor-core GEMM of this shape.  CTA = 6 warps: warp 0 TMA producer, warp 1 MMA issuer (+ TMEM
+// alloc; only the leader of the pair issues), warps 2-5 epilogue (tcgen05.ld -> registers -> 16-byte global
+// stores).  Operand stages are bf16 tiles of 64 K elements in the 128-byte swizzle.
 #include <cuda.h>
 #include <algorithm>
 
@@ -21,157 +22,28 @@
 
 namespace b200smpl {
 
-
-template <int BN, int STAGES>
-struct GemmSmem {
-  static constexpr int A_BYTES = BM * BK * 2;
-  static constexpr int B_BYTES = BN * BK * 2;
-  static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  static constexpr int TOTAL = STAGES * STAGE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/;
-};
-
-// Backward (data-gradient) GEMM.  grid: (body tiles of 128, 1, k splits)
-//   D[split][body][f] = sum_seg sum_{n in split} A_seg[body][n] * B_seg[f][n],   D row-major, ld = ldd
-// A stage = 8 chunks x (128 bodies x 16 B): chunk c at +2048 B  ->  LBO = 2048, SBO = 128.
-template <int BN, int STAGES>
-__global__ void __launch_bounds__(GEMM_THREADS, 1)
-umma_gemm_kernel(const __grid_constant__ GemmOps ops, int nseg, int nc8, int slab_begin, int slab_end,
-                 int slabs_per_split, float* __restrict__ D, int ldd, long long split_stride) {
-  using SM = GemmSmem<BN, STAGES>;
-  constexpr uint32_t TMEM_COLS = BN <= 32 ? 32 : (BN <= 64 ? 64 : (BN <= 128 ? 128 : 256));
-  extern __shared__ unsigned char smem_dyn[];
-  unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~(uintptr_t)1023);
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + STAGES * SM::STAGE_BYTES);
-  uint64_t* empty_bar = full_bar + STAGES;
-  uint64_t* tmem_full_bar = empty_bar + STAGES;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full_bar + 1);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int m0 = blockIdx.x * BM;
-  const int s_begin = slab_begin + blockIdx.z * slabs_per_split;
-  const int s_end = min(slab_end, s_begin + slabs_per_split);
-  const int slabs = max(0, s_end - s_begin);
-  const int total_iters = slabs * nseg;
-
-  if (warp == 0 && lane == 0) {
-    for (int s = 0; s < nseg; ++s) prefetch_tmap(&ops.b[s]);
-  }
-  if (warp == 1 && lane == 0) {
-    for (int i = 0; i < STAGES; ++i) {
-      mbar_init(&full_bar[i], 1);
-      mbar_init(&empty_bar[i], 1);
-    }
-    mbar_init(tmem_full_bar, 1);
-    fence_barrier_init();
-  }
-  if (warp == 1) {
-    __syncwarp();
-    tmem_alloc(tmem_slot, TMEM_COLS);
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    // ===== producer (whole warp walks the loop, one elected lane issues): one bulk copy (A) + one tensor-map
-    // load (B) per stage =====
-    {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int it = 0; it < total_iters; ++it) {
-        const int seg = it / slabs, slab = s_begin + (it - seg * slabs);
-        mbar_wait(&empty_bar[stage], phase ^ 1);
-        unsigned char* sa = smem + stage * SM::STAGE_BYTES;
-        unsigned char* sb = sa + SM::A_BYTES;
-        if (elect_one()) {
-        mbar_arrive_expect_tx(&full_bar[stage], SM::STAGE_BYTES);
-        // dvp [S/128][n/8][128][8]: the 8 chunks of this K slab for the 128 bodies are 16 contiguous KB
-        bulk_g2s(sa, ops.a[seg] + (((size_t)blockIdx.x * nc8 + (size_t)slab * 8) * 128) * 8, SM::A_BYTES, &full_bar[stage]);
-        tma_load_2d(sb, &ops.b[seg], &full_bar[stage], slab * BK, 0);
-        }
-        __syncwarp();
-        if (++stage == STAGES) {
-          stage = 0;
-          phase ^= 1;
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===== MMA issuer (whole warp walks the loop, one elected lane issues) =====
-    {
-      constexpr uint32_t idesc = make_idesc(BM, BN);
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int it = 0; it < total_iters; ++it) {
-        mbar_wait(&full_bar[stage], phase);
-        tc_fence_after();
-        const uint32_t sa = smem_u32(smem + stage * SM::STAGE_BYTES);
-        const uint64_t da = make_nosw_desc(sa, 2048, 128), db = make_sw128_desc(sa + SM::A_BYTES);
-        if (elect_one()) {
-#pragma unroll
-          for (int k = 0; k < BK / UMMA_K; ++k) {
-            // A: two 16-byte chunks per UMMA_K -> +4096 B; B: +32 bytes inside the swizzle row (16-byte units)
-            umma_bf16(tmem_base, da + (uint64_t)(k * (4096 >> 4)), db + 2 * k, idesc, (it | k) != 0);
-          }
-          umma_commit(&empty_bar[stage]);            // frees the smem slot when these MMAs retire
-          if (it == total_iters - 1) umma_commit(tmem_full_bar);
-        }
-        __syncwarp();
-        if (++stage == STAGES) {
-          stage = 0;
-          phase ^= 1;
-        }
-      }
-    }
-  } else {
-    // ===== epilogue: warps 2..5 own TMEM lane quadrants (warp % 4) =====
-    const int q = warp & 3;
-    const int row = m0 + q * 32 + lane;
-    float* drow = D + (long long)blockIdx.z * split_stride + (long long)row * ldd;
-    if (total_iters > 0) {
-      mbar_wait(tmem_full_bar, 0);
-      tc_fence_after();
-#pragma unroll 1
-      for (int c0 = 0; c0 < BN; c0 += 32) {
-        uint32_t v[32];
-        tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, v);
-        float* o = drow + c0;
-#pragma unroll
-        for (int i = 0; i < 32; i += 4)
-          if (c0 + i < BN)                         // BN is a multiple of 16, not of 32: the last block may be half
-            *reinterpret_cast<uint4*>(o + i) = make_uint4(v[i], v[i + 1], v[i + 2], v[i + 3]);
-      }
-    } else {
-#pragma unroll 1
-      for (int c0 = 0; c0 < BN; c0 += 4) *reinterpret_cast<uint4*>(drow + c0) = make_uint4(0u, 0u, 0u, 0u);
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, TMEM_COLS);
-  }
-}
-
 // ---------------------------------------------------------------------------------------------
-// The same GEMM on a CTA PAIR (tcgen05 cta_group::2, cluster of 2 along the body tiles): M = 256 bodies (128
-// per CTA, each CTA streams its own dvp tile and accumulates into its own TMEM), the B operand (Wb slab,
-// BN x 64) is split -- each CTA loads and holds BN/2 rows, the pair's tensor cores read both halves -- which
-// halves the per-SM shared-memory write and read traffic of B, the bound of the single-CTA kernel.
-// Only the leader (rank 0) issues MMAs; it waits for its own stage and, through a relayed remote arrive, for
-// the peer's; its commits are multicast to the barriers of both CTAs.
+// Backward (data-gradient) GEMM on a CTA PAIR (cluster of 2 along the body tiles).  grid: (body tiles rounded up
+// to even, 1, k splits)
+//   D[split][body][f] = sum_{n in split} dvp[body][n] * Wb[f][n],   D row-major, ld = ldd
+// Each CTA streams its own dvp tile and accumulates into its own TMEM; the B operand (Wb slab, BN x 64) is split --
+// each CTA loads and holds BN/2 rows, the pair's tensor cores read both halves.  Only the leader (rank 0) issues
+// MMAs; it waits for its own stage and, through a relayed remote arrive, for the peer's; its commits are multicast
+// to the barriers of both CTAs.
+// An odd number of body tiles leaves rank 1 of the last cluster without a tile: that padding CTA streams the last
+// real tile's dvp again (so the pair MMA reads defined operands) and stores nothing.
 // ---------------------------------------------------------------------------------------------
 // One stage = one 64-row K slab with everything the split needs, each loaded ONCE: dvp_hi (and dvp_lo) tiles of
 // this CTA's 128 bodies, this CTA's half of the Wb_hi (and Wb_lo) slab; the three products hi.hi, lo.hi, hi.lo
 // are issued back to back on the resident tiles (fp32 mode: 60 KB per stage, 3 stages; bf16 mode: 30 KB, 6).
+// A stage = 8 chunks x (128 bodies x 16 B): chunk c at +2048 B  ->  LBO = 2048, SBO = 128.
 template <int BN>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
-umma_gemm2_kernel(const __grid_constant__ GemmOps ops, int split3, int nc8, int slab_begin, int slab_end,
+umma_gemm2_kernel(const __grid_constant__ GemmOps ops, int split3, int ntiles, int nc8, int slab_begin, int slab_end,
                   int slabs_per_split, float* __restrict__ D, int ldd, long long split_stride) {
   constexpr int BNH = BN / 2;
   constexpr int A_BYTES = BM * BK * 2, B_BYTES = BNH * BK * 2;
+  static_assert(B_BYTES % 1024 == 0, "the 128-byte swizzle needs every stage offset 1024-byte aligned");
   constexpr int MAX_STAGES = 6;
   constexpr uint32_t TMEM_COLS = 256;
   const int stage_bytes = (split3 ? 2 : 1) * (A_BYTES + B_BYTES);
@@ -186,14 +58,15 @@ umma_gemm2_kernel(const __grid_constant__ GemmOps ops, int split3, int nc8, int 
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
+  const bool padding = (int)blockIdx.x >= ntiles;     // CTA-uniform
   const int m0 = blockIdx.x * BM;
   const int s_begin = slab_begin + blockIdx.z * slabs_per_split;
   const int s_end = min(slab_end, s_begin + slabs_per_split);
   const int total_iters = max(0, s_end - s_begin);
 
   if (warp == 0 && lane == 0) {
-    prefetch_tmap(&ops.b[0]);
-    if (split3) prefetch_tmap(&ops.b[2]);
+    prefetch_tmap(&ops.wb_hi);
+    if (split3) prefetch_tmap(&ops.wb_lo);
   }
   if (warp == 1 && lane == 0) {
     for (int i = 0; i < MAX_STAGES; ++i) {
@@ -224,6 +97,7 @@ umma_gemm2_kernel(const __grid_constant__ GemmOps ops, int split3, int nc8, int 
     // ===== producer (both CTAs): own dvp tiles + own halves of the Wb slabs =====
     // dvp is read once, the model slabs by every body pair: keep the latter in L2
     const uint64_t pol_stream = l2_policy_evict_first(), pol_keep = l2_policy_evict_last();
+    const int tile = padding ? ntiles - 1 : (int)blockIdx.x;
     int stage = 0;
     uint32_t phase = 0;
     for (int it = 0; it < total_iters; ++it) {
@@ -232,12 +106,12 @@ umma_gemm2_kernel(const __grid_constant__ GemmOps ops, int split3, int nc8, int 
       unsigned char* sa = smem + stage * stage_bytes;
       if (elect_one()) {
         mbar_arrive_expect_tx(&full_bar[stage], (uint32_t)stage_bytes);
-        const size_t aoff = (((size_t)blockIdx.x * nc8 + (size_t)slab * 8) * 128) * 8;
-        bulk_g2s_hint(sa, ops.a[0] + aoff, A_BYTES, &full_bar[stage], pol_stream);
-        tma_load_2d_hint(sa + off_bhi, &ops.b[0], &full_bar[stage], slab * BK, (int)rank * BNH, pol_keep);
+        const size_t aoff = (((size_t)tile * nc8 + (size_t)slab * 8) * 128) * 8;
+        bulk_g2s_hint(sa, ops.dvp_hi + aoff, A_BYTES, &full_bar[stage], pol_stream);
+        tma_load_2d_hint(sa + off_bhi, &ops.wb_hi, &full_bar[stage], slab * BK, (int)rank * BNH, pol_keep);
         if (split3) {
-          bulk_g2s_hint(sa + off_alo, ops.a[1] + aoff, A_BYTES, &full_bar[stage], pol_stream);
-          tma_load_2d_hint(sa + off_blo, &ops.b[2], &full_bar[stage], slab * BK, (int)rank * BNH, pol_keep);
+          bulk_g2s_hint(sa + off_alo, ops.dvp_lo + aoff, A_BYTES, &full_bar[stage], pol_stream);
+          tma_load_2d_hint(sa + off_blo, &ops.wb_lo, &full_bar[stage], slab * BK, (int)rank * BNH, pol_keep);
         }
       }
       __syncwarp();
@@ -284,8 +158,10 @@ umma_gemm2_kernel(const __grid_constant__ GemmOps ops, int split3, int nc8, int 
         if (++stage == nstages) { stage = 0; phase ^= 1; }
       }
     }
-  } else {
+  } else if (!padding) {
     // ===== epilogue: warps 2..5 own TMEM lane quadrants (warp % 4) of this CTA's 128 bodies =====
+    // (the padding CTA skips it: the leader's epilogue waits for the pair's last MMA before the cluster barrier
+    // that precedes the TMEM dealloc)
     const int q = warp & 3;
     const int row = m0 + q * 32 + lane;
     float* drow = D + (long long)blockIdx.z * split_stride + (long long)row * ldd;
@@ -559,8 +435,6 @@ int make_map(CUtensorMap* map, const void* base, int k_extent, int rows, int pit
   return 0;
 }
 
-constexpr int BWD_STAGES = 4;
-
 // Work list of the body-stationary forward GEMM (host side; pure arithmetic, also exposed to the CPU tests through
 // b200smpl_debug_fwd_gemm_worklist).  CTA pairs are scheduled per TPC (2 SMs).  The (body pair, row-tile pair) list,
 // body pair major, is cut into one equal range per TPC; a range that crosses into the next body pair becomes two
@@ -660,9 +534,8 @@ extern "C" int b200smpl_debug_fwd_gemm_worklist(int body_tiles, int row_tiles, i
 namespace b200smpl {
 
 // number of split-K partials the backward GEMM writes for slab width S
-int blend_bwd_umma_splits(const DevModel& m, int mode, int S, int num_sms) {
-  (void)mode;
-  const int mtiles = (S + BM - 1) / BM;
+int blend_bwd_umma_splits(const DevModel& m, int S, int num_sms) {
+  const int mtiles = round_up((S + BM - 1) / BM, 2);      // an odd tile count launches one padding CTA
   const int slabs = (m.n_rows + BK - 1) / BK;
   // CTA pairs are scheduled per TPC (2 SMs): never more pairs than TPCs, or a second, nearly empty wave runs
   int want = std::max(1, num_sms / mtiles);
@@ -671,36 +544,16 @@ int blend_bwd_umma_splits(const DevModel& m, int mode, int S, int num_sms) {
 }
 
 template <int BN>
-static int launch_bwd_bn(const GemmOps& ops, int nseg, int nc8, int slab_begin, int slab_end, int nsplit, int Sw,
-                         float* dfeat_part, int nf_pad, long long split_stride, cudaStream_t st) {
-  using SM = GemmSmem<BN, BWD_STAGES>;
-  auto kern = umma_gemm_kernel<BN, BWD_STAGES>;
-  B200_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SM::TOTAL));
-  const int slabs = slab_end - slab_begin;
-  const int sps = (slabs + nsplit - 1) / nsplit;
-  dim3 grid(Sw / BM, 1, nsplit);
-  LaunchTimer _timer_316("blend_bwd_umma", st);
-  kern<<<grid, GEMM_THREADS, SM::TOTAL, st>>>(ops, nseg, nc8, slab_begin, slab_end, sps, dfeat_part, nf_pad, split_stride);
-  B200_LAUNCH_CHECK("blend_bwd_umma");
-  return 0;
-}
-
-template <int BN>
-static int launch_bwd_bn_2cta(GemmOps& ops, const DevModel& m, int nseg, int row_end, int slab_begin, int slab_end,
-                              int nsplit, int Sw, float* dfeat_part, int nf_pad, long long split_stride, cudaStream_t st) {
+static int launch_bwd_pair(const GemmOps& ops, int split3, int ntiles, int nc8, int slab_begin, int slab_end,
+                           int nsplit, float* dfeat_part, long long split_stride, cudaStream_t st) {
   constexpr int smem = 6 * (BM * BK * 2 + (BN / 2) * BK * 2) + 1024 + 512;
-  // every CTA loads BN/2 rows of the Wb slab: tensor maps with that box height
-  int rc;
-  const __nv_bfloat16* bsrc[MAX_SEG] = {m.Wb_hi, m.Wb_hi, m.Wb_lo};
-  for (int s = 0; s < nseg; ++s)
-    if ((rc = make_map(&ops.b[s], bsrc[s], row_end, nf_pad, m.n_pad, BN / 2))) return rc;
   auto kern = umma_gemm2_kernel<BN>;
   B200_SMEM_ATTR_ONCE(kern, smem);
   const int slabs = slab_end - slab_begin;
   const int sps = (slabs + nsplit - 1) / nsplit;
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(Sw / BM, 1, nsplit);
+  cfg.gridDim = dim3(round_up(ntiles, 2), 1, nsplit);
   cfg.blockDim = dim3(GEMM_THREADS, 1, 1);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
@@ -714,8 +567,8 @@ static int launch_bwd_bn_2cta(GemmOps& ops, const DevModel& m, int nseg, int row
   cfg.attrs = attr;
   cfg.numAttrs = pdl_enabled() ? 2 : 1;
   LaunchTimer _timer("blend_bwd_umma", st);
-  B200_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, ops, nseg == 3 ? 1 : 0, m.n_pad / 8, slab_begin, slab_end, sps, dfeat_part,
-                                   nf_pad, split_stride));
+  B200_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, ops, split3, ntiles, nc8, slab_begin, slab_end, sps, dfeat_part, BN,
+                                   split_stride));
   B200_LAUNCH_CHECK("blend_bwd_umma");
   return 0;
 }
@@ -725,32 +578,24 @@ static int launch_bwd_bn_2cta(GemmOps& ops, const DevModel& m, int nseg, int row
 int launch_blend_bwd_umma(const DevModel& m, int mode, const __nv_bfloat16* dvp_hi, const __nv_bfloat16* dvp_lo,
                           int S, int Sw, float* dfeat_part, int nsplit, int row_begin, int row_end,
                           cudaStream_t st) {
+  // nf_pad = round_up(num_betas + NPOSE, 16): 208 for 1 beta, 224 for 2..MAX_BETAS
+  const int nf_pad = m.fl.nf_pad;
+  if (nf_pad != 208 && nf_pad != 224)
+    return fail(B200SMPL_ERR_INVALID, "unsupported num_betas for the tensor-core backward (nf_pad=" + std::to_string(nf_pad) + ")");
+  const bool split3 = (mode != B200SMPL_MODE_BF16) && dvp_lo != nullptr;
   GemmOps ops;
   memset(&ops, 0, sizeof(ops));
-  const int nf_pad = m.fl.nf_pad;
+  ops.dvp_hi = dvp_hi;
+  ops.dvp_lo = dvp_lo;
+  // every CTA of a pair loads nf_pad/2 rows of the Wb slab.  K extent = row_end: model columns beyond it are never
+  // read (TMA zero-fills out-of-bounds)
   int rc;
-  const bool split3 = (mode != B200SMPL_MODE_BF16) && dvp_lo != nullptr;
-  const int nseg = split3 ? 3 : 1;
-  // K extent = row_end: model columns beyond it are never read (TMA zero-fills out-of-bounds)
-  ops.a[0] = dvp_hi;
-  if ((rc = make_map(&ops.b[0], m.Wb_hi, row_end, nf_pad, m.n_pad, nf_pad))) return rc;
-  if (split3) {
-    ops.a[1] = dvp_lo;
-    if ((rc = make_map(&ops.b[1], m.Wb_hi, row_end, nf_pad, m.n_pad, nf_pad))) return rc;
-    ops.a[2] = dvp_hi;
-    if ((rc = make_map(&ops.b[2], m.Wb_lo, row_end, nf_pad, m.n_pad, nf_pad))) return rc;
-  }
+  if ((rc = make_map(&ops.wb_hi, m.Wb_hi, row_end, nf_pad, m.n_pad, nf_pad / 2))) return rc;
+  if (split3 && (rc = make_map(&ops.wb_lo, m.Wb_lo, row_end, nf_pad, m.n_pad, nf_pad / 2))) return rc;
   const int slab_begin = row_begin / BK, slab_end = (row_end + BK - 1) / BK;
   const long long split_stride = (long long)S * nf_pad;
-  // CTA pairs where the body tiles pair up; the single-CTA kernel takes an odd number of tiles and nf_pad = 208
-  // (1 beta).  nf_pad <= round_up(MAX_BETAS + NPOSE, 16) = 224.
-  if (nf_pad == 224 && (Sw / BM) % 2 == 0)
-    return launch_bwd_bn_2cta<224>(ops, m, nseg, row_end, slab_begin, slab_end, nsplit, Sw, dfeat_part, nf_pad, split_stride, st);
-  switch (nf_pad) {
-    case 224: return launch_bwd_bn<224>(ops, nseg, m.n_pad / 8, slab_begin, slab_end, nsplit, Sw, dfeat_part, nf_pad, split_stride, st);
-    case 208: return launch_bwd_bn<208>(ops, nseg, m.n_pad / 8, slab_begin, slab_end, nsplit, Sw, dfeat_part, nf_pad, split_stride, st);
-    default: return fail(B200SMPL_ERR_INVALID, "unsupported num_betas for the tensor-core backward (nf_pad=" + std::to_string(nf_pad) + ")");
-  }
+  auto launch = nf_pad == 224 ? launch_bwd_pair<224> : launch_bwd_pair<208>;
+  return launch(ops, split3 ? 1 : 0, Sw / BM, m.n_pad / 8, slab_begin, slab_end, nsplit, dfeat_part, split_stride, st);
 }
 
 }  // namespace b200smpl

@@ -241,7 +241,7 @@ int launch_blend_fwd_umma(const DevModel& m, int mode, const __nv_bfloat16* feat
 int launch_blend_bwd_umma(const DevModel& m, int mode, const __nv_bfloat16* dvp_hi, const __nv_bfloat16* dvp_lo,
                           int S, int Sw, float* dfeat_part, int nsplit, int row_begin, int row_end,
                           cudaStream_t st);
-int blend_bwd_umma_splits(const DevModel& m, int mode, int S, int num_sms);
+int blend_bwd_umma_splits(const DevModel& m, int S, int num_sms);
 // blend GEMM with the skinning in its epilogue (fused_fwd.cu); forward-only calls
 int launch_blend_lbs_fwd(const DevModel& m, int mode, const __nv_bfloat16* feat, int S, int Sw, float* vpT,
                          const float* A_blk, int b0, int nb, const float* transl, float* verts, int num_sms,

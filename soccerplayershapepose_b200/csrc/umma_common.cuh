@@ -12,13 +12,14 @@ constexpr int BM = 128;
 constexpr int BK = 64;                 // bf16 elements = 128 bytes = one swizzle row
 constexpr int UMMA_K = 16;
 constexpr int GEMM_THREADS = 192;
-constexpr int MAX_SEG = 3;
 
 // backward operands: A = dvp chunks [S/128][n/8][128][8] (plain pointers, one 16 KB bulk copy per stage
-// straight into the no-swizzle core-matrix layout), B = Wb rows through a 128-byte-swizzle tensor map
+// straight into the no-swizzle core-matrix layout), B = Wb rows through a 128-byte-swizzle tensor map.
+// The lo halves are read only by the bf16x3 split (fp32 modes).
 struct GemmOps {
-  const __nv_bfloat16* a[MAX_SEG];
-  CUtensorMap b[MAX_SEG];
+  const __nv_bfloat16* dvp_hi;
+  const __nv_bfloat16* dvp_lo;
+  CUtensorMap wb_hi, wb_lo;
 };
 
 // ---- PTX wrappers ---------------------------------------------------------------------------
@@ -86,28 +87,6 @@ __device__ __forceinline__ void prefetch_tmap(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
 }
 
-__device__ __forceinline__ void tmem_alloc(uint32_t* smem_dst, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)), "r"(ncols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-// D[tmem] (+)= A[smem] . B[smem]^T, bf16 x bf16 -> fp32
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                          uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 // 32 lanes x 32 columns of fp32 accumulators -> 32 registers per thread (thread = TMEM lane)
 __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t (&v)[32]) {
   asm volatile(
@@ -144,6 +123,7 @@ __host__ __device__ constexpr uint32_t make_idesc(int M, int N) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
+// D[tmem] (+)= A[smem] . B[smem]^T, bf16 x bf16 -> fp32, issued by the leader CTA for the pair
 __device__ __forceinline__ void umma_bf16_2cta(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
                                                uint32_t accumulate) {
   asm volatile(

@@ -266,11 +266,11 @@ def test_full_size_properties(engine, dev, mode):
         assert _rel(b, 2 * a) < 1e-5
 
 
-@pytest.mark.parametrize("nb,B", [(1, 37), (4, 130), (16, 256)])
+@pytest.mark.parametrize("nb,B", [(1, 37), (1, 256), (4, 130), (16, 256), (16, 300)])
 def test_other_beta_counts_and_tile_counts(synthetic_model, dev, nb, B):
-    """Models with another number of betas (other K layouts / gradient widths: nf_pad 208 takes the single-CTA
-    gradient GEMM, 224 the CTA-pair one) at batch sizes with an odd (37 -> 1), even (130 -> 2, 256 -> 2) number
-    of 128-body tiles: forward and backward against the oracle."""
+    """Models with another number of betas (other K layouts / gradient widths: the CTA-pair gradient GEMM with
+    nf_pad 208 for 1 beta, 224 otherwise) at batch sizes with an odd (37 -> 1, 300 -> 3: the last cluster has a
+    padding CTA), or even (130 -> 2, 256 -> 2) number of 128-body tiles: forward and backward against the oracle."""
     model = dict(synthetic_model)
     sd = synthetic_model["shapedirs"]
     if nb <= sd.shape[2]:
