@@ -329,6 +329,10 @@ B200SMPL_API int b200smpl_multitask_loss_backward(const b200smpl_multitask_loss_
  * silhouette_loss: loss_per_body[b] += weight * mean over the S^2 pixels of (alpha - target)^2 (target [B][S][S]
  * uint8, non-zero = inside), with the gradient of that term written to grad_vertices / grad_t; it never writes the
  * image.  The call adds into loss_per_body so that it can follow b200smpl_fit_loss on the same buffer.
+ * silhouette_loss_value: the same loss_per_body[b] += weight * mean (alpha - target)^2 without the gradient (for
+ * validation and no-grad passes): no backward pass, no per-vertex accumulator (the shared memory of the render,
+ * 138 KB for SMPL) and no image.  sigma >= 0: sigma == 0 scores the hard silhouette.  The per-body sum is
+ * deterministic (no global atomics); small batches split a body's bands over a thread-block cluster.
  * No workspace is needed at present (workspace_bytes returns 0; the fields may be NULL / 0).
  */
 typedef struct b200smpl_silhouette_args {
@@ -346,6 +350,10 @@ B200SMPL_API int b200smpl_silhouette_render_backward(const b200smpl_silhouette_a
                                                      float* grad_vertices, float* grad_t, void* stream);
 B200SMPL_API int b200smpl_silhouette_loss(const b200smpl_silhouette_args* args, const uint8_t* target, float weight,
                                           float* loss_per_body, float* grad_vertices, float* grad_t, void* stream);
+/* loss_per_body[b] += weight * mean over the S^2 pixels of (alpha - target)^2; no gradient, no image.
+ * sigma >= 0: sigma == 0 scores the hard silhouette. */
+B200SMPL_API int b200smpl_silhouette_loss_value(const b200smpl_silhouette_args* args, const uint8_t* target,
+                                                float weight, float* loss_per_body, void* stream);
 
 /* Test hook (host arithmetic only, no device): the cluster work list of the forward blend GEMM for `body_tiles`
  * 128-body tiles x `row_tiles` 128-row tiles on a device with `num_sms` SMs.  Writes (body-tile pair, first row-tile

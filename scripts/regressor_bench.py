@@ -5,12 +5,16 @@ per GPU, data-parallel over NCCL when launched under torchrun.  One CUDA graph p
 
   python scripts/regressor_bench.py [--steps 50] [--batch 256] [--input encoder|features] [--res 256]
                                     [--loss fused|eager] [--no-overlap] [--eager]
+                                    [--silhouette-weight W [--sil-res S] [--sil-sigma SIGMA]]
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 scripts/regressor_bench.py ...
 
 --input encoder (default): the reference's SingleInputRegressor (models/regressor.py: ResNet-18 over 18 x res x res
 proxy inputs + IEFModule([512,512])), 11.9 M parameters = 47.6 MB all-reduced per step.  BASELINE.json says 224x224
 crops; the reference's regressor input is 18x256x256 (config.REGRESSOR_IMG_WH, PyTorch3DTest.py:241): --res picks.
 --input features: synthetic 512-d features into IEFModule([1024,1024]) (the round-1 head-only configuration).
+--silhouette-weight W > 0 adds the silhouette term (initial weight W; PyTorch3DTest.py:1084-1087) at S x S pixels:
+the targets are the hard silhouettes of the label bodies; the fused loss runs ops.silhouette_term, the eager loss
+renders the soft silhouettes first.
 Prints one JSON line (rank 0)."""
 import argparse, json, os, sys
 import torch
@@ -32,6 +36,9 @@ ap.add_argument("--no-overlap", action="store_true", help="one all-reduce after 
 ap.add_argument("--eager", action="store_true", help="no CUDA graph: eager step (DistributedDataParallel when N > 1)")
 ap.add_argument("--amp", action="store_true", help="run the (library, cuDNN) encoder under bf16 autocast; the head, the SMPL "
                                                    "layer and the loss stay fp32")
+ap.add_argument("--silhouette-weight", type=float, default=0.0, help="> 0: add the silhouette term at this weight")
+ap.add_argument("--sil-res", type=int, default=config.REGRESSOR_IMG_WH, help="silhouette resolution S")
+ap.add_argument("--sil-sigma", type=float, default=1.0, help="soft silhouette blur (px^2)")
 args = ap.parse_args()
 steps, B = args.steps, args.batch
 rank, world, local = (int(os.environ.get(k, d)) for k, d in (("RANK", 0), ("WORLD_SIZE", 1), ("LOCAL_RANK", 0)))
@@ -55,10 +62,15 @@ if args.input == "encoder":
 else:
     head = regressor.IEFModule((1024, 1024), in_features=512).to(dev)
     feats = torch.randn(B, 512, device=dev)
-crit = regressor.MultiTaskLoss(("verts", "joints2D", "joints3D", "shape_params", "pose_params"),
-                               {"verts": 1.0, "joints2D": 0.1, "joints3D": 1.0, "shape_params": 0.1, "pose_params": 0.1}).to(dev)
+sil = args.silhouette_weight > 0
+crit = regressor.MultiTaskLoss(("verts", "joints2D", "joints3D", "shape_params", "pose_params") + (("silhouette",) if sil else ()),
+                               {"verts": 1.0, "joints2D": 0.1, "joints3D": 1.0, "shape_params": 0.1, "pose_params": 0.1,
+                                "silhouette": args.silhouette_weight},
+                               faces=smpl.faces_int32(dev) if sil else None, silhouette_sigma=args.sil_sigma,
+                               silhouette_wh=args.sil_res).to(dev)
 fused = args.loss == "fused"
 r6, proj = regressor.gpu_ops()
+render = regressor.gpu_silhouette_renderer(smpl.faces_int32(dev), args.sil_res, args.sil_sigma) if sil else None
 
 
 class Step(torch.nn.Module):
@@ -67,7 +79,8 @@ class Step(torch.nn.Module):
         self.head, self.crit = head, crit
 
     def forward(self, f, labels):
-        out = regressor.predict(self.head, smpl, f, r6, None if fused else proj)
+        out = regressor.predict(self.head, smpl, f, r6, None if fused else proj,
+                                render_silhouettes=None if fused else render)
         return (self.crit.forward_fused(labels, out) if fused else self.crit(labels, out))[0]
 
 
@@ -79,6 +92,8 @@ with torch.no_grad():
     labels = {"verts": t.vertices, "joints3D": t.joints[:, config.ALL_JOINTS_TO_COCO_MAP, :].contiguous(), "shape_params": betas,
               "pose_params_rot_matrices": rot,
               "joints2D": ops.orthographic_project(t.joints, cam, 512.0)[:, config.SMPL_TO_KPRCNN_MAP, :].contiguous()}
+    if sil:
+        labels["silhouette"] = smpl.render_silhouettes(t.vertices, cam, img_wh=args.sil_res, sigma=0.0) > 0.5
 
 if args.eager:
     model = Step()
@@ -94,7 +109,7 @@ if args.eager:
         return loss
 else:
     gstep = regressor.GraphedTrainStep(head, crit, smpl, feats, labels, r6, proj, lr=1e-4, world_size=world,
-                                       fused_loss=fused, overlap=not args.no_overlap)
+                                       fused_loss=fused, overlap=not args.no_overlap, render_silhouettes=render)
 
     def step():
         return gstep(feats, labels)
@@ -116,8 +131,10 @@ if rank == 0:
     what = ("18x%dx%d crops -> ResNet-18%s -> IEF head (512,512)" % (args.res, args.res, " (bf16 autocast)" if args.amp else " (fp32/TF32 cuDNN)")
             if args.input == "encoder"
             else "512-d features -> IEF head (1024,1024)")
-    print(json.dumps({"workload": "BASELINE.json configs[4]: regressor step: %s -> SMPL -> 5-term multi-task loss (%s kernels), "
-                                  "batch %d per GPU x %d GPU(s), %s" % (what, args.loss, B, world,
+    terms = "5-term" if not sil else "6-term (+ silhouette at %dx%d, sigma %g, weight %g)" % (
+        args.sil_res, args.sil_res, args.sil_sigma, args.silhouette_weight)
+    print(json.dumps({"workload": "BASELINE.json configs[4]: regressor step: %s -> SMPL -> %s multi-task loss (%s kernels), "
+                                  "batch %d per GPU x %d GPU(s), %s" % (what, terms, args.loss, B, world,
                                                                        "eager" if args.eager else "one CUDA graph per step"),
                       "ms_per_step": ms / steps, "crops_per_s": B * world * steps / (ms / 1e3),
                       "allreduced_params": nparams if world > 1 else 0, "allreduced_mb": nparams * 4 / 1e6 if world > 1 else 0,

@@ -8,6 +8,11 @@ the kernels' bins (32 x 8 tiles met by each face's grown box, 256 pixels each). 
 read in the same run.  Bodies: 64 distinct posed synthetic bodies, repeated down the batch.
 
     python scripts/silhouette_bench.py [--tag b200] [--quick]
+    python scripts/silhouette_bench.py --value [--tag b200] [--quick]
+
+--value times only the gradient-free loss (b200smpl_silhouette_loss_value) against the fused loss with its
+backward and the soft render, hard and soft, at B in {64, 256, 1024}, S in {128, 256}; it writes
+profiles/r04_silhouette_value_<tag>.json.
 """
 import argparse
 import json
@@ -83,10 +88,13 @@ def main():
     ap.add_argument("--tag", default="b200")
     ap.add_argument("--quick", action="store_true", help="small sizes only (rehearsal)")
     ap.add_argument("--out", default=None, help="output path (default profiles/r03_silhouette_<tag>.json)")
+    ap.add_argument("--value", action="store_true", help="only the gradient-free loss against the fused loss and render")
     a = ap.parse_args()
     assert torch.cuda.is_available(), "silhouette_bench needs a CUDA device"
     smpl = SMPL(model_data=make_synthetic_smpl(1234)).to(DEV)
     faces = smpl.faces_int32(DEV)
+    if a.value:
+        return value_leg(a, smpl, faces)
     res = {"card": card(), "render": [], "eager": [], "fitter": []}
     Bs, Ss = ([8], [64]) if a.quick else ([64, 1024], [256, 512])
     for B in Bs:
@@ -153,6 +161,30 @@ def main():
             res["fitter"].append(row)
             print(json.dumps(row), flush=True)
     out = a.out or os.path.join(ROOT, "profiles", "r03_silhouette_{}.json".format(a.tag))
+    with open(out, "w") as fh:
+        json.dump(res, fh, indent=1)
+    print("wrote", out)
+
+
+def value_leg(a, smpl, faces):
+    res = {"card": card(), "value": []}
+    Bs, Ss = ([8, 64], [64]) if a.quick else ([64, 256, 1024], [128, 256])
+    for B in Bs:
+        v, t = bodies(smpl, B)
+        for S in Ss:
+            f = config.FOCAL_LENGTH * S / 512
+            target = ops.render_silhouettes(v * 1.02, faces, t, S, f, 0.0) > 0.5
+            lpb = torch.zeros(B, device=DEV)
+            for sigma in (0.0, 1.0):
+                row = {"B": B, "S": S, "sigma": sigma,
+                       "value_ms": timed(lambda: ops.silhouette_loss_value(v, faces, t, target, S, f, sigma, 1.0, lpb)),
+                       "render_ms": timed(lambda: ops.render_silhouettes(v, faces, t, S, f, sigma))}
+                if sigma > 0:
+                    row["fused_loss_ms"] = timed(lambda: ops.silhouette_loss(v, faces, t, target, S, f, sigma, 1.0, lpb))
+                    row["value_vs_fused"] = row["value_ms"] / row["fused_loss_ms"]
+                res["value"].append(row)
+                print(json.dumps(row), flush=True)
+    out = a.out or os.path.join(ROOT, "profiles", "r04_silhouette_value_{}.json".format(a.tag))
     with open(out, "w") as fh:
         json.dump(res, fh, indent=1)
     print("wrote", out)

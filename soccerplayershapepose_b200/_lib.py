@@ -132,6 +132,7 @@ SYMBOLS = {
     "b200smpl_silhouette_render_backward": (c_int, [POINTER(SilhouetteArgs), c_void_p, c_void_p, c_void_p, c_void_p]),
     "b200smpl_silhouette_loss": (c_int, [POINTER(SilhouetteArgs), c_void_p, c_float, c_void_p, c_void_p, c_void_p,
                                          c_void_p]),
+    "b200smpl_silhouette_loss_value": (c_int, [POINTER(SilhouetteArgs), c_void_p, c_float, c_void_p, c_void_p]),
     "b200smpl_debug_fwd_gemm_worklist":(c_int, [c_int, c_int, c_int, c_void_p, c_int]),
     "b200smpl_last_error": (c_char_p, []),
     "b200smpl_abi_version": (c_int, []),

@@ -20,9 +20,16 @@
 // so that prod_{g != f} (1 - D_g) is exact without dividing by a vanishing factor.  d alpha / d(u, v) is reduced
 // over the warp and accumulated per vertex in shared memory; the flush applies the chain rule through the
 // projection, writes grad_vertices without global atomics and reduces grad_t over the block.
+// The gradient-free loss runs the forward's per-pixel pass and sums (alpha - target)^2 instead of writing alpha; when
+// it splits a body's bands, the CTAs form a cluster whose partial sums are added in rank order.
+#include <cooperative_groups.h>
+
+#include <algorithm>
 #include <cmath>
 
 #include "common.cuh"
+
+namespace cg = cooperative_groups;
 
 namespace b200smpl {
 namespace {
@@ -37,6 +44,7 @@ constexpr float SIL_ZMIN = 1e-3f;   // a face with a vertex at z + tz <= ZMIN is
 constexpr float SIL_AREA_MIN = 1e-8f;
 constexpr float SIL_SAT = 1e-30f;   // 1 - D_f below this counts as saturated (exactly 0 in the products)
 constexpr float SIL_SLACK = 1e-2f;  // px added to every culling box (the per-pixel tests are exact)
+constexpr int SIL_MAX_CLUSTER = 8;  // CTAs per body of sil_loss_value (the portable cluster size)
 
 struct SilArgs {
   int V, F, S;
@@ -161,8 +169,11 @@ __device__ int band_list(const SilArgs& a, const float2* P, uint16_t* L, int* wc
 }
 
 // ---- forward -----------------------------------------------------------------------------------------------------
-__device__ void tile_fwd(const SilArgs& a, const float2* P, const uint16_t* L, int n, int row0, int col0,
-                         float* __restrict__ alpha) {
+// VALUE = false: writes the tile's alpha.  VALUE = true: writes nothing and returns the lane's share of
+// sum (alpha - target)^2 (the same per-pixel alpha and the same summation order as pass 1 of the fused loss).
+template <bool VALUE>
+__device__ float tile_fwd(const SilArgs& a, const float2* P, const uint16_t* L, int n, int row0, int col0,
+                          float* __restrict__ alpha, const uint8_t* __restrict__ target) {
   const int lane = threadIdx.x & 31;
   const float px = col0 + lane + 0.5f;
   const float x0 = col0 + 0.5f, x1 = col0 + SIL_TW - 0.5f, y0 = row0 + 0.5f, y1 = row0 + SIL_TH - 0.5f;
@@ -195,13 +206,22 @@ __device__ void tile_fwd(const SilArgs& a, const float2* P, const uint16_t* L, i
       }
     }
   }
+  float lsum = 0.f;
   const int col = col0 + lane;
-  if (col >= a.S) return;
+  if (col >= a.S) return lsum;
 #pragma unroll
   for (int r = 0; r < SIL_TH; ++r) {
     const int row = row0 + r;
-    if (row < a.S) alpha[(size_t)row * a.S + col] = nsat[r] ? 1.f : 1.f - prod[r];
+    if (row >= a.S) continue;
+    const float al = nsat[r] ? 1.f : 1.f - prod[r];
+    if (VALUE) {
+      const float d = al - (target[(size_t)row * a.S + col] ? 1.f : 0.f);
+      lsum += d * d;
+    } else {
+      alpha[(size_t)row * a.S + col] = al;
+    }
   }
+  return lsum;
 }
 
 __global__ void __launch_bounds__(SIL_THREADS, 1) sil_fwd(SilArgs a, float* __restrict__ alpha) {
@@ -221,7 +241,7 @@ __global__ void __launch_bounds__(SIL_THREADS, 1) sil_fwd(SilArgs a, float* __re
     const int n = band_list(a, P, L, wcnt, r0 + 0.5f, r0 + rows - 0.5f, a.rad + SIL_SLACK);
     const int ntr = (rows + SIL_TH - 1) / SIL_TH;
     for (int tile = warp; tile < ntr * ntc; tile += SIL_WARPS)
-      tile_fwd(a, P, L, n, r0 + (tile / ntc) * SIL_TH, (tile % ntc) * SIL_TW, out);
+      tile_fwd<false>(a, P, L, n, r0 + (tile / ntc) * SIL_TH, (tile % ntc) * SIL_TW, out, nullptr);
     __syncthreads();                                      // the next band rewrites L
   }
 }
@@ -410,6 +430,55 @@ __global__ void __launch_bounds__(SIL_THREADS, 1) sil_loss(SilArgs a, const uint
   sil_bwd_body<true>(a, nullptr, target, weight, loss, grad_verts, grad_t);
 }
 
+// ---- gradient-free loss ------------------------------------------------------------------------------------------
+// loss[b] += weight * mean (alpha - target)^2 without the backward's pass 2 or its accumulator G, so the shared
+// memory is that of sil_fwd.  Grid (B, split), cluster (1, split, 1): the CTAs of one cluster share a body's bands
+// as sil_fwd's do, and rank 0 adds their partial sums in rank order through distributed shared memory, so the
+// result is deterministic for a given split and needs neither global atomics nor a workspace.
+__global__ void __launch_bounds__(SIL_THREADS, 1) sil_loss_value(SilArgs a, const uint8_t* __restrict__ target,
+                                                                 float weight, float* __restrict__ loss) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  __shared__ int wcnt[SIL_WARPS];
+  __shared__ float red[SIL_WARPS];
+  __shared__ float part;
+  cg::cluster_group cluster = cg::this_cluster();
+  float2* P = reinterpret_cast<float2*>(smem);
+  uint16_t* L = reinterpret_cast<uint16_t*>(smem + (size_t)a.V * sizeof(float2));
+  const int b = blockIdx.x;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  project_body(a, b, P);
+  __syncthreads();
+  const size_t img = (size_t)a.S * a.S;
+  const uint8_t* tg = target + b * img;
+  const int nbands = (a.S + SIL_BAND - 1) / SIL_BAND, ntc = (a.S + SIL_TW - 1) / SIL_TW;
+  float lsum = 0.f;
+  for (int band = blockIdx.y; band < nbands; band += gridDim.y) {
+    const int r0 = band * SIL_BAND;
+    const int rows = min(SIL_BAND, a.S - r0);
+    const int n = band_list(a, P, L, wcnt, r0 + 0.5f, r0 + rows - 0.5f, a.rad + SIL_SLACK);
+    const int ntr = (rows + SIL_TH - 1) / SIL_TH;
+    for (int tile = warp; tile < ntr * ntc; tile += SIL_WARPS)
+      lsum += tile_fwd<true>(a, P, L, n, r0 + (tile / ntc) * SIL_TH, (tile % ntc) * SIL_TW, nullptr, tg);
+    __syncthreads();                                      // the next band rewrites L
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) lsum += __shfl_xor_sync(0xffffffffu, lsum, o);
+  if (lane == 0) red[warp] = lsum;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float s = 0.f;
+    for (int w = 0; w < SIL_WARPS; ++w) s += red[w];
+    part = s;
+  }
+  cluster.sync();
+  if (cluster.block_rank() == 0 && threadIdx.x == 0) {
+    float s = 0.f;
+    for (unsigned r = 0; r < cluster.num_blocks(); ++r) s += *cluster.map_shared_rank(&part, r);
+    loss[b] += weight * s / (float)img;
+  }
+  cluster.sync();                                         // every partial stays readable until rank 0 has read it
+}
+
 size_t sil_smem(const b200smpl_silhouette_args* p, bool bwd) {
   return (size_t)p->num_verts * sizeof(float2) * (bwd ? 2 : 1) + (size_t)p->num_faces * 3 * sizeof(uint16_t);
 }
@@ -509,6 +578,40 @@ int b200smpl_silhouette_loss(const b200smpl_silhouette_args* args, const uint8_t
   sil_loss<<<args->batch, SIL_THREADS, smem, (cudaStream_t)stream>>>(a, target, weight, loss_per_body, grad_vertices,
                                                                      grad_t);
   B200_LAUNCH_CHECK("sil_loss");
+  return 0;
+}
+
+int b200smpl_silhouette_loss_value(const b200smpl_silhouette_args* args, const uint8_t* target, float weight,
+                                   float* loss_per_body, void* stream) {
+  B200_NVTX("b200smpl_silhouette_loss_value");
+  SilArgs a;
+  size_t smem = 0;
+  if (int rc = sil_prepare(args, false, a, smem)) return rc;
+  if (!target || !loss_per_body || !std::isfinite(weight))
+    return fail(B200SMPL_ERR_INVALID, "silhouette_loss_value: NULL pointer or non-finite weight");
+  int dev = 0, sms = 0;
+  B200_CUDA_TRY(cudaGetDevice(&dev));
+  B200_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  // small batches: a cluster of CTAs per body, as many as fill the SMs (sil_fwd's split, capped at a portable cluster)
+  const int nbands = (a.S + SIL_BAND - 1) / SIL_BAND;
+  const int split = std::max(1, std::min({SIL_MAX_CLUSTER, nbands, (sms + args->batch - 1) / args->batch}));
+  B200_SMEM_ATTR_ONCE(sil_loss_value, smem);
+  cudaLaunchConfig_t cfg;
+  memset(&cfg, 0, sizeof(cfg));
+  cfg.gridDim = dim3(args->batch, split, 1);
+  cfg.blockDim = dim3(SIL_THREADS, 1, 1);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = (cudaStream_t)stream;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 1;
+  attr[0].val.clusterDim.y = split;
+  attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  LaunchTimer _timer("sil_loss_value", (cudaStream_t)stream);
+  B200_CUDA_TRY(cudaLaunchKernelEx(&cfg, sil_loss_value, a, target, weight, loss_per_body));
+  B200_LAUNCH_CHECK("sil_loss_value");
   return 0;
 }
 

@@ -338,7 +338,7 @@ def multitask_loss(log_var: torch.Tensor, *, verts=None, verts_label=None, joint
                    label2d=None, vis=None, map3d=None, label3d=None, shape=None, shape_label=None, pose=None,
                    pose_label=None, proj_wh: float = 512.0, norm_wh: float = 256.0):
     """Fused HomoscedasticUncertaintyWeightedMultiTaskLoss (losses/multi_task_loss.py:92-130 without the silhouette
-    term): `log_var` (5,) = log-variances of (verts, joints2D, joints3D, shape_params, pose_params); a term is
+    term, which regressor.MultiTaskLoss adds with `silhouette_term`): `log_var` (5,) = log-variances of (verts, joints2D, joints3D, shape_params, pose_params); a term is
     evaluated when its prediction (its joint map for the joint terms) is given.  Returns (loss, parts (5,))."""
     return _MultiTaskLoss.apply(log_var, verts, joints, cam, shape, pose, verts_label, map2d, label2d, vis, map3d,
                                 label3d, shape_label, pose_label, proj_wh, norm_wh)
@@ -457,6 +457,76 @@ def silhouette_loss(vertices: torch.Tensor, faces, cam_t: torch.Tensor, target: 
                                                         loss_per_body.data_ptr(), gv.data_ptr(), gt.data_ptr(),
                                                         _stream(vertices)), "silhouette_loss")
     return loss_per_body, gv, gt
+
+
+def _binary_target(target: torch.Tensor, B: int, S: int, device: torch.device) -> torch.Tensor:
+    """(B,S,S) mask as contiguous uint8 on `device`: floating point `>= 0.5`, other dtypes non-zero (as
+    `silhouette_iou` reads masks).  Plain tensor ops, so a CUDA graph can capture it."""
+    if tuple(target.shape) != (B, S, S):
+        raise ValueError("target has shape {}, expected {}".format(tuple(target.shape), (B, S, S)))
+    mask = target >= 0.5 if target.dtype.is_floating_point else target != 0
+    return mask.to(device=device, dtype=torch.uint8).contiguous()
+
+
+def silhouette_loss_value(vertices: torch.Tensor, faces, cam_t: torch.Tensor, target: torch.Tensor, img_wh: int,
+                          focal_length: float = config.FOCAL_LENGTH, sigma: float = 1.0, weight: float = 1.0,
+                          loss_per_body: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """loss_per_body[b] += weight * mean over the S^2 pixels of (alpha_b - target_b)^2 without the gradient: one
+    kernel that neither writes the image nor runs the backward (validation and no-grad passes).  sigma == 0 scores
+    the hard silhouette.  Returns loss_per_body (B,), a plain tensor."""
+    vertices, cam_t = _req(vertices, "vertices"), _req(cam_t, "cam_t")
+    B, S = vertices.shape[0], int(img_wh)
+    faces32 = _faces_int32(faces, vertices.device, vertices.shape[1])
+    args = silhouette_args(vertices, faces32, cam_t, S, focal_length, sigma)
+    tgt = _binary_target(target, B, S, vertices.device)
+    if loss_per_body is None:
+        loss_per_body = torch.zeros(B, dtype=torch.float32, device=vertices.device)
+    elif (tuple(loss_per_body.shape) != (B,) or loss_per_body.dtype != torch.float32
+          or loss_per_body.device != vertices.device or not loss_per_body.is_contiguous()):
+        raise ValueError("loss_per_body must be a contiguous float32 ({},) tensor on the device of vertices".format(B))
+    with torch.cuda.device(vertices.device):
+        _lib.check(_lib.load().b200smpl_silhouette_loss_value(ctypes.byref(args), tgt.data_ptr(), float(weight),
+                                                              loss_per_body.data_ptr(), _stream(vertices)),
+                   "silhouette_loss_value")
+    return loss_per_body
+
+
+class _SilhouetteTerm(torch.autograd.Function):
+    """Batch mean of the per-body silhouette loss through the fused loss kernel: its forward keeps the gradients of
+    the term, its backward scales them by the upstream gradient on the device (no host read: graph-capturable)."""
+
+    @staticmethod
+    def forward(ctx, vertices, cam_t, faces32, tgt, img_wh, focal_length, sigma):
+        args = silhouette_args(vertices, faces32, cam_t, img_wh, focal_length, sigma)
+        B = vertices.shape[0]
+        loss = torch.zeros(B, dtype=torch.float32, device=vertices.device)
+        gv, gt = torch.empty_like(vertices), torch.empty_like(cam_t)
+        with torch.cuda.device(vertices.device):
+            _lib.check(_lib.load().b200smpl_silhouette_loss(ctypes.byref(args), tgt.data_ptr(), 1.0 / B,
+                                                            loss.data_ptr(), gv.data_ptr(), gt.data_ptr(),
+                                                            _stream(vertices)), "silhouette_loss")
+        ctx.save_for_backward(gv, gt)
+        return loss.sum()
+
+    @staticmethod
+    def backward(ctx, g):
+        gv, gt = ctx.saved_tensors
+        return gv * g, gt * g, None, None, None, None, None
+
+
+def silhouette_term(vertices: torch.Tensor, faces, cam_t: torch.Tensor, target: torch.Tensor, img_wh: int,
+                    focal_length: float = config.FOCAL_LENGTH, sigma: float = 1.0) -> torch.Tensor:
+    """Scalar silhouette term: the batch mean of the per-body mean over the S^2 pixels of (alpha - target)^2,
+    differentiable w.r.t. `vertices` and `cam_t` (sigma > 0).  When a gradient is needed the fused loss kernel runs
+    and keeps it; otherwise (no_grad, or no input requires a gradient) only the gradient-free value kernel runs.
+    target (B,S,S): floating point `>= 0.5` or non-zero is inside."""
+    vertices, cam_t = _req(vertices, "vertices"), _req(cam_t, "cam_t")
+    B, S = vertices.shape[0], int(img_wh)
+    faces32 = _faces_int32(faces, vertices.device, vertices.shape[1])
+    tgt = _binary_target(target, B, S, vertices.device)
+    if torch.is_grad_enabled() and (vertices.requires_grad or cam_t.requires_grad):
+        return _SilhouetteTerm.apply(vertices, cam_t, faces32, tgt, S, float(focal_length), float(sigma))
+    return silhouette_loss_value(vertices, faces32, cam_t, tgt, S, focal_length, sigma, 1.0 / B).sum()
 
 
 def silhouette_iou(pred: torch.Tensor, target: torch.Tensor) -> torch.Tensor:

@@ -6,7 +6,8 @@ Mirrors the reference's training step (PlayerReconstruction/PyTorch3DTest.py:104
              -> rot6d_to_rotmat (utils/rigid_transform_utils.py:27-41)           [C-ABI kernel]
              -> SMPL(body_pose, global_orient, betas, pose2rot=False)            [C-ABI kernels]
              -> orthographic projection of the joints, COCO map, pixels          [fused C-ABI kernel]
-             -> HomoscedasticUncertaintyWeightedMultiTaskLoss (losses/multi_task_loss.py:92-130)
+             -> (silhouette term: the predicted bodies' soft silhouettes, PyTorch3DTest.py:1084-1087)
+             -> HomoscedasticUncertaintyWeightedMultiTaskLoss (losses/multi_task_loss.py:92-144)
              -> backward -> (data-parallel: NCCL all-reduce of the head's gradients) -> Adam
 
 The CNN encoder in front is the caller's (BASELINE.json: "CNN features -> SMPL head"); the head's three linear
@@ -68,12 +69,23 @@ class IEFModule(nn.Module):
 
 
 class MultiTaskLoss(nn.Module):
-    """HomoscedasticUncertaintyWeightedMultiTaskLoss (losses/multi_task_loss.py:16-152) without the silhouette
-    term: MSE(mean) per task * exp(-log_var) + log_var, log_var0 = -log(w + 1e-6), log-variances trainable."""
+    """HomoscedasticUncertaintyWeightedMultiTaskLoss (losses/multi_task_loss.py:16-152): MSE(mean) per task *
+    exp(-log_var) + log_var, log_var0 = -log(w + 1e-6), log-variances trainable.
 
-    TASKS = ("verts", "joints2D", "joints3D", "shape_params", "pose_params")
+    "silhouette" (losses/multi_task_loss.py:132-144): L = batch mean of the per-body mean over the S^2 pixels of
+    (alpha - target)^2, alpha the soft silhouette of the predicted body and target = labels["silhouette"] (B,S,S)
+    (floating point >= 0.5 or non-zero is inside).  The form of the reference's silhouette loss could not be read;
+    this squared error is the fitter's stated definition (DESIGN.md section 11).  The camera is
+    `SMPL.render_silhouettes`': t = [tx, ty, 2 f / (proj_wh s + 1e-9)] from the head's weak-perspective cam, f =
+    config.FOCAL_LENGTH, rendered at S = `silhouette_wh` with focal length f S / proj_wh and blur `silhouette_sigma`.
+    `faces` (F,3) are required with the term and kept as a non-persistent buffer (state_dicts gain only
+    `silhouette_log_var`)."""
 
-    def __init__(self, losses_on: Sequence[str], init_loss_weights: Optional[Dict[str, float]] = None, eps: float = 1e-6):
+    TASKS = ("verts", "joints2D", "joints3D", "shape_params", "pose_params", "silhouette")
+
+    def __init__(self, losses_on: Sequence[str], init_loss_weights: Optional[Dict[str, float]] = None, eps: float = 1e-6,
+                 faces=None, silhouette_sigma: float = 1.0, silhouette_wh: int = config.REGRESSOR_IMG_WH,
+                 proj_wh: float = 512.0):
         super().__init__()
         self.losses_on = tuple(losses_on)
         for t in self.losses_on:
@@ -82,6 +94,29 @@ class MultiTaskLoss(nn.Module):
             w = None if init_loss_weights is None else init_loss_weights.get(t)
             lv = 0.0 if w is None else float(-np.log(w + eps))
             setattr(self, t + "_log_var", nn.Parameter(torch.tensor(lv).float()))
+        if "silhouette" in self.losses_on:
+            if faces is None:
+                raise ValueError("the silhouette term needs the mesh faces (faces=...)")
+            faces = torch.as_tensor(faces)
+            if faces.dim() != 2 or faces.shape[1] != 3 or faces.dtype.is_floating_point:
+                raise ValueError("faces must be an integer (F, 3) array")
+            self.register_buffer("silhouette_faces", faces.to(torch.int32).contiguous(), persistent=False)
+            self.silhouette_sigma = float(silhouette_sigma)
+            self.silhouette_wh = int(silhouette_wh)
+            self.proj_wh = float(proj_wh)
+
+    def _silhouette_target(self, labels: Dict[str, torch.Tensor], B: int) -> torch.Tensor:
+        tgt = labels["silhouette"]
+        S = self.silhouette_wh
+        if tuple(tgt.shape) != (B, S, S):
+            raise ValueError("labels['silhouette'] has shape {}, expected {}".format(tuple(tgt.shape), (B, S, S)))
+        return tgt
+
+    def silhouette_camera(self, cam: torch.Tensor) -> Tuple[torch.Tensor, float]:
+        """Camera translation (B,3) from the head's weak-perspective cam (differentiable) and the render focal length."""
+        from .cam_utils import convert_weak_perspective_to_camera_translation_torch
+        t = convert_weak_perspective_to_camera_translation_torch(cam, config.FOCAL_LENGTH, self.proj_wh)
+        return t.contiguous(), config.FOCAL_LENGTH * self.silhouette_wh / self.proj_wh
 
     def forward(self, labels: Dict[str, torch.Tensor], outputs: Dict[str, torch.Tensor]):
         total, parts = 0.0, {}
@@ -107,6 +142,13 @@ class MultiTaskLoss(nn.Module):
             add("shape_params", torch.mean((outputs["shape_params"] - labels["shape_params"]) ** 2))
         if "pose_params" in self.losses_on:
             add("pose_params", torch.mean((outputs["pose_params_rot_matrices"] - labels["pose_params_rot_matrices"]) ** 2))
+        if "silhouette" in self.losses_on:
+            if outputs.get("silhouettes") is None:
+                raise ValueError("the silhouette term needs outputs['silhouettes']: pass render_silhouettes to predict")
+            alpha = outputs["silhouettes"]
+            tgt = self._silhouette_target(labels, alpha.shape[0])
+            mask = tgt >= 0.5 if tgt.dtype.is_floating_point else tgt != 0
+            add("silhouette", torch.mean((alpha - mask.to(alpha.dtype)) ** 2))
         return total, parts
 
 
@@ -134,7 +176,16 @@ class MultiTaskLoss(nn.Module):
         loss, parts = ops.multitask_loss(lv, joints=outputs["joints"], cam=outputs["cam"], proj_wh=512.0,
                                          norm_wh=float(config.REGRESSOR_IMG_WH), **kw)
         names = ("verts", "joints2D", "joints3D", "shape_params", "pose_params")
-        return loss, {n: parts[i] for i, n in enumerate(names) if n in on}
+        parts = {n: parts[i] for i, n in enumerate(names) if n in on}
+        if "silhouette" in on:
+            verts = outputs["verts"]
+            t, f = self.silhouette_camera(outputs["cam"])
+            L = ops.silhouette_term(verts, self.silhouette_faces, t, self._silhouette_target(labels, verts.shape[0]),
+                                    self.silhouette_wh, f, self.silhouette_sigma)
+            lv = self.silhouette_log_var
+            parts["silhouette"] = L * torch.exp(-lv)
+            loss = loss + parts["silhouette"] + lv
+        return loss, parts
 
 
 _INDEX_CACHE: Dict[Tuple[str, str], torch.Tensor] = {}
@@ -157,10 +208,12 @@ def _index(name: str, device: torch.device) -> torch.Tensor:
 
 
 def predict(head: nn.Module, smpl: Callable, features: torch.Tensor, rot6d_to_rotmat: Callable,
-            project_pixels: Optional[Callable], need_verts: bool = True) -> Dict[str, torch.Tensor]:
+            project_pixels: Optional[Callable], need_verts: bool = True,
+            render_silhouettes: Optional[Callable] = None) -> Dict[str, torch.Tensor]:
     """PyTorch3DTest.py:1046-1071: head -> rotation matrices -> SMPL -> COCO joints in 3D and in pixels.
     `smpl`, `rot6d_to_rotmat` and `project_pixels(joints, cam) -> (B,90,2) pixels` are injected so that the same
-    code runs on the C-ABI kernels (GPU) and on the oracle (CPU tests)."""
+    code runs on the C-ABI kernels (GPU) and on the oracle (CPU tests).  `render_silhouettes(verts, cam) -> (B,S,S)`
+    soft alpha (PyTorch3DTest.py:1084-1087; `gpu_silhouette_renderer` on the GPU) fills "silhouettes"."""
     cam, pose6d, shape = head(features)
     rotmats = rot6d_to_rotmat(pose6d.contiguous()).view(-1, 24, 3, 3)
     out = smpl(body_pose=rotmats[:, 1:], global_orient=rotmats[:, 0].unsqueeze(1), betas=shape, pose2rot=False,
@@ -171,18 +224,23 @@ def predict(head: nn.Module, smpl: Callable, features: torch.Tensor, rot6d_to_ro
     if project_pixels is not None:       # None: the fused loss projects / gathers inside its kernel
         res["joints2D"] = project_pixels(out.joints, cam).index_select(1, _index("SMPL_TO_KPRCNN_MAP", dev))
         res["joints3D"] = out.joints.index_select(1, _index("ALL_JOINTS_TO_COCO_MAP", dev))
+    if render_silhouettes is not None:
+        res["silhouettes"] = render_silhouettes(out.vertices, cam)
     return res
 
 
 def train_step(head: nn.Module, criterion: MultiTaskLoss, optimiser: torch.optim.Optimizer, smpl: Callable,
                features: torch.Tensor, labels: Dict[str, torch.Tensor], rot6d_to_rotmat: Callable,
-               project_pixels: Optional[Callable], fused_loss: bool = False) -> torch.Tensor:
+               project_pixels: Optional[Callable], fused_loss: bool = False,
+               render_silhouettes: Optional[Callable] = None) -> torch.Tensor:
     """One optimisation step (PyTorch3DTest.py:1097-1102).  When `head` / `criterion` are wrapped in
     DistributedDataParallel the backward all-reduces their gradients (NCCL on the GPUs).  `fused_loss`: evaluate
-    the loss with the fused kernels (CUDA only)."""
+    the loss with the fused kernels (CUDA only).  `render_silhouettes`: see `predict` (the eager silhouette term;
+    the fused one renders inside its kernel)."""
     optimiser.zero_grad(set_to_none=True)
     outputs = predict(head, smpl, features, rot6d_to_rotmat, None if fused_loss else project_pixels,
-                      need_verts="verts" in _tasks(criterion))
+                      need_verts=_needs_verts(criterion), render_silhouettes=_renderer(criterion, fused_loss,
+                                                                                       render_silhouettes))
     crit = getattr(criterion, "module", criterion)
     loss, _ = crit.forward_fused(labels, outputs) if fused_loss else criterion(labels, outputs)
     loss.backward()
@@ -192,6 +250,16 @@ def train_step(head: nn.Module, criterion: MultiTaskLoss, optimiser: torch.optim
 
 def _tasks(criterion) -> Sequence[str]:
     return getattr(criterion, "module", criterion).losses_on
+
+
+def _needs_verts(criterion) -> bool:
+    tasks = _tasks(criterion)
+    return "verts" in tasks or "silhouette" in tasks
+
+
+def _renderer(criterion, fused_loss: bool, render_silhouettes: Optional[Callable]) -> Optional[Callable]:
+    """The renderer `predict` runs: only for the eager loss of a criterion with the silhouette term."""
+    return render_silhouettes if ("silhouette" in _tasks(criterion) and not fused_loss) else None
 
 
 class _BasicBlock(nn.Module):
@@ -270,6 +338,20 @@ def gpu_ops():
     return ops.rot6d_to_rotmat, (lambda joints, cam: ops.orthographic_project(joints, cam, 512.0))
 
 
+def gpu_silhouette_renderer(faces, img_wh: int = config.REGRESSOR_IMG_WH, sigma: float = 1.0,
+                            proj_wh: float = 512.0) -> Callable:
+    """`render_silhouettes(verts, cam) -> (B, img_wh, img_wh)` soft alpha for `predict` on a CUDA device
+    (ops.render_silhouettes with the camera of `SMPL.render_silhouettes` and of MultiTaskLoss's silhouette term)."""
+    from . import ops
+    from .cam_utils import convert_weak_perspective_to_camera_translation_torch
+    f = config.FOCAL_LENGTH * float(img_wh) / float(proj_wh)
+
+    def render(verts: torch.Tensor, cam: torch.Tensor) -> torch.Tensor:
+        t = convert_weak_perspective_to_camera_translation_torch(cam, config.FOCAL_LENGTH, proj_wh)
+        return ops.render_silhouettes(verts, faces, t.contiguous(), img_wh, focal_length=f, sigma=sigma)
+    return render
+
+
 class GraphedTrainStep:
     """The training step of `train_step` captured ONCE in a CUDA graph and replayed: (encoder +) head forward, SMPL
     layer, loss, backward, gradient all-reduce (NCCL) and a capturable Adam step.  The eager step is bound by ~100
@@ -281,13 +363,15 @@ class GraphedTrainStep:
     so the NCCL kernels of the late layers overlap the encoder's backward, as DistributedDataParallel does eagerly.
     The SMPL layer has no parameters: the buckets are the head (+ encoder) and the loss's log-variances.  Inputs are
     copied into static buffers before each replay; `world_size > 1` requires an initialised NCCL process group.
-    `fused_loss`: the loss through the fused kernels of csrc/loss.cu instead of eager PyTorch ops.
+    `fused_loss`: the loss through the fused kernels of csrc/loss.cu instead of eager PyTorch ops (with the
+    silhouette term, ops.silhouette_term); `render_silhouettes`: see `predict`, for the eager loss.  The silhouette
+    label is one more static label buffer.
     """
 
     def __init__(self, head: nn.Module, criterion: MultiTaskLoss, smpl: Callable, features: torch.Tensor,
                  labels: Dict[str, torch.Tensor], rot6d_to_rotmat: Callable, project_pixels: Optional[Callable],
                  lr: float = 1e-4, world_size: int = 1, warmup: int = 3, fused_loss: bool = False,
-                 bucket_mb: float = 8.0, overlap: bool = True):
+                 bucket_mb: float = 8.0, overlap: bool = True, render_silhouettes: Optional[Callable] = None):
         dev = features.device
         if dev.type != "cuda":
             raise RuntimeError("GraphedTrainStep needs CUDA tensors")
@@ -312,7 +396,8 @@ class GraphedTrainStep:
         self.optimiser = torch.optim.Adam(self.params, lr=lr, capturable=True)
         self.features = features.clone()
         self.labels = {k: v.clone() for k, v in labels.items()}
-        need_verts = "verts" in criterion.losses_on
+        need_verts = _needs_verts(criterion)
+        render = _renderer(criterion, fused_loss, render_silhouettes)
         comm = torch.cuda.Stream(device=dev) if (self.world > 1 and overlap) else None
         state = {"pending": list(counts), "sent": [False] * len(self.buckets)}
 
@@ -340,7 +425,7 @@ class GraphedTrainStep:
             self.flat_grad.zero_()
             state["pending"], state["sent"] = list(counts), [False] * len(self.buckets)
             outputs = predict(head, smpl, self.features, rot6d_to_rotmat, None if fused_loss else project_pixels,
-                              need_verts=need_verts)
+                              need_verts=need_verts, render_silhouettes=render)
             loss, _ = criterion.forward_fused(self.labels, outputs) if fused_loss else criterion(self.labels, outputs)
             loss.backward()
             if self.world > 1:
