@@ -46,6 +46,7 @@ blend_fwd_simt_kernel(const float* __restrict__ W32, int n_pad, int nf, const fl
 
 int launch_blend_fwd_simt(const DevModel& m, const float* featf, int S, int Sw, float* vpT, int row_begin,
                           int row_end, cudaStream_t st) {
+  if (row_begin >= row_end) return 0;        // joints only, and the model has no virtual joint rows
   dim3 grid((row_end - row_begin) / 32, Sw / 32);
   LaunchTimer _timer_46("blend_fwd_simt", st);
   blend_fwd_simt_kernel<<<grid, dim3(32, 8), 0, st>>>(m.W32, m.n_pad, m.fl.nf, featf, m.fl.nf_pad, S, vpT,

@@ -482,6 +482,8 @@ int build_bs_work(int bp_total, int wtp_total, int tpcs, BsWork& work) {
 // bodies wide (make_plan), which the work list always fits.
 int launch_blend_fwd_umma(const DevModel& m, int mode, const __nv_bfloat16* feat, int S, int Sw, float* vpT,
                           int row_begin, int row_end, int num_sms, cudaStream_t st) {
+  // a joints-only call on a model without picked or regressed joints has no rows to blend
+  if (row_begin >= row_end) return 0;
   const int pslabs = m.fl.pseg / BK;
   const int use_lo = (mode == B200SMPL_MODE_BF16) ? 0 : 1;
   if (1 + 2 * pslabs > WS_MAX_SLABS) return fail(B200SMPL_ERR_INVALID, "feature pitch too large for the resident operand");

@@ -85,6 +85,8 @@ class SMPLEngine:
         data, nbytes = ctypes.c_void_p(), ctypes.c_size_t()
         _lib.check(self.lib.b200smpl_model_debug_array(self.handle, name.encode(), ctypes.byref(data),
                                                        ctypes.byref(nbytes)), "b200smpl_model_debug_array")
+        if nbytes.value == 0:                 # an empty table (a model without virtual joint rows) has no address
+            return np.zeros(0, dtype=dtype)
         buf = (ctypes.c_uint8 * nbytes.value).from_address(data.value)
         return np.frombuffer(buf, dtype=dtype).copy()
 

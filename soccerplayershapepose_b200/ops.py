@@ -23,6 +23,10 @@ def _req(t: torch.Tensor, name: str) -> torch.Tensor:
     return t.contiguous()
 
 
+def _aligned8(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
+    return t if t is None or t.data_ptr() % 8 == 0 else t.clone(memory_format=torch.contiguous_format)
+
+
 class _Rot6d(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x):
@@ -261,6 +265,9 @@ class _MultiTaskLoss(torch.autograd.Function):
         verts, joints, cam = f(verts, "verts"), f(joints, "joints"), f(cam, "cam")
         shape, pose = f(shape, "shape"), f(pose, "pose")
         verts_label, label2d, label3d = f(verts_label, "verts_label"), f(label2d, "label2d"), f(label3d, "label3d")
+        # the vertex term reads 8-byte pieces: a contiguous slice that starts 4 bytes off (e.g. a narrow of a flat
+        # buffer) is copied into fresh storage
+        verts, verts_label = _aligned8(verts), _aligned8(verts_label)
         shape_label, pose_label = f(shape_label, "shape_label"), f(pose_label, "pose_label")
         ref = joints if joints is not None else (verts if verts is not None else (shape if shape is not None else pose))
         if ref is None:
