@@ -42,6 +42,13 @@ from .smpl import SMPL
 FROZEN_FULL_JOINTS = (7, 8, 22, 23)       # body_pose[:, 6:8] and body_pose[:, 21:] in full-pose numbering
 
 
+def _target_masks(silhouettes: torch.Tensor, shape: tuple, dev: torch.device) -> torch.Tensor:
+    """The fitters' target masks: `silhouettes` of the given shape as bool on `dev`, non-zero is inside."""
+    if tuple(silhouettes.shape) != shape:
+        raise ValueError("silhouettes has shape {}, expected {}".format(tuple(silhouettes.shape), shape))
+    return silhouettes.to(device=dev) != 0
+
+
 class BatchedFitter:
     def __init__(self, smpl: SMPL, lr: float = 1e-3, shape_weight: float = 0.0, joints2d_log_var: float = 0.0,
                  proj_wh: float = 512.0, norm_wh: float = float(config.REGRESSOR_IMG_WH),
@@ -91,7 +98,8 @@ class BatchedFitter:
             None if vis is None else vis.data_ptr(), st["betas"].data_ptr(), B, joints.shape[1], self.jmap.numel(),
             st["betas"].shape[1], self.proj_wh, self.norm_wh, self.log_var, self.shape_weight, st["loss"].data_ptr(),
             st["gj"].data_ptr(), st["gcam"].data_ptr(), st["gbetas_prior"].data_ptr(), stream), "fit_loss")
-        cam_extra = self._silhouette_term(st, verts, stream) if sil else None
+        cam_extra = self._silhouette_term(verts, st["cam"], st["sil"], st["loss"], st["gv"], st["t"], st["gt"],
+                                          st["gcam_sil"], stream) if sil else None
         gb, gp, _, _ = self.eng.backward(st["betas"], st["rot"], None, None, None, st["gv"] if sil else None, st["gj"],
                                          None, axis_angle=False, mode=self.mode, need_transl=False, need_cam=False,
                                          saved=saved)
@@ -110,22 +118,35 @@ class BatchedFitter:
                    "fit_update")
         self._parity ^= 1
 
-    def _silhouette_term(self, st: Dict[str, torch.Tensor], verts: torch.Tensor, stream) -> torch.Tensor:
-        """Adds the silhouette term to st['loss'], writes d loss / d vertices to st['gv'] and returns d loss / d cam
-        through t = [tx, ty, 2 f / (proj_wh s + 1e-9)] (cam_utils.py:44-52), the cam group's extra gradient."""
-        cam, t, gt, gce = st["cam"], st["t"], st["gt"], st["gcam_sil"]
+    # ---- the silhouette term on caller-owned buffers (this fitter's iteration and MultiViewFitter's view steps) -----
+    def _silhouette_args(self, verts: torch.Tensor, cam: torch.Tensor, t: torch.Tensor):
+        """Writes t = [tx, ty, 2 f / (proj_wh s + 1e-9)] (cam_utils.py:44-52) of the weak-perspective `cam` (B,3) into
+        `t` and returns the rasteriser's arguments for `verts` seen through it, with proj_wh s + 1e-9."""
+        from .ops import silhouette_args
         f = config.FOCAL_LENGTH
         den = self.proj_wh * cam[:, 0] + 1e-9
         t[:, :2] = cam[:, 1:]
         t[:, 2] = (2 * f) / den
-        from .ops import silhouette_args
-        args = silhouette_args(verts, self.faces, t, self.sil_wh, f * self.sil_wh / self.proj_wh, self.sil_sigma)
-        _lib.check(self.lib.b200smpl_silhouette_loss(ctypes.byref(args), st["sil"].data_ptr(), self.sil_weight,
-                                                     st["loss"].data_ptr(), st["gv"].data_ptr(), gt.data_ptr(), stream),
+        return silhouette_args(verts, self.faces, t, self.sil_wh, f * self.sil_wh / self.proj_wh, self.sil_sigma), den
+
+    def _silhouette_term(self, verts: torch.Tensor, cam: torch.Tensor, target: torch.Tensor, loss: torch.Tensor,
+                         gv: torch.Tensor, t: torch.Tensor, gt: torch.Tensor, gcam: torch.Tensor, stream) -> torch.Tensor:
+        """Adds `silhouette_weight * mean((alpha - target)^2)` to `loss` (B,), writes d loss / d vertices to `gv` and
+        returns d loss / d cam chained through t (`gcam`, the camera's extra gradient); `t`, `gt` are (B,3) scratch."""
+        args, den = self._silhouette_args(verts, cam, t)
+        _lib.check(self.lib.b200smpl_silhouette_loss(ctypes.byref(args), target.data_ptr(), self.sil_weight,
+                                                     loss.data_ptr(), gv.data_ptr(), gt.data_ptr(), stream),
                    "silhouette_loss")
-        gce[:, 0] = -gt[:, 2] * (2 * f * self.proj_wh) / (den * den)
-        gce[:, 1:] = gt[:, :2]
-        return gce
+        gcam[:, 0] = -gt[:, 2] * (2 * config.FOCAL_LENGTH * self.proj_wh) / (den * den)
+        gcam[:, 1:] = gt[:, :2]
+        return gcam
+
+    def _silhouette_value(self, verts: torch.Tensor, cam: torch.Tensor, target: torch.Tensor, loss: torch.Tensor,
+                          t: torch.Tensor, stream) -> None:
+        """Adds the same term to `loss` without its gradient (b200smpl_silhouette_loss_value: validation passes)."""
+        args, _ = self._silhouette_args(verts, cam, t)
+        _lib.check(self.lib.b200smpl_silhouette_loss_value(ctypes.byref(args), target.data_ptr(), self.sil_weight,
+                                                           loss.data_ptr(), stream), "silhouette_loss_value")
 
     def silhouette_iou(self, rotmats: torch.Tensor, betas: torch.Tensor, cam: torch.Tensor,
                        silhouettes: torch.Tensor) -> torch.Tensor:
@@ -149,9 +170,7 @@ class BatchedFitter:
         B = rotmats.shape[0]
         f32 = dict(dtype=torch.float32, device=dev)
         use_sil = silhouettes is not None and self.sil_weight > 0.0
-        if silhouettes is not None and tuple(silhouettes.shape) != (B, self.sil_wh, self.sil_wh):
-            raise ValueError("silhouettes has shape {}, expected {}".format(tuple(silhouettes.shape),
-                                                                           (B, self.sil_wh, self.sil_wh)))
+        masks = None if silhouettes is None else _target_masks(silhouettes, (B, self.sil_wh, self.sil_wh), dev)
         # the state buffers (and the graph captured over them) are kept per problem shape and reused by later calls
         key = (B, int(betas.shape[1]), vis is not None) + (("sil",) if use_sil else ())
         cached = self._cache.get(key)
@@ -188,7 +207,7 @@ class BatchedFitter:
         if vis is not None:
             st["vis"].copy_(vis.to(device=dev, dtype=torch.uint8))
         if use_sil:
-            st["sil"].copy_(silhouettes.to(device=dev) != 0)
+            st["sil"].copy_(masks)
         for name in ("rot", "betas", "cam"):
             st["m_" + name].zero_()
             st["v_" + name].zero_()
@@ -256,21 +275,28 @@ class MultiViewFitter:
     `optim.Adam([cam_wp_mult, global_orient_mult])` does.  After the training pass every view is evaluated again
     (the `is_train = False` pass) and the parameters of the epoch are kept when the summed validation loss is the
     best the player has seen in any phase so far (:1823-1838, 1938-1954); each phase ends by restoring its
-    parameters to their best epoch (:1846-1847, 1961-1962).  Differences, stated: the loss is the joints2D term only
-    (the silhouette term of `BatchedFitter` is not wired into this loop), model selection uses that loss instead of the
-    metrics tracker's joints2D / silhouette metrics, and the shuffled view order of an epoch is shared by all
-    players of the batch (the reference shuffles per player).
+    parameters to their best epoch (:1846-1847, 1961-1962).  The loss of a view is the joints2D term, plus, with
+    `fit(..., silhouettes=masks)` and silhouette_weight > 0, the silhouette term of `BatchedFitter` on that view's
+    mask, seen through that view's camera.  Differences, stated: model selection uses the summed validation loss
+    instead of the metrics tracker's joints2D / silhouette metrics, and the shuffled view order of an epoch is shared
+    by all players of the batch (the reference shuffles per player).
 
-    Every step is the C-ABI sequence of `BatchedFitter` (joints-only forward, fused loss, backward, fused Adam);
-    the glue between steps (slice copies, the per-epoch comparison) is a handful of tiny elementwise torch ops.
+    Every step is the C-ABI sequence of `BatchedFitter` (joints-only forward, fused loss, backward, fused Adam; with
+    the silhouette term the full-vertex forward, fit_loss, the fused silhouette loss and the backward with vertex
+    gradients); the glue between steps (slice copies, the per-epoch comparison) is a handful of tiny elementwise torch
+    ops.  The validation pass adds the silhouette term through the gradient-free value kernel.
     """
 
     def __init__(self, smpl: SMPL, lr: float = 1e-3, rounds: int = 3, shape_weight: float = 0.0,
                  joints2d_log_var: float = 0.0, proj_wh: float = 512.0, norm_wh: float = float(config.REGRESSOR_IMG_WH),
                  betas: tuple = (0.9, 0.999), eps: float = 1e-8, mode: Optional[str] = None,
-                 use_cuda_graph: bool = True):
+                 use_cuda_graph: bool = True, silhouette_weight: float = 0.0, silhouette_sigma: float = 1.0,
+                 silhouette_wh: int = 256):
+        """silhouette_weight, silhouette_sigma and silhouette_wh: as in `BatchedFitter`."""
         self.base = BatchedFitter(smpl, lr=lr, shape_weight=shape_weight, joints2d_log_var=joints2d_log_var,
-                                  proj_wh=proj_wh, norm_wh=norm_wh, betas=betas, eps=eps, use_cuda_graph=False, mode=mode)
+                                  proj_wh=proj_wh, norm_wh=norm_wh, betas=betas, eps=eps, use_cuda_graph=False, mode=mode,
+                                  silhouette_weight=silhouette_weight, silhouette_sigma=silhouette_sigma,
+                                  silhouette_wh=silhouette_wh)
         self.rounds = int(rounds)
         self.use_graph = bool(use_cuda_graph)
         dev = self.base.dev
@@ -291,17 +317,19 @@ class MultiViewFitter:
             ctypes.c_void_p(torch.cuda.current_stream(b.dev).cuda_stream)), "fit_adam_step")
 
     def _loss(self, st, v, need_grad):
-        """Forward of view v with the current parameters; fills st['loss'] (and the gradients).  The training pass
-        keeps the forward's transforms and joint rows for its backward (no pose stage / blend GEMM recomputation)."""
+        """Forward of view v with the current parameters; fills st['loss'] (and the gradients, with the silhouette
+        term's camera gradient or None).  The training pass keeps the forward's transforms and blend rows for its
+        backward (no pose stage / blend GEMM recomputation)."""
         b = self.base
+        sil = "sil" in st
         st["rot"][:, :9] = st["go"][v]
         if need_grad:
-            _, joints, _, saved = b.eng.forward(st["betas"], st["rot"], None, None, axis_angle=False, mode=b.mode,
-                                                want_vertices=False, save=True, saved_buffer=st.get("saved"))
+            verts, joints, _, saved = b.eng.forward(st["betas"], st["rot"], None, None, axis_angle=False, mode=b.mode,
+                                                    want_vertices=sil, save=True, saved_buffer=st.get("saved"))
             st["saved"] = saved
         else:
-            _, joints, _ = b.eng.forward(st["betas"], st["rot"], None, None, axis_angle=False, mode=b.mode,
-                                         want_vertices=False)
+            verts, joints, _ = b.eng.forward(st["betas"], st["rot"], None, None, axis_angle=False, mode=b.mode,
+                                             want_vertices=sil)
         vis = st.get("vis")
         stream = ctypes.c_void_p(torch.cuda.current_stream(b.dev).cuda_stream)
         P = st["rot"].shape[0]
@@ -311,14 +339,19 @@ class MultiViewFitter:
             st["betas"].shape[1], b.proj_wh, b.norm_wh, b.log_var, b.shape_weight, st["loss"].data_ptr(),
             st["gj"].data_ptr(), st["gcam"].data_ptr(), st["gbetas_prior"].data_ptr(), stream), "fit_loss")
         if not need_grad:
+            if sil:
+                b._silhouette_value(verts, st["cam"][v], st["sil"][v], st["loss"], st["t"], stream)
             return None
-        gb, gp, _, _ = b.eng.backward(st["betas"], st["rot"], None, None, None, None, st["gj"], None,
-                                      axis_angle=False, mode=b.mode, need_transl=False, need_cam=False, saved=st["saved"])
-        return gb, gp
+        cam_extra = b._silhouette_term(verts, st["cam"][v], st["sil"][v], st["loss"], st["gv"], st["t"], st["gt"],
+                                       st["gcam_sil"], stream) if sil else None
+        gb, gp, _, _ = b.eng.backward(st["betas"], st["rot"], None, None, None, st["gv"] if sil else None, st["gj"],
+                                      None, axis_angle=False, mode=b.mode, need_transl=False, need_cam=False,
+                                      saved=st["saved"])
+        return gb, gp, cam_extra
 
     # ---- static state + the two kinds of work units (one optimiser step on one view; one validation pass) --------
-    def _state(self, P, V, nb, has_vis):
-        key = (P, V, nb, has_vis)
+    def _state(self, P, V, nb, has_vis, use_sil):
+        key = (P, V, nb, has_vis) + (("sil",) if use_sil else ())
         c = self._cache.get(key)
         if c is not None:
             return c
@@ -332,6 +365,11 @@ class MultiViewFitter:
               "gbetas_prior": torch.zeros((P, nb), **f32)}
         if has_vis:
             st["vis"] = torch.empty((V, P, b.jmap.numel()), dtype=torch.uint8, device=dev)
+        if use_sil:
+            st["sil"] = torch.empty((V, P, b.sil_wh, b.sil_wh), dtype=torch.uint8, device=dev)
+            st["gv"] = torch.empty((P, b.eng.num_verts, 3), **f32)
+            for name in ("t", "gt", "gcam_sil"):
+                st[name] = torch.empty((P, 3), **f32)
         c = {"st": st,
              # dense per-view gradients: all zero except the slice of the view being stepped (written before the
              # Adam launch, cleared after it) -- the other views move by their momentum only, as under
@@ -350,12 +388,14 @@ class MultiViewFitter:
     def _view_step(self, c, phase, v):
         st, step, mom, never = c["st"], c["step"], c["mom"], c["never"]
         V, P = st["go"].shape[0], st["go"].shape[1]
-        gb, gp = self._loss(st, v, need_grad=True)
+        gb, gp, cam_extra = self._loss(st, v, need_grad=True)
         step += self._inc
         if phase == "A":                                        # per-view camera and global orientation
             g_go, g_cam = c["g_go"], c["g_cam"]
             g_go[v] = gp[:, :9]
             g_cam[v] = st["gcam"]
+            if cam_extra is not None:                           # the silhouette's pull through t
+                g_cam[v].add_(cam_extra)
             self._adam(st["go"].view(V * P, 9), g_go.view(V * P, 9), None, mom["go"][0].view(V * P, 9),
                        mom["go"][1].view(V * P, 9), step, None, never)
             self._adam(st["cam"].view(V * P, 3), g_cam.view(V * P, 3), None, mom["cam"][0].view(V * P, 3),
@@ -407,10 +447,13 @@ class MultiViewFitter:
 
     def fit(self, body_pose: torch.Tensor, betas: torch.Tensor, global_orient: torch.Tensor, cam: torch.Tensor,
             keypoints2d: torch.Tensor, vis: Optional[torch.Tensor] = None, iterations: int = 10,
-            view_orders=None, seed: int = 0) -> Dict[str, torch.Tensor]:
+            view_orders=None, seed: int = 0, silhouettes: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
         """body_pose (P,23,3,3) and betas (P,10) shared by the views; global_orient (P,V,3,3), cam (P,V,3),
         keypoints2d (P,V,17,2) [, vis (P,V,17)] per view.  `iterations` epochs per phase.  `view_orders`: optional
         list (one per epoch, in execution order: round 0 phase A, round 0 phase B, ...) of view permutations.
+        silhouettes (P, V, silhouette_wh, silhouette_wh) target masks or None: with silhouette_weight > 0 every view's
+        loss, in the steps and in the validation passes, gains the silhouette term; either way the result then carries
+        `silhouette_iou` (P,V) of the returned parameters.
 
         With `use_cuda_graph` the work units -- (phase, view) optimiser steps and the two validation passes -- are
         captured once per problem shape over static state buffers and replayed: an epoch is V + 1 graph launches
@@ -419,8 +462,12 @@ class MultiViewFitter:
         dev = b.dev
         f32 = dict(dtype=torch.float32, device=dev)
         P, V = global_orient.shape[0], global_orient.shape[1]
-        c = self._state(P, V, int(betas.shape[1]), vis is not None)
+        use_sil = silhouettes is not None and b.sil_weight > 0.0
+        masks = None if silhouettes is None else _target_masks(silhouettes, (P, V, b.sil_wh, b.sil_wh), dev)
+        c = self._state(P, V, int(betas.shape[1]), vis is not None, use_sil)
         st = c["st"]
+        if use_sil:
+            st["sil"].copy_(masks.transpose(0, 1))
         st["go"].copy_(global_orient.to(**f32).reshape(P, V, 9).transpose(0, 1))
         st["cam"].copy_(cam.to(**f32).transpose(0, 1))
         st["label"].copy_(keypoints2d.to(**f32).transpose(0, 1))
@@ -463,11 +510,22 @@ class MultiViewFitter:
 
         go = final["go"].transpose(0, 1).reshape(P, V, 3, 3).contiguous()
         cam_out = final["cam"].transpose(0, 1).contiguous()
-        return {"body_pose": final["bp"].reshape(P, 23, 3, 3).clone(), "betas": final["betas"].clone(), "global_orient": go,
-                "cam": cam_out,
-                "translation": convert_weak_perspective_to_camera_translation_torch(
-                    cam_out.reshape(P * V, 3), config.FOCAL_LENGTH, b.proj_wh).reshape(P, V, 3),
-                "best_loss": c["best_metric"].clone(), "initial_loss": first_val,
-                "last": {"body_pose": st["bp"].reshape(P, 23, 3, 3).clone(), "betas": st["betas"].clone(),
-                         "global_orient": st["go"].transpose(0, 1).reshape(P, V, 3, 3).clone(),
-                         "cam": st["cam"].transpose(0, 1).clone()}}
+        out = {"body_pose": final["bp"].reshape(P, 23, 3, 3).clone(), "betas": final["betas"].clone(), "global_orient": go,
+               "cam": cam_out,
+               "translation": convert_weak_perspective_to_camera_translation_torch(
+                   cam_out.reshape(P * V, 3), config.FOCAL_LENGTH, b.proj_wh).reshape(P, V, 3),
+               "best_loss": c["best_metric"].clone(), "initial_loss": first_val,
+               "last": {"body_pose": st["bp"].reshape(P, 23, 3, 3).clone(), "betas": st["betas"].clone(),
+                        "global_orient": st["go"].transpose(0, 1).reshape(P, V, 3, 3).clone(),
+                        "cam": st["cam"].transpose(0, 1).clone()}}
+        if silhouettes is not None:
+            out["silhouette_iou"] = self.silhouette_iou(out["body_pose"], out["betas"], go, cam_out, silhouettes)
+        return out
+
+    def silhouette_iou(self, body_pose: torch.Tensor, betas: torch.Tensor, global_orient: torch.Tensor,
+                       cam: torch.Tensor, silhouettes: torch.Tensor) -> torch.Tensor:
+        """IoU (P,V) of the binary silhouette of every view against `silhouettes` (P,V,S,S), shapes as in `fit`
+        (`BatchedFitter.silhouette_iou` per view)."""
+        return torch.stack([self.base.silhouette_iou(torch.cat([global_orient[:, v:v + 1], body_pose], 1), betas,
+                                                     cam[:, v], silhouettes[:, v])
+                            for v in range(global_orient.shape[1])], 1)
