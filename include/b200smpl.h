@@ -355,6 +355,32 @@ B200SMPL_API int b200smpl_silhouette_loss(const b200smpl_silhouette_args* args, 
 B200SMPL_API int b200smpl_silhouette_loss_value(const b200smpl_silhouette_args* args, const uint8_t* target,
                                                 float weight, float* loss_per_body, void* stream);
 
+/*
+ * The regressor's input on the device -- replaces the reference's per-crop host code create_proxy_representation
+ * (predict/predict_3D.py:67-81) over convert_2Djoints_to_gaussian_heatmaps (utils/label_conversions.py:58-87).
+ * Definition (DESIGN.md section 12): out[b] is (1 + K, out_wh, out_wh) fp32 with
+ *   channel 0     the binary mask resized by nearest neighbour: out[b][0][y][x] = masks[b][(y in_wh) / out_wh]
+ *                 [(x in_wh) / out_wh] != 0 (exact integer division; cv2.INTER_NEAREST for 512 -> 256);
+ *   channel 1 + j keypoint j scaled by out_wh / in_wh in double precision and truncated toward zero to (cu, cv)
+ *                 (the reference's astype(np.int16)); out[b][1 + j][v][u] = exp(-((u-cu)/std)^2/2 - ((v-cv)/std)^2/2)
+ *                 for integer pixel coordinates u, v.  The channel is all zero when vis[b][j] == 0, when the keypoint
+ *                 is not finite or when a truncated centre leaves the int16 range (numpy's cast would wrap it).
+ * masks [B][in_wh][in_wh] uint8 (non-zero = inside), keypoints [B][K][2] pixels (x, y) of the in_wh image, vis [B][K]
+ * uint8 or NULL (all visible).  out is [B][1 + K][out_wh][out_wh] (channels_last = 0) or [B][out_wh][out_wh][1 + K]
+ * (channels_last = 1, torch.channels_last strides of the same logical shape), at any 4-byte-aligned address.
+ * Sizes: batch >= 1, 1 <= in_wh, out_wh <= 16384, 1 <= num_keypoints <= B200SMPL_PROXY_MAX_KEYPOINTS, finite std > 0
+ * (output pixels; 4 in the reference); otherwise B200SMPL_ERR_INVALID.  One kernel launch, no workspace.
+ */
+#define B200SMPL_PROXY_MAX_KEYPOINTS 32
+typedef struct b200smpl_proxy_args {
+  int32_t batch, in_wh, out_wh, num_keypoints, channels_last, reserved0;
+  float std;
+  const uint8_t* masks;      /* [B][in_wh][in_wh], non-zero = inside */
+  const float* keypoints;    /* [B][K][2] pixels of the in_wh image */
+  const uint8_t* vis;        /* [B][K] or NULL */
+} b200smpl_proxy_args;
+B200SMPL_API int b200smpl_proxy_representation(const b200smpl_proxy_args* args, float* out, void* stream);
+
 /* Test hook (host arithmetic only, no device): the cluster work list of the forward blend GEMM for `body_tiles`
  * 128-body tiles x `row_tiles` 128-row tiles on a device with `num_sms` SMs.  Writes (body-tile pair, first row-tile
  * pair, end row-tile pair) per cluster into out[3 * capacity]; returns the number of clusters or -1. */

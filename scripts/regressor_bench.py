@@ -3,7 +3,7 @@
 loss (verts, joints2D, joints3D, shape, pose) -> backward -> gradient all-reduce -> Adam, batch 256 crops per step
 per GPU, data-parallel over NCCL when launched under torchrun.  One CUDA graph per step.
 
-  python scripts/regressor_bench.py [--steps 50] [--batch 256] [--input encoder|features] [--res 256]
+  python scripts/regressor_bench.py [--steps 50] [--batch 256] [--input encoder|proxy|features] [--res 256]
                                     [--loss fused|eager] [--no-overlap] [--eager]
                                     [--silhouette-weight W [--sil-res S] [--sil-sigma SIGMA]]
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 scripts/regressor_bench.py ...
@@ -11,6 +11,9 @@ per GPU, data-parallel over NCCL when launched under torchrun.  One CUDA graph p
 --input encoder (default): the reference's SingleInputRegressor (models/regressor.py: ResNet-18 over 18 x res x res
 proxy inputs + IEFModule([512,512])), 11.9 M parameters = 47.6 MB all-reduced per step.  BASELINE.json says 224x224
 crops; the reference's regressor input is 18x256x256 (config.REGRESSOR_IMG_WH, PyTorch3DTest.py:241): --res picks.
+--input proxy: the same encoder step fed what a detector gives instead of finished proxies: 512 x 512 uint8 masks (the
+label bodies' hard silhouettes) and the 17 COCO keypoints of labels["joints2D"] (512-px); the captured step builds
+the 18 x res x res proxy itself (ops.proxy_representation, channels_last), so a step copies only the raw inputs.
 --input features: synthetic 512-d features into IEFModule([1024,1024]) (the round-1 head-only configuration).
 --silhouette-weight W > 0 adds the silhouette term (initial weight W; PyTorch3DTest.py:1084-1087) at S x S pixels:
 the targets are the hard silhouettes of the label bodies; the fused loss runs ops.silhouette_term, the eager loss
@@ -29,7 +32,7 @@ from soccerplayershapepose_b200.synthetic_inputs import make_smpl_inputs        
 ap = argparse.ArgumentParser()
 ap.add_argument("--steps", type=int, default=50)
 ap.add_argument("--batch", type=int, default=256)
-ap.add_argument("--input", default="encoder", choices=["encoder", "features"])
+ap.add_argument("--input", default="encoder", choices=["encoder", "proxy", "features"])
 ap.add_argument("--res", type=int, default=256)
 ap.add_argument("--loss", default="fused", choices=["fused", "eager"])
 ap.add_argument("--no-overlap", action="store_true", help="one all-reduce after the backward instead of bucketed overlap")
@@ -48,7 +51,7 @@ if world > 1:
     dist.init_process_group("nccl", device_id=dev)
 smpl = SMPL(model_data=make_synthetic_smpl(1234), mode="fp32").to(dev)
 torch.manual_seed(0)
-if args.input == "encoder":
+if args.input in ("encoder", "proxy"):
     head = regressor.SingleInputRegressor(resnet_in_channels=18).to(dev).to(memory_format=torch.channels_last)
     if args.amp:
         enc_fwd = head.image_encoder.forward
@@ -94,6 +97,9 @@ with torch.no_grad():
               "joints2D": ops.orthographic_project(t.joints, cam, 512.0)[:, config.SMPL_TO_KPRCNN_MAP, :].contiguous()}
     if sil:
         labels["silhouette"] = smpl.render_silhouettes(t.vertices, cam, img_wh=args.sil_res, sigma=0.0) > 0.5
+    if args.input == "proxy":
+        masks = (smpl.render_silhouettes(t.vertices, cam, img_wh=512, sigma=0.0, proj_wh=512) > 0.5).to(torch.uint8)
+        feats = regressor.ProxyInputs(masks, labels["joints2D"], None, args.res)
 
 if args.eager:
     model = Step()
@@ -103,7 +109,10 @@ if args.eager:
 
     def step():
         opt.zero_grad(set_to_none=True)
-        loss = model(feats, labels)
+        f = feats
+        if args.input == "proxy":
+            f = ops.proxy_representation(feats.masks, feats.keypoints, None, args.res, channels_last=True)
+        loss = model(f, labels)
         loss.backward()
         opt.step()
         return loss
@@ -127,10 +136,25 @@ e1.record()
 torch.cuda.synchronize()
 ms = sharding.max_over_ranks(e0.elapsed_time(e1), dev)
 nparams = sum(p.numel() for p in list(head.parameters()) + list(crit.parameters()))
+
+
+def power_limit():
+    import subprocess
+    try:
+        r = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader,nounits", "-i", str(local)],
+                           capture_output=True, text=True, timeout=30)
+        return float(r.stdout.strip().splitlines()[0])
+    except Exception:                          # noqa: BLE001
+        return "not read"
+
+
 if rank == 0:
     what = ("18x%dx%d crops -> ResNet-18%s -> IEF head (512,512)" % (args.res, args.res, " (bf16 autocast)" if args.amp else " (fp32/TF32 cuDNN)")
-            if args.input == "encoder"
+            if args.input != "features"
             else "512-d features -> IEF head (1024,1024)")
+    if args.input == "proxy":
+        what = "512x512 uint8 masks + 17 keypoints -> proxy kernel -> " + what
+    nbytes = lambda ts: sum(x.numel() * x.element_size() for x in ts if x is not None)   # noqa: E731
     terms = "5-term" if not sil else "6-term (+ silhouette at %dx%d, sigma %g, weight %g)" % (
         args.sil_res, args.sil_res, args.sil_sigma, args.silhouette_weight)
     print(json.dumps({"workload": "BASELINE.json configs[4]: regressor step: %s -> SMPL -> %s multi-task loss (%s kernels), "
@@ -141,6 +165,9 @@ if rank == 0:
                       "allreduce": "none" if world == 1 else ("DistributedDataParallel" if args.eager else
                                                               ("one flat all-reduce after the backward" if args.no_overlap
                                                                else "8 MB buckets on a side stream, overlapped with the backward (forked inside the graph)")),
+                      "input": args.input, "card": torch.cuda.get_device_name(dev), "power_limit_w": power_limit(),
+                      "input_bytes_copied_per_step": nbytes(feats[:3] if args.input == "proxy" else [feats]),
+                      "label_bytes_copied_per_step": nbytes(labels.values()),
                       "loss_first": float(l0), "loss_last": float(l1)}))
 if world > 1:
     torch.cuda.synchronize()

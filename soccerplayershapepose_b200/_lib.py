@@ -89,6 +89,17 @@ class SilhouetteArgs(Structure):
     ]
 
 
+PROXY_MAX_KEYPOINTS = 32
+
+
+class ProxyArgs(Structure):
+    _fields_ = [
+        ("batch", c_int32), ("in_wh", c_int32), ("out_wh", c_int32), ("num_keypoints", c_int32),
+        ("channels_last", c_int32), ("reserved0", c_int32), ("std", c_float),
+        ("masks", c_void_p), ("keypoints", c_void_p), ("vis", c_void_p),
+    ]
+
+
 # every symbol include/b200smpl.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "b200smpl_model_create": (c_int, [POINTER(ModelDesc), c_int, POINTER(c_void_p)]),
@@ -133,6 +144,7 @@ SYMBOLS = {
     "b200smpl_silhouette_loss": (c_int, [POINTER(SilhouetteArgs), c_void_p, c_float, c_void_p, c_void_p, c_void_p,
                                          c_void_p]),
     "b200smpl_silhouette_loss_value": (c_int, [POINTER(SilhouetteArgs), c_void_p, c_float, c_void_p, c_void_p]),
+    "b200smpl_proxy_representation": (c_int, [POINTER(ProxyArgs), c_void_p, c_void_p]),
     "b200smpl_debug_fwd_gemm_worklist":(c_int, [c_int, c_int, c_int, c_void_p, c_int]),
     "b200smpl_last_error": (c_char_p, []),
     "b200smpl_abi_version": (c_int, []),

@@ -545,3 +545,56 @@ def silhouette_iou(pred: torch.Tensor, target: torch.Tensor) -> torch.Tensor:
     inter = (p & t).flatten(1).sum(1).double()
     union = (p | t).flatten(1).sum(1).double()
     return torch.where(union > 0, inter / union.clamp(min=1), torch.ones_like(union)).float()
+
+
+# ---- the regressor's input (DESIGN.md section 12) ----------------------------------------------------------------------
+def proxy_representation(masks: torch.Tensor, keypoints: torch.Tensor, vis: Optional[torch.Tensor] = None,
+                         out_wh: int = config.REGRESSOR_IMG_WH, std: float = 4.0, channels_last: bool = False,
+                         out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """The regressor's 1 + K channel input built on the device in one kernel (create_proxy_representation,
+    predict/predict_3D.py:67-81, over convert_2Djoints_to_gaussian_heatmaps, utils/label_conversions.py:58-87):
+    masks (B, in_wh, in_wh) bool / uint8 (non-zero is inside) or floating point (`>= 0.5`), keypoints (B, K, 2)
+    float32 pixels (x, y) of the in_wh image, vis (B, K) or None (non-zero = visible) -> (B, 1 + K, out_wh, out_wh)
+    float32: channel 0 the nearest-neighbour resize of the mask, channel 1 + j a Gaussian of std `std` output pixels
+    around keypoint j scaled to out_wh and truncated to integers; an invisible or non-finite keypoint gives a zero
+    channel.  channels_last: the result (or `out`) has torch.channels_last strides.  `out`: a preallocated float32
+    tensor of that shape and memory format to write (e.g. a CUDA graph's static buffer).  Plain tensor ops and one
+    C-ABI call, so a CUDA graph can capture it."""
+    if not masks.is_cuda:
+        raise RuntimeError("masks must be a CUDA tensor: the b200 ops have no CPU implementation")
+    if masks.dim() != 3 or masks.shape[1] != masks.shape[2]:
+        raise ValueError("masks has shape {}, expected (B, in_wh, in_wh)".format(tuple(masks.shape)))
+    B, in_wh, dev = masks.shape[0], masks.shape[1], masks.device
+    if masks.dtype == torch.uint8:
+        m8 = masks.contiguous()
+    elif masks.dtype == torch.bool:
+        m8 = masks.contiguous().view(torch.uint8)
+    elif masks.dtype.is_floating_point:
+        m8 = _binary_target(masks, B, in_wh, dev)
+    else:
+        raise TypeError("masks must be bool, uint8 or floating point, got {}".format(masks.dtype))
+    kp = _req(keypoints, "keypoints")
+    if kp.device != dev or kp.dim() != 3 or kp.shape[0] != B or kp.shape[2] != 2:
+        raise ValueError("keypoints has shape {} on {}, expected ({}, K, 2) on {}".format(
+            tuple(kp.shape), kp.device, B, dev))
+    K, S = kp.shape[1], int(out_wh)
+    if not 1 <= K <= _lib.PROXY_MAX_KEYPOINTS:
+        raise ValueError("need 1 <= K <= {} keypoints, got {}".format(_lib.PROXY_MAX_KEYPOINTS, K))
+    v8 = None
+    if vis is not None:
+        if vis.device != dev or tuple(vis.shape) != (B, K):
+            raise ValueError("vis has shape {} on {}, expected {} on {}".format(tuple(vis.shape), vis.device, (B, K), dev))
+        v8 = (vis != 0).to(torch.uint8)
+    fmt = torch.channels_last if channels_last else torch.contiguous_format
+    if out is None:
+        out = torch.empty((B, 1 + K, S, S), dtype=torch.float32, device=dev, memory_format=fmt)
+    elif (tuple(out.shape) != (B, 1 + K, S, S) or out.dtype != torch.float32 or out.device != dev
+          or not out.is_contiguous(memory_format=fmt)):
+        raise ValueError("out must be a float32 {} tensor on {} in {}".format((B, 1 + K, S, S), dev, fmt))
+    args = _lib.ProxyArgs(batch=B, in_wh=in_wh, out_wh=S, num_keypoints=K, channels_last=int(bool(channels_last)),
+                          reserved0=0, std=float(std), masks=m8.data_ptr(), keypoints=kp.data_ptr(),
+                          vis=None if v8 is None else v8.data_ptr())
+    with torch.cuda.device(dev):
+        _lib.check(_lib.load().b200smpl_proxy_representation(ctypes.byref(args), out.data_ptr(), _stream(masks)),
+                   "proxy_representation")
+    return out

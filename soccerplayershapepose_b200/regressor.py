@@ -18,7 +18,7 @@ device; the head and `MultiTaskLoss` themselves are device-agnostic (the CPU tes
 """
 from __future__ import annotations
 
-from typing import Callable, Dict, Optional, Sequence, Tuple
+from typing import Callable, Dict, NamedTuple, Optional, Sequence, Tuple, Union
 
 import numpy as np
 import torch
@@ -352,6 +352,25 @@ def gpu_silhouette_renderer(faces, img_wh: int = config.REGRESSOR_IMG_WH, sigma:
     return render
 
 
+class ProxyInputs(NamedTuple):
+    """What a detector gives per crop, for `GraphedTrainStep` to build the proxy representation from inside its graph
+    (`ops.proxy_representation`): masks (B, in_wh, in_wh) bool / uint8 / float, keypoints (B, K, 2) float32 pixels
+    of the in_wh image, vis (B, K) or None; out_wh / std as in the op."""
+    masks: torch.Tensor
+    keypoints: torch.Tensor
+    vis: Optional[torch.Tensor] = None
+    out_wh: int = config.REGRESSOR_IMG_WH
+    std: float = 4.0
+
+
+def _channels_last(module: nn.Module) -> bool:
+    """True when the module's first 4-D parameter (an encoder's first convolution) is in torch.channels_last."""
+    for p in module.parameters():
+        if p.dim() == 4:
+            return p.is_contiguous(memory_format=torch.channels_last) and not p.is_contiguous()
+    return False
+
+
 class GraphedTrainStep:
     """The training step of `train_step` captured ONCE in a CUDA graph and replayed: (encoder +) head forward, SMPL
     layer, loss, backward, gradient all-reduce (NCCL) and a capturable Adam step.  The eager step is bound by ~100
@@ -363,15 +382,29 @@ class GraphedTrainStep:
     so the NCCL kernels of the late layers overlap the encoder's backward, as DistributedDataParallel does eagerly.
     The SMPL layer has no parameters: the buckets are the head (+ encoder) and the loss's log-variances.  Inputs are
     copied into static buffers before each replay; `world_size > 1` requires an initialised NCCL process group.
+    `features` may be a `ProxyInputs`: the static input buffers are then the masks, keypoints and vis, the captured
+    step starts with the proxy kernel writing a static proxy buffer in the encoder's memory format, and a call copies
+    only those raw inputs (pass a `ProxyInputs` of the same shapes, with vis given iff it was given here).
     `fused_loss`: the loss through the fused kernels of csrc/loss.cu instead of eager PyTorch ops (with the
     silhouette term, ops.silhouette_term); `render_silhouettes`: see `predict`, for the eager loss.  The silhouette
     label is one more static label buffer.
     """
 
-    def __init__(self, head: nn.Module, criterion: MultiTaskLoss, smpl: Callable, features: torch.Tensor,
+    def __init__(self, head: nn.Module, criterion: MultiTaskLoss, smpl: Callable,
+                 features: Union[torch.Tensor, ProxyInputs],
                  labels: Dict[str, torch.Tensor], rot6d_to_rotmat: Callable, project_pixels: Optional[Callable],
                  lr: float = 1e-4, world_size: int = 1, warmup: int = 3, fused_loss: bool = False,
                  bucket_mb: float = 8.0, overlap: bool = True, render_silhouettes: Optional[Callable] = None):
+        from . import ops
+        self.proxy = None
+        if isinstance(features, ProxyInputs):
+            self.proxy = ProxyInputs(features.masks.clone(), features.keypoints.clone(),
+                                     None if features.vis is None else features.vis.clone(), int(features.out_wh),
+                                     float(features.std))
+            B, K, S = features.masks.shape[0], features.keypoints.shape[1], self.proxy.out_wh
+            proxy_cl = _channels_last(head)
+            features = torch.empty((B, 1 + K, S, S), dtype=torch.float32, device=features.masks.device,
+                                   memory_format=torch.channels_last if proxy_cl else torch.contiguous_format)
         dev = features.device
         if dev.type != "cuda":
             raise RuntimeError("GraphedTrainStep needs CUDA tensors")
@@ -394,7 +427,7 @@ class GraphedTrainStep:
         for p in order:
             counts[bucket_of[p]] += 1
         self.optimiser = torch.optim.Adam(self.params, lr=lr, capturable=True)
-        self.features = features.clone()
+        self.features = features if self.proxy is not None else features.clone()
         self.labels = {k: v.clone() for k, v in labels.items()}
         need_verts = _needs_verts(criterion)
         render = _renderer(criterion, fused_loss, render_silhouettes)
@@ -424,6 +457,9 @@ class GraphedTrainStep:
         def one_step():
             self.flat_grad.zero_()
             state["pending"], state["sent"] = list(counts), [False] * len(self.buckets)
+            if self.proxy is not None:
+                ops.proxy_representation(self.proxy.masks, self.proxy.keypoints, self.proxy.vis, self.proxy.out_wh,
+                                         self.proxy.std, channels_last=proxy_cl, out=self.features)
             outputs = predict(head, smpl, self.features, rot6d_to_rotmat, None if fused_loss else project_pixels,
                               need_verts=need_verts, render_silhouettes=render)
             loss, _ = criterion.forward_fused(self.labels, outputs) if fused_loss else criterion(self.labels, outputs)
@@ -447,8 +483,17 @@ class GraphedTrainStep:
         with torch.cuda.graph(self.graph):
             self.loss = one_step()
 
-    def __call__(self, features: torch.Tensor, labels: Dict[str, torch.Tensor]) -> torch.Tensor:
-        self.features.copy_(features, non_blocking=True)
+    def __call__(self, features: Union[torch.Tensor, ProxyInputs], labels: Dict[str, torch.Tensor]) -> torch.Tensor:
+        if self.proxy is None:
+            self.features.copy_(features, non_blocking=True)
+        else:
+            if not isinstance(features, ProxyInputs) or (features.vis is None) != (self.proxy.vis is None):
+                raise TypeError("this step was captured from ProxyInputs{}: pass the same kind of inputs".format(
+                    "" if self.proxy.vis is None else " with vis"))
+            self.proxy.masks.copy_(features.masks, non_blocking=True)
+            self.proxy.keypoints.copy_(features.keypoints, non_blocking=True)
+            if features.vis is not None:
+                self.proxy.vis.copy_(features.vis, non_blocking=True)
         for k, v in labels.items():
             self.labels[k].copy_(v, non_blocking=True)
         self.graph.replay()
