@@ -220,6 +220,8 @@ B200SMPL_API int b200smpl_perspective_project_camk_backward(const float* points,
  * vis [B][nmap] uint8 or NULL, loss: device buffer of 2 floats zeroed by the caller ([0] receives
  * the loss, [1] is scratch for the visible-pair count),
  * grad_joints [B][NJ][3] and grad_cam [B][3] written (d loss / d .) when non-NULL.
+ * No visible pair (vis all zero): the mean counts as 0, so loss = log_var and the gradients are zero (the
+ * reference's mean over an empty selection is NaN).  batch, num_joints, nmap >= 1, else B200SMPL_ERR_INVALID.
  */
 B200SMPL_API int b200smpl_joints2d_loss(const float* joints, const float* cam, const int32_t* joint_map, const float* label,
                            const uint8_t* vis, int batch, int num_joints, int nmap, float proj_wh, float norm_wh,
@@ -237,6 +239,9 @@ B200SMPL_API int b200smpl_joints2d_loss(const float* joints, const float* cam, c
  *   reprojection error (cam_utils.py:5-26 -> joints2d_utils.py:5-10 -> multi_task_loss.py:97-113 for ONE player)
  *   * exp(-log_var) + log_var + shape_weight * mean(betas^2)   (multi_task_loss.py:120-124 against zeros);
  *   grad_joints [B][NJ][3], grad_cam [B][3], grad_betas [B][nb] (shape term only; may be NULL) are written.
+ *   A player with no visible pair gets the mean 0: loss = log_var + the shape term, zero joint and camera gradients
+ *   (a fully occluded player never turns the best-iterate comparison into NaN).  batch, num_joints, nmap and
+ *   num_betas >= 1, else B200SMPL_ERR_INVALID.
  * fit_mark_best: improved[b] = loss < best_loss (best_loss, best_iter updated); step[1] = step[0] + 1.
  * fit_adam_step: params [B][cols]; rows flagged improved are first copied to best_params (the parameters that
  *   produced this iteration's loss, player_recon.py:1258-1262), then torch.optim.Adam's update with the gradient

@@ -254,6 +254,20 @@ def joints2d_loss(pred_pixels: torch.Tensor, label_pixels: torch.Tensor, log_var
     return mse * torch.exp(-log_var) + log_var
 
 
+def fit_loss_per_player(pred_pixels: torch.Tensor, label_pixels: torch.Tensor, log_var: float, betas: torch.Tensor,
+                        shape_weight: float, img_wh: float = 256.0, vis: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Per-player loss of the fitting loop (B,): `joints2d_loss` applied to ONE player (pred/label (B,K,2) pixels, vis
+    (B,K) bool or None) + shape_weight * mean(betas^2).  A player with no visible keypoint has mean 0 (loss =
+    log_var + shape term), where `joints2d_loss` would return NaN."""
+    w = torch.ones(pred_pixels.shape[:2], dtype=pred_pixels.dtype, device=pred_pixels.device) if vis is None \
+        else vis.to(pred_pixels.dtype)
+    d = ((2.0 * pred_pixels) / img_wh - 1.0) - ((2.0 * label_pixels) / img_wh - 1.0)
+    sq = (d * d).sum(-1) * w
+    count = 2.0 * w.sum(1)
+    mse = sq.sum(1) / count.clamp(min=1.0)          # an empty sum over a zero count stays 0
+    return mse * float(np.exp(-log_var)) + log_var + shape_weight * (betas * betas).mean(1)
+
+
 def init_log_var(weight: float, eps: float = 1e-6) -> float:
     """losses/multi_task_loss.py:38: log_var0 = -log(w + eps)."""
     return float(-np.log(weight + eps))

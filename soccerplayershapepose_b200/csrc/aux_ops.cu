@@ -138,15 +138,18 @@ __global__ void ortho_bwd_kernel(const float* __restrict__ pts, const float* __r
   for (int i = threadIdx.x; i < n; i += blockDim.x) {
     const float* p = pts + ((size_t)b * n + i) * 3;
     const float gu = gout[((size_t)b * n + i) * 2] * k, gv = gout[((size_t)b * n + i) * 2 + 1] * k;
+    // __fmul_rn is never contracted into the sums: the compiler unswitches this loop on gpts, and a product that is
+    // stored in one copy but fused into gtx / gty in the other would give grad_cam other last bits without grad_points
+    const float sgu = __fmul_rn(s, gu), sgv = __fmul_rn(s, gv);
     if (gpts != nullptr) {
       float* g = gpts + ((size_t)b * n + i) * 3;
-      g[0] = s * gu;
-      g[1] = s * gv;
+      g[0] = sgu;
+      g[1] = sgv;
       g[2] = 0.f;
     }
     gs += gu * (p[0] + tx) + gv * (p[1] + ty);
-    gtx += s * gu;
-    gty += s * gv;
+    gtx += sgu;
+    gty += sgv;
   }
   if (gcam != nullptr) {
     gs = block_sum(gs, sh);
@@ -427,7 +430,7 @@ int b200smpl_joints2d_loss(const float* joints, const float* cam, const int32_t*
                            const uint8_t* vis, int batch, int num_joints, int nmap, float proj_wh, float norm_wh,
                            float log_var, float* loss, float* grad_joints, float* grad_cam, void* stream) {
   B200_NVTX("b200smpl_joints2d_loss");
-  if (!joints || !cam || !joint_map || !label || !loss || batch < 1 || nmap < 1)
+  if (!joints || !cam || !joint_map || !label || !loss || batch < 1 || num_joints < 1 || nmap < 1)
     return fail(B200SMPL_ERR_INVALID, "bad argument");
   cudaStream_t st = (cudaStream_t)stream;
   const float* count_ptr = nullptr;

@@ -237,6 +237,8 @@ int b200smpl_fit_loss(const float* joints, const float* cam, const int32_t* join
   if (!joints || !cam || !joint_map || !label || !betas || !loss_per_body || !grad_joints || !grad_cam || batch < 1 ||
       nmap < 1)
     return fail(B200SMPL_ERR_INVALID, "bad argument");
+  // mean(beta^2) over no betas would be 0 / 0 = NaN for every body, whatever shape_weight is
+  if (num_joints < 1 || num_betas < 1) return fail(B200SMPL_ERR_INVALID, "num_joints and num_betas must be >= 1");
   LaunchTimer _timer("fit_loss", (cudaStream_t)stream);
   fit_loss_kernel<<<(batch + 3) / 4, 128, 0, (cudaStream_t)stream>>>(joints, cam, joint_map, label, vis, betas, batch,
                                                                      num_joints, nmap, num_betas, proj_wh, norm_wh, log_var,

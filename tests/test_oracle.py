@@ -250,3 +250,40 @@ def test_five_term_multitask_loss_matches_the_reference_class(intree_golden):
     total, parts = crit(labels, outputs)
     np.testing.assert_allclose(total.item(), g["loss5_out"], rtol=1e-6)
     np.testing.assert_allclose([parts[k].item() for k in names], g["loss5_parts"], rtol=1e-6)
+
+
+def test_fit_loss_per_player_is_joints2d_loss_per_player_plus_shape_term():
+    """The per-player fitting loss the fit_loss kernel is checked against: for each player, `joints2d_loss` on that
+    player alone plus shape_weight * mean(beta^2), values and gradients; a player with no visible keypoint gets
+    log_var + the shape term and no keypoint gradient (where `joints2d_loss` is NaN)."""
+    g = torch.Generator().manual_seed(7)
+    B, K, lv, sw, wh = 6, 45, -0.7, 0.3, 200.0
+    pred = (torch.rand(B, K, 2, generator=g, dtype=torch.float64) * 512).requires_grad_(True)
+    label = torch.rand(B, K, 2, generator=g, dtype=torch.float64) * 512
+    betas = torch.randn(B, 10, generator=g, dtype=torch.float64).requires_grad_(True)
+    vis = torch.rand(B, K, generator=g) > 0.4
+    vis[2] = False
+    vis[3] = False
+    vis[3, 5] = True
+    got = O.fit_loss_per_player(pred, label, lv, betas, sw, wh, vis)
+    got.sum().backward()
+    pred2 = pred.detach().clone().requires_grad_(True)
+    betas2 = betas.detach().clone().requires_grad_(True)
+    lv_t = torch.tensor(lv, dtype=torch.float64)
+    for b in range(B):
+        shape = sw * (betas2[b] ** 2).mean()
+        if b == 2:
+            assert torch.isnan(O.joints2d_loss(pred2[b:b + 1], label[b:b + 1], lv_t, wh, vis[b:b + 1]))
+            want = lv_t + shape
+        else:
+            want = O.joints2d_loss(pred2[b:b + 1], label[b:b + 1], lv_t, wh, vis[b:b + 1]) + shape
+        want.backward()
+        assert abs(got[b].item() - want.item()) < 1e-12 * max(1.0, abs(want.item())), b
+    torch.testing.assert_close(pred.grad, pred2.grad, rtol=1e-12, atol=1e-15)
+    torch.testing.assert_close(betas.grad, betas2.grad, rtol=1e-12, atol=1e-15)
+    assert pred.grad[2].abs().max().item() == 0.0
+    # without a mask every keypoint counts
+    full = O.fit_loss_per_player(pred.detach(), label, lv, betas.detach(), sw, wh)
+    for b in range(B):
+        want = O.joints2d_loss(pred.detach()[b:b + 1], label[b:b + 1], lv_t, wh) + sw * (betas.detach()[b] ** 2).mean()
+        assert abs(full[b].item() - want.item()) < 1e-12 * max(1.0, abs(want.item())), b
