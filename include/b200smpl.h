@@ -386,6 +386,34 @@ typedef struct b200smpl_proxy_args {
 } b200smpl_proxy_args;
 B200SMPL_API int b200smpl_proxy_representation(const b200smpl_proxy_args* args, float* out, void* stream);
 
+/*
+ * Reconstruction errors on the device -- replaces the reference's host-side metrics (the tracker of
+ * metrics/train_loss_and_metrics_tracker.py:117-121 over utils/eval_utils.py procrustes_analysis_batch and
+ * scale_and_translation_transform_batch, after a .cpu().numpy() of the meshes).  Definition (DESIGN.md section 13),
+ * per body and point set, with N points p_i (prediction) and q_i (target):
+ *   E        (1/N) sum_i |p_i - q_i|, the mean Euclidean distance (not the RMS);
+ *   SC       E of p_i' = (p_i - mu_P) r_Q / r_P + mu_Q, r = sqrt(sum |p_i - mu|^2 / N);
+ *   PA       E of p_i' = s R (p_i - mu_P) + mu_Q, R the rotation in SO(3) maximising tr(R K), K = sum x_i y_i^T of
+ *            the centred points, s = tr(R K) / sum |x_i|^2 (a mirrored prediction still gets a proper rotation).
+ *   When all predicted points of a set coincide, p_i' = mu_Q; a non-finite point makes the three columns of its set
+ *   NaN.  The vertex set is rows [0, num_verts) of the meshes, the joint set rows joint_map[0 .. num_map) of the joints.
+ * out is [B][6]: pve pve_sc pve_pa mpjpe mpjpe_sc mpjpe_pa, at any 4-byte-aligned address; the three columns of an
+ * absent pair are not written.  Inputs are fp32 at any 4-byte-aligned address.  Results are bitwise deterministic and
+ * independent of a body's position in the batch.  B200SMPL_ERR_INVALID, before any launch, for batch < 1, a NULL out,
+ * a prediction without its target (or the reverse), num_verts < 1 with vertices given, num_joints or num_map < 1 with
+ * joints given, a NULL joint_map with joints given, or neither pair given.  Entries of joint_map must lie in
+ * [0, num_joints) (not checked: device memory).  One kernel launch, no workspace.
+ */
+typedef struct b200smpl_recon_error_args {
+  int32_t batch, num_verts, num_joints, num_map, reserved0, reserved1;
+  const float* pred_vertices;    /* [B][V][3] or NULL */
+  const float* target_vertices;  /* [B][V][3], NULL iff pred_vertices is */
+  const float* pred_joints;      /* [B][NJ][3] or NULL */
+  const float* target_joints;    /* [B][NJ][3], NULL iff pred_joints is */
+  const int32_t* joint_map;      /* [num_map] device, entries in [0, NJ) */
+} b200smpl_recon_error_args;
+B200SMPL_API int b200smpl_reconstruction_errors(const b200smpl_recon_error_args* args, float* out, void* stream);
+
 /* Test hook (host arithmetic only, no device): the cluster work list of the forward blend GEMM for `body_tiles`
  * 128-body tiles x `row_tiles` 128-row tiles on a device with `num_sms` SMs.  Writes (body-tile pair, first row-tile
  * pair, end row-tile pair) per cluster into out[3 * capacity]; returns the number of clusters or -1. */

@@ -100,6 +100,15 @@ class ProxyArgs(Structure):
     ]
 
 
+class ReconErrorArgs(Structure):
+    _fields_ = [
+        ("batch", c_int32), ("num_verts", c_int32), ("num_joints", c_int32), ("num_map", c_int32),
+        ("reserved0", c_int32), ("reserved1", c_int32),
+        ("pred_vertices", c_void_p), ("target_vertices", c_void_p), ("pred_joints", c_void_p),
+        ("target_joints", c_void_p), ("joint_map", c_void_p),
+    ]
+
+
 # every symbol include/b200smpl.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "b200smpl_model_create": (c_int, [POINTER(ModelDesc), c_int, POINTER(c_void_p)]),
@@ -145,6 +154,7 @@ SYMBOLS = {
                                          c_void_p]),
     "b200smpl_silhouette_loss_value": (c_int, [POINTER(SilhouetteArgs), c_void_p, c_float, c_void_p, c_void_p]),
     "b200smpl_proxy_representation": (c_int, [POINTER(ProxyArgs), c_void_p, c_void_p]),
+    "b200smpl_reconstruction_errors": (c_int, [POINTER(ReconErrorArgs), c_void_p, c_void_p]),
     "b200smpl_debug_fwd_gemm_worklist":(c_int, [c_int, c_int, c_int, c_void_p, c_int]),
     "b200smpl_last_error": (c_char_p, []),
     "b200smpl_abi_version": (c_int, []),

@@ -40,6 +40,8 @@ ALL_JOINTS_TO_H36M_MAP = list(range(NUM_ALL_JOINTS - NUM_H36M_JOINTS, NUM_ALL_JO
 # 17 -> LSP-17 / LSP-14 re-ordering of the H36M block
 H36M_TO_J17 = [6, 5, 4, 1, 2, 3, 16, 15, 14, 11, 12, 13, 8, 10, 0, 7, 9]
 H36M_TO_J14 = H36M_TO_J17[:14]
+# the LSP-14 joints of the superset, joints[:, ALL_JOINTS_TO_H36M_MAP][:, H36M_TO_J14] (the MPJPE joints)
+ALL_JOINTS_TO_J14_MAP = [ALL_JOINTS_TO_H36M_MAP[i] for i in H36M_TO_J14]
 # Keypoint-RCNN order is the COCO order
 SMPL_TO_KPRCNN_MAP = list(ALL_JOINTS_TO_COCO_MAP)
 

@@ -598,3 +598,61 @@ def proxy_representation(masks: torch.Tensor, keypoints: torch.Tensor, vis: Opti
         _lib.check(_lib.load().b200smpl_proxy_representation(ctypes.byref(args), out.data_ptr(), _stream(masks)),
                    "proxy_representation")
     return out
+
+
+# ---- reconstruction errors (DESIGN.md section 13) ---------------------------------------------------------------------
+def _point_pair(pred: Optional[torch.Tensor], target: Optional[torch.Tensor], what: str):
+    if (pred is None) != (target is None):
+        raise ValueError("pred_{0} and target_{0} must both be given or both be None".format(what))
+    if pred is None:
+        return None, None
+    pred, target = _req(pred, "pred_" + what), _req(target, "target_" + what)
+    if pred.dim() != 3 or pred.shape[2] != 3 or pred.shape[1] < 1 or target.shape != pred.shape:
+        raise ValueError("pred_{0} {1} and target_{0} {2} must both be (B, N, 3) with N >= 1".format(
+            what, tuple(pred.shape), tuple(target.shape)))
+    if target.device != pred.device:
+        raise ValueError("pred_{0} is on {1}, target_{0} on {2}".format(what, pred.device, target.device))
+    return pred, target
+
+
+def reconstruction_errors(pred_vertices: Optional[torch.Tensor] = None, target_vertices: Optional[torch.Tensor] = None,
+                          pred_joints: Optional[torch.Tensor] = None, target_joints: Optional[torch.Tensor] = None,
+                          joint_map: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Per-body reconstruction errors in one kernel (the reference's metrics tracker over utils/eval_utils.py, without
+    the copy to the host) -> (B, 6) float32 columns pve, pve_sc, pve_pa, mpjpe, mpjpe_sc, mpjpe_pa: the mean Euclidean
+    distance between prediction and target (in the inputs' units), as given, after the scale-and-translation
+    correction (SC) and after the Procrustes similarity alignment (PA, a proper rotation).  Vertices (B, V, 3) float32;
+    joints (B, NJ, 3) float32 with `joint_map` (M,) integer rows in [0, NJ) (e.g.
+    config.ALL_JOINTS_TO_H36M_MAP[H36M_TO_J14]); the joints get their own transforms.  The columns of an absent pair
+    are NaN.  Plain tensor ops and one C-ABI call (the joint-map range check is cached and skipped inside a
+    capture), so a CUDA graph can capture it."""
+    pv, tv = _point_pair(pred_vertices, target_vertices, "vertices")
+    pj, tj = _point_pair(pred_joints, target_joints, "joints")
+    if pv is None and pj is None:
+        raise ValueError("reconstruction_errors needs vertices, joints or both")
+    if pj is None and joint_map is not None:
+        raise ValueError("joint_map given without joints")
+    B, dev = (pv if pv is not None else pj).shape[0], (pv if pv is not None else pj).device
+    if pv is not None and pj is not None and (pj.shape[0] != B or pj.device != dev):
+        raise ValueError("vertices ({}, on {}) and joints ({}, on {}) disagree in batch or device".format(
+            B, dev, pj.shape[0], pj.device))
+    m32, M = None, 0
+    if pj is not None:
+        if joint_map is None:
+            raise ValueError("joints need a joint_map")
+        M = joint_map.numel()
+        if M < 1:
+            raise ValueError("joint_map is empty")
+        m32 = _checked_joint_map(joint_map, dev, pj.shape[1])
+    out = torch.full((B, 6), float("nan"), dtype=torch.float32, device=dev)
+    args = _lib.ReconErrorArgs(batch=B, num_verts=0 if pv is None else pv.shape[1],
+                               num_joints=0 if pj is None else pj.shape[1], num_map=M, reserved0=0, reserved1=0,
+                               pred_vertices=None if pv is None else pv.data_ptr(),
+                               target_vertices=None if tv is None else tv.data_ptr(),
+                               pred_joints=None if pj is None else pj.data_ptr(),
+                               target_joints=None if tj is None else tj.data_ptr(),
+                               joint_map=None if m32 is None else m32.data_ptr())
+    with torch.cuda.device(dev):
+        _lib.check(_lib.load().b200smpl_reconstruction_errors(ctypes.byref(args), out.data_ptr(), _stream(out)),
+                   "reconstruction_errors")
+    return out

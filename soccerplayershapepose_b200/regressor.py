@@ -248,6 +248,38 @@ def train_step(head: nn.Module, criterion: MultiTaskLoss, optimiser: torch.optim
     return loss.detach()
 
 
+def validation_step(head: nn.Module, criterion: MultiTaskLoss, smpl: Callable, features: torch.Tensor,
+                    labels: Dict[str, torch.Tensor], rot6d_to_rotmat: Callable, project_pixels: Optional[Callable],
+                    fused_loss: bool = False,
+                    render_silhouettes: Optional[Callable] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """One validation batch (the reference's `is_train = False` pass, PyTorch3DTest.py:947-1118) -> (loss, errors).
+    Under torch.no_grad: `predict` (forward-only SMPL calls), the criterion as `train_step` evaluates it (eager or
+    `fused_loss`; the fused silhouette term then only evaluates its value), the target bodies from
+    labels["pose_params_rot_matrices"] and labels["shape_params"] (PyTorch3DTest.py:1036-1042), and one T-pose forward
+    (zero pose, zero translation) of the predicted and target shapes.  errors (B, 7) float32 on the device: pve,
+    pve_sc, pve_pa, mpjpe, mpjpe_sc, mpjpe_pa (`ops.reconstruction_errors` on the vertices and the LSP-14 joints,
+    config.ALL_JOINTS_TO_J14_MAP) and pve_t_sc (pve_sc of the T-pose meshes), in the SMPL model's units.  It never
+    synchronises with the host (after the first call, which checks the joint map once) and touches no gradient or
+    optimiser state.  Per-epoch sums stay on the device: `sums += errors.sum(0)`."""
+    from . import ops
+    with torch.no_grad():
+        outputs = predict(head, smpl, features, rot6d_to_rotmat, None if fused_loss else project_pixels,
+                          need_verts=True, render_silhouettes=_renderer(criterion, fused_loss, render_silhouettes))
+        crit = getattr(criterion, "module", criterion)
+        loss, _ = crit.forward_fused(labels, outputs) if fused_loss else criterion(labels, outputs)
+        rot, shape = labels["pose_params_rot_matrices"], labels["shape_params"]
+        target = smpl(body_pose=rot[:, 1:], global_orient=rot[:, 0].unsqueeze(1), betas=shape, pose2rot=False)
+        pred_shape = outputs["shape_params"]
+        B, dev = pred_shape.shape[0], pred_shape.device
+        eye = torch.eye(3, dtype=torch.float32, device=dev).expand(2 * B, 24, 3, 3)
+        tpose = smpl(body_pose=eye[:, 1:], global_orient=eye[:, :1], betas=torch.cat([pred_shape, shape]),
+                     transl=torch.zeros((2 * B, 3), dtype=torch.float32, device=dev), pose2rot=False).vertices
+        errors = ops.reconstruction_errors(outputs["verts"], target.vertices, outputs["joints"], target.joints,
+                                           _index32("ALL_JOINTS_TO_J14_MAP", dev))
+        t_sc = ops.reconstruction_errors(tpose[:B], tpose[B:])[:, 1:2]
+        return loss.detach(), torch.cat([errors, t_sc], dim=1)
+
+
 def _tasks(criterion) -> Sequence[str]:
     return getattr(criterion, "module", criterion).losses_on
 
